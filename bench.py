@@ -2,7 +2,7 @@
 """Benchmark of the ModelBiLSTM hot path (BASELINE.json metric: classified sites/s,
 both_bilstm bn13_sn16 hidden 256, batch 65536).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision fp16|fp32]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--precision fp16|fp32] [--dump-outputs DIR]
 
 One "step" = one batch of 65 536 synthetic sites through the forward pass.  Prints ONE JSON
 line (rank 0).  See DESIGN.md section "Measurement" for what every key means.
@@ -119,6 +119,26 @@ def make_pool(n_buffers, batch, seed=0, T=13, S=16):
     base = synthetic.make_features(batch, T, S, seed=seed)
     keys = ("kmer", "base_means", "base_stds", "base_signal_lens", "signals")
     return [tuple(np.ascontiguousarray(np.roll(base[k], 977 * b, axis=0)) for k in keys) for b in range(n_buffers)]
+
+
+DUMP_MAX_BYTES = 60_000_000          # array data; with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(directory, arrays, max_bytes=DUMP_MAX_BYTES):
+    """Write each (name, tensor) of `arrays` (equal first dimension) as directory/<name>.npy in float32.  When they
+    would take more than `max_bytes` together, every array is cut to the same fixed, seeded sample of rows (ascending)
+    and the sampled row indices are written as directory/rows.npy (float64), all within `max_bytes`."""
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    n = arrays[0][1].shape[0]
+    row_bytes = sum(4 * (t.numel() // n) for _, t in arrays)
+    if n * row_bytes > max_bytes:
+        rows = np.sort(np.random.default_rng(0).choice(n, max_bytes // (row_bytes + 8), replace=False))
+        np.save(os.path.join(directory, "rows.npy"), rows.astype(np.float64))
+        idx = torch.from_numpy(rows)
+        arrays = [(name, t.index_select(0, idx.to(t.device))) for name, t in arrays]
+    for name, t in arrays:
+        np.save(os.path.join(directory, name + ".npy"), t.float().cpu().numpy())
 
 
 def port_baseline_run(sites, threads):
@@ -252,12 +272,20 @@ def main():
     ap.add_argument("--module", default="both_bilstm", choices=["both_bilstm", "seq_bilstm", "signal_bilstm"])
     ap.add_argument("--seq_len", type=int, default=13)
     ap.add_argument("--signal_len", type=int, default=16)
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0: logits, probs, labels) as DIR/<name>.npy in float32, "
+                         "at most 64 MB (a fixed, seeded sample of rows, listed in DIR/rows.npy, above that); inputs, weights "
+                         "and initial states are seeded, so equal arguments give equal inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs dumps the device forward: it needs --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if args.steps is None:
         args.steps = 100 if args.precision == "fp16" else 4
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         reference_arm(args, rank, world)
         return
@@ -313,7 +341,7 @@ def main():
     barrier()
     ev0.record()
     for i in range(args.steps):
-        model(*dev_pool[i % len(dev_pool)])
+        out = model(*dev_pool[i % len(dev_pool)])
     ev1.record()
     barrier()
     launches = model.launch_count() - launches0
@@ -331,6 +359,9 @@ def main():
             kern_ms += float(t.value)
             kern_launches += int(cnt.value)
     _native.check(L.dsp_set_timing(model._handle, 0))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, [("logits", out[0]), ("probs", out[1]), ("labels", model.last_labels)])
+    del out
 
     # ---- e2e: host buffers through the public host API, H2D + D2H inside ----------------
     # Every step's inputs start in pinned host memory and its logits/probs/labels end in pinned

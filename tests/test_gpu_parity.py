@@ -226,6 +226,70 @@ def test_init_hidden_mode_reproduces_reference_rng_stream():
     assert same_label / len(gold) >= LABEL_AGREEMENT
 
 
+def _compare_call_lines(lines, gold, prob_tol):
+    """call_mods lines against the reference's: sample info and 5-mer identical, probabilities within prob_tol.
+    Returns the number of label flips."""
+    assert len(lines) == len(gold)
+    flips = 0
+    for a, b in zip(lines, gold):
+        wa, wb = a.split("\t"), b.split("\t")
+        assert len(wa) == 10 and wa[:6] == wb[:6] and wa[9] == wb[9]
+        assert abs(float(wa[6]) - float(wb[6])) <= prob_tol and abs(float(wa[7]) - float(wb[7])) <= prob_tol
+        flips += wa[8] != wb[8]
+    return flips
+
+
+def test_call_mods_fp16_reproduces_reference_lines():
+    # the fp16 path through _call_mods against the reference's own run (callmods_77.tsv.gz), equal seeds
+    from oracle.run_ref_callmods import features_batch
+    from deepsignal_plant_b200.models import ModelBiLSTM
+    e = cases.MANIFEST["callmods"]
+    torch.manual_seed(e["weight_seed"])
+    model = ModelBiLSTM(13, 16, 3, 1, 2, 0, 256, 16, 4, True, True, module="both_bilstm", precision="fp16",
+                        state_mode="init_hidden").cuda(0).eval()
+    batch = features_batch(e["n"], 13, 16, e["feature_seed"])
+    torch.manual_seed(e["rng_seed"])
+    lines, acc, nb = cm._call_mods(batch, model, e["batch"], 0)
+    assert model.launch_count() > 0 and nb == (e["n"] + e["batch"] - 1) // e["batch"]
+    gold = cases.read_gz("callmods_%d.tsv.gz" % e["rng_seed"]).splitlines()
+    assert _compare_call_lines(lines, gold, PROB_TOL) <= max(1, int(len(gold) * (1 - LABEL_AGREEMENT)))
+
+
+def test_call_mods_worker_loop_reproduces_reference_lines(tmp_path, monkeypatch):
+    # _call_mods_q (call_modifications.py:195-259): constructor call with the reference's positional arguments,
+    # checkpoint load, queue loop until "kill"; the expectation is the reference's CPU _call_mods run at the same
+    # seeds (callmods_99.tsv.gz, manifest "callmods_worker")
+    import queue
+    import types
+    from oracle.run_ref_callmods import features_batch
+    from deepsignal_plant_b200.models import ModelBiLSTM
+    e = cases.MANIFEST["callmods_worker"]
+    n, bs = e["n"], e["batch"]
+    torch.manual_seed(e["weight_seed"])
+    ckpt = str(tmp_path / "both_bilstm.b13_s16_epoch0.ckpt")
+    torch.save(ModelBiLSTM(13, 16, 3, 1, 2, 0, 256, 16, 4, True, True).state_dict(), ckpt)   # train.py:161
+
+    class InitHiddenModel(ModelBiLSTM):
+        def __init__(self, *a, **kw):
+            super().__init__(*a, state_mode="init_hidden", **kw)
+    args = types.SimpleNamespace(seq_len=13, signal_len=16, layernum1=3, layernum2=1, class_num=2, dropout_rate=0, hid_rnn=256,
+                                 n_vocab=16, n_embed=4, is_base="yes", is_signallen="yes", model_type="both_bilstm", batch_size=bs)
+    fq, pq = queue.Queue(), queue.Queue()
+    fq.put(features_batch(n, 13, 16, e["feature_seed"]))
+    fq.put("kill")
+    orig = cm._call_mods
+
+    def seeded(batch, model, batch_size, device=0):      # the reference run seeds right before _call_mods
+        torch.manual_seed(e["rng_seed"])
+        return orig(batch, model, batch_size, device)
+    monkeypatch.setattr(cm, "ModelBiLSTM", InitHiddenModel)
+    monkeypatch.setattr(cm, "_call_mods", seeded)
+    cm._call_mods_q(ckpt, fq, pq, None, args, 0)
+    lines = pq.get_nowait()
+    gold = cases.read_gz("callmods_%d.tsv.gz" % e["rng_seed"]).splitlines()
+    assert _compare_call_lines(lines, gold, PROB_TOL) <= 1
+
+
 def test_forward_host_matches_device_path():
     case = cases.slice_case(cases.load_case("both_13_16_s1"), 3000)
     dev = torch.device("cuda:0")
