@@ -21,6 +21,7 @@ SYMBOLS = (
     "dsp_format_features", "dsp_parse_calls", "dsp_format_freq",
     "dsp_comm_create", "dsp_comm_export", "dsp_comm_connect", "dsp_comm_destroy", "dsp_freq_aggregate_distributed",
     "dsp_comm_route_rows", "dsp_comm_last_timing", "dsp_freq_aggregate_host", "dsp_device_warmup",
+    "dsp_train_shape", "dsp_train_arena_bytes", "dsp_train_workspace_bytes", "dsp_train_forward", "dsp_train_backward",
 )
 
 MODULES = {"both_bilstm": 0, "seq_bilstm": 1, "signal_bilstm": 2}
@@ -103,6 +104,14 @@ def lib():
                                                  C.POINTER(i64), C.POINTER(i64), vp, vp]
     L.dsp_comm_route_rows.argtypes = [vp, vp, i64, i32, i32, vp, vp, i64, C.POINTER(i64), vp]
     L.dsp_comm_last_timing.argtypes = [vp, vp]
+    L.dsp_train_shape.argtypes = [vp, C.POINTER(i32), C.POINTER(i32)]
+    L.dsp_train_arena_bytes.argtypes = [vp, i64]
+    L.dsp_train_arena_bytes.restype = i64
+    L.dsp_train_workspace_bytes.argtypes = [vp, i64]
+    L.dsp_train_workspace_bytes.restype = i64
+    L.dsp_train_forward.argtypes = [vp, C.POINTER(vp), i32, fp, fp, fp, fp, fp, C.POINTER(vp), u64, C.POINTER(vp), i64, vp,
+                                    fp, vp]
+    L.dsp_train_backward.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(vp), vp, fp, i64, vp, C.POINTER(vp), vp]
     for name in SYMBOLS:
         getattr(L, name)  # AttributeError here means header and library disagree
     _lib = L

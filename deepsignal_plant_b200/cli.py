@@ -9,16 +9,53 @@ reference's flag names and defaults.
     python -m deepsignal_plant_b200 extract   -i reads.npz -o features.dspf     # ... -> binary hand-off (feature_bin.py)
     python -m deepsignal_plant_b200 call_mods -i features.dspf -m model.ckpt -o calls.tsv      # same calls, no text parsing
     python -m deepsignal_plant_b200 pack_features -i features.tsv -o features.dspf             # an existing text file -> binary
+    python -m deepsignal_plant_b200 train --train_file train.dspf --valid_file valid.dspf --model_dir models/
 
 Multi-GPU: launch ``call_mods`` or ``call_freq`` under torchrun, one process per GPU.  ``call_mods`` cuts the feature
 file (or the reads archive) into contiguous shards and concatenates the output in file order, no collective on the
 data path; ``call_freq`` parses contiguous byte shards, exchanges the records by site key over NVLink peer memory and
 every rank writes its slice of the table (freq_dist.py).  ``extract`` here takes reads that are already decoded
-(reading fast5 needs h5py: outside this implementation); ``train`` and ``denoise`` stay with the reference."""
+(reading fast5 needs h5py: outside this implementation); ``train`` runs the reference's training loop on the fp32 training kernels (train.py); ``denoise`` stays with the
+reference."""
 from __future__ import annotations
 
 import argparse
 import sys
+
+
+def add_train_parser(sub):
+    """The reference's ``train`` flags and defaults (``deepsignal_plant.py`` train parser)."""
+    tp = sub.add_parser("train", description="train a model on labelled features (.dspf or the reference's text file)")
+    g = tp.add_argument_group("INPUT")
+    g.add_argument("--train_file", type=str, required=True)
+    g.add_argument("--valid_file", type=str, required=True)
+    g = tp.add_argument_group("OUTPUT")
+    g.add_argument("--model_dir", type=str, required=True)
+    g = tp.add_argument_group("MODEL_HYPER")
+    g.add_argument("--model_type", type=str, default="both_bilstm",
+                   choices=["both_bilstm", "seq_bilstm", "signal_bilstm"], required=False)
+    g.add_argument("--seq_len", type=int, default=13, required=False)
+    g.add_argument("--signal_len", type=int, default=16, required=False)
+    g.add_argument("--layernum1", type=int, default=3, required=False)
+    g.add_argument("--layernum2", type=int, default=1, required=False)
+    g.add_argument("--class_num", type=int, default=2, required=False)
+    g.add_argument("--dropout_rate", type=float, default=0.5, required=False)
+    g.add_argument("--n_vocab", type=int, default=16, required=False)
+    g.add_argument("--n_embed", type=int, default=4, required=False)
+    g.add_argument("--is_base", type=str, default="yes", required=False)
+    g.add_argument("--is_signallen", type=str, default="yes", required=False)
+    g.add_argument("--hid_rnn", type=int, default=256, required=False)
+    g = tp.add_argument_group("TRAINING")
+    g.add_argument("--optim_type", type=str, default="Adam", choices=["Adam", "RMSprop", "SGD"], required=False)
+    g.add_argument("--batch_size", type=int, default=512, required=False)
+    g.add_argument("--lr", type=float, default=0.001, required=False)
+    g.add_argument("--max_epoch_num", type=int, default=10, required=False)
+    g.add_argument("--min_epoch_num", type=int, default=5, required=False)
+    g.add_argument("--step_interval", type=int, default=100, required=False)
+    g.add_argument("--pos_weight", type=float, default=1.0, required=False)
+    g.add_argument("--init_model", type=str, default=None, required=False)
+    g.add_argument("--tseed", type=int, default=1234, required=False)
+    return tp
 
 
 def build_parser():
@@ -27,6 +64,7 @@ def build_parser():
     sub = parser.add_subparsers(title="modules", dest="module")
     cm = sub.add_parser("call_mods", description="call modifications")
     cf = sub.add_parser("call_freq", description="call frequency of modifications at genome level")
+    add_train_parser(sub)
 
     ex = sub.add_parser("extract", description="extract features from decoded re-squiggled reads (an .npz archive written by "
                                                "extract_features.save_reads) into the reference's feature file")
@@ -184,6 +222,9 @@ def main(argv=None):
         from .feature_bin import pack_feature_file
         n = pack_feature_file(args.input_path, args.write_path, nthreads=args.host_threads or None)
         print("[pack_features] {} sites -> {}".format(n, args.write_path))
+    elif args.module == "train":
+        from .train import main as train_main
+        train_main(args)
     elif args.module == "call_freq":
         from .call_mods_freq import call_mods_frequency_to_file
         call_mods_frequency_to_file(args)

@@ -582,6 +582,55 @@ int dsp_forward_host_wait(dsp_handle h, int64_t ticket) {
     return DSP_OK;
 }
 
+int dsp_train_shape(dsp_handle h, int32_t* n_params, int32_t* n_masks) {
+    DSP_REQUIRE(h, DSP_ERR_INVALID, "dsp_train_shape: null handle");
+    return train_shape(h, n_params, n_masks);
+}
+
+int64_t dsp_train_arena_bytes(dsp_handle h, int64_t n) { return (h && n >= 0) ? train_arena_bytes(h, n) : -1; }
+int64_t dsp_train_workspace_bytes(dsp_handle h, int64_t n) { return (h && n >= 0) ? train_workspace_bytes(h, n) : -1; }
+
+static int train_check(Model* m, const char* who, const float* const* params, int32_t n_params, const float* const* masks,
+                       const void* arena, int64_t n) {
+    int32_t np = 0, nm = 0;
+    train_shape(m, &np, &nm);
+    DSP_REQUIRE(params && masks && arena, DSP_ERR_INVALID, "%s: null argument", who);
+    DSP_REQUIRE(n_params == np, DSP_ERR_INVALID, "%s: %d parameters given, this configuration has %d", who, n_params, np);
+    for (int i = 0; i < np; ++i) DSP_REQUIRE(params[i], DSP_ERR_INVALID, "%s: parameter %d is null", who, i);
+    DSP_REQUIRE(n >= 1, DSP_ERR_INVALID, "%s: batch must hold at least one site", who);
+    return DSP_OK;
+}
+
+int dsp_train_forward(dsp_handle h, const float* const* params, int32_t n_params, const float* kmer,
+                      const float* base_means, const float* base_stds, const float* base_signal_lens,
+                      const float* signals, const float* const* states, uint64_t seed,
+                      const float* const* dropout_masks, int64_t n, void* arena, float* logits, void* stream) {
+    DSP_REQUIRE(h, DSP_ERR_INVALID, "dsp_train_forward: null handle");
+    Model* m = h;
+    int rc = train_check(m, "dsp_train_forward", params, n_params, dropout_masks, arena, n);
+    if (rc) return rc;
+    DSP_REQUIRE(logits, DSP_ERR_INVALID, "dsp_train_forward: null output pointer");
+    if (has_seq(m)) DSP_REQUIRE(kmer && base_means && base_stds && base_signal_lens, DSP_ERR_INVALID,
+                                "dsp_train_forward: sequence features are required for this module");
+    if (has_signal(m)) DSP_REQUIRE(signals, DSP_ERR_INVALID, "dsp_train_forward: signals are required for this module");
+    DeviceGuard guard(m->cfg.device);
+    return train_forward(m, params, kmer, base_means, base_stds, base_signal_lens, signals, states, seed, dropout_masks, n,
+                         arena, logits, (cudaStream_t)stream);
+}
+
+int dsp_train_backward(dsp_handle h, const float* const* params, int32_t n_params, const float* const* dropout_masks,
+                       const void* arena, const float* dlogits, int64_t n, void* workspace, float* const* grads,
+                       void* stream) {
+    DSP_REQUIRE(h, DSP_ERR_INVALID, "dsp_train_backward: null handle");
+    Model* m = h;
+    int rc = train_check(m, "dsp_train_backward", params, n_params, dropout_masks, arena, n);
+    if (rc) return rc;
+    DSP_REQUIRE(dlogits && workspace && grads, DSP_ERR_INVALID, "dsp_train_backward: null argument");
+    for (int i = 0; i < n_params; ++i) DSP_REQUIRE(grads[i], DSP_ERR_INVALID, "dsp_train_backward: gradient %d is null", i);
+    DeviceGuard guard(m->cfg.device);
+    return train_backward(m, params, dropout_masks, arena, dlogits, n, workspace, grads, (cudaStream_t)stream);
+}
+
 int64_t dsp_launch_count(dsp_handle h) { return h ? h->launches : 0; }
 
 int dsp_set_timing(dsp_handle h, int enable) {

@@ -144,6 +144,16 @@ int f32_head_flat(Model* m, const float* hfinal, int64_t n, float* logits, float
 int philox_normal(Model* m, float* out, int64_t count, uint64_t seed, uint64_t stream_id,
                   cudaStream_t st);
 
+// ---- fp32 training path (kernels_train.cu) ----------------------------------------------
+int train_shape(const Model* m, int32_t* n_params, int32_t* n_masks);
+int64_t train_arena_bytes(const Model* m, int64_t n);
+int64_t train_workspace_bytes(const Model* m, int64_t n);
+int train_forward(Model* m, const float* const* params, const float* kmer, const float* means, const float* stds,
+                  const float* lens, const float* signals, const float* const* states6, uint64_t seed,
+                  const float* const* masks, int64_t n, void* arena, float* logits, cudaStream_t st);
+int train_backward(Model* m, const float* const* params, const float* const* masks, const void* arena,
+                   const float* dlogits, int64_t n, void* workspace, float* const* grads, cudaStream_t st);
+
 }  // namespace dsp
 
 // the opaque handle type of the C ABI

@@ -10,8 +10,10 @@ and ``load_state_dict`` / ``model_dict.update(para_dict)`` work unchanged,
 
 Differences, all deliberate:
 
-* Only inference is implemented.  ``forward`` in ``train()`` mode raises: the training loop
-  (``train.py``) is outside this hot path and there is no autograd through the kernels.
+* Training is opt-in: ``ModelBiLSTM(..., trainable=True)`` in ``train()`` mode runs ``forward`` through
+  the fp32 training kernels (``csrc/kernels_train.cu``) inside a ``torch.autograd.Function``, so the
+  reference's loop (``train.py:104-128``) works as written.  Without ``trainable=True``, ``forward`` in
+  ``train()`` mode raises as before.  ``eval()`` always runs the inference path of ``precision``.
 * Inputs must be CUDA tensors on the module's device -- there is no CPU path.
 * Initial LSTM states.  The reference draws fresh ``torch.randn`` states on every call
   (``models.py:169-176``).  ``state_mode`` selects how this module gets them:
@@ -38,7 +40,7 @@ class ModelBiLSTM(nn.Module):
                  dropout_rate=0.5, hidden_size=256,
                  vocab_size=16, embedding_size=4, is_base=True, is_signallen=True,
                  module="both_bilstm", device=0, precision=None, max_batch=65536,
-                 state_mode="philox", seed=0):
+                 state_mode="philox", seed=0, trainable=False):
         super().__init__()
         self.model_type = "BiLSTM"
         self.module = module
@@ -96,6 +98,9 @@ class ModelBiLSTM(nn.Module):
         self.max_batch = int(max_batch)
         self.state_mode = state_mode
         self.seed = int(seed)
+        self.dropout_rate = float(dropout_rate)
+        self.trainable = bool(trainable)
+        self.last_dropout_masks = None
         self._calls = 0
         self._handle = None
         self._handle_device = None
@@ -142,7 +147,7 @@ class ModelBiLSTM(nn.Module):
     def __del__(self):
         self._destroy()
 
-    def _ensure_handle(self, dev):
+    def _create_handle(self, dev):
         L = _native.lib()
         if self._handle is not None and self._handle_device != dev.index:
             self._destroy()
@@ -159,6 +164,10 @@ class ModelBiLSTM(nn.Module):
             self._handle = h
             self._handle_device = dev.index
             self._packed_key = None
+        return self._handle
+
+    def _ensure_handle(self, dev):
+        self._create_handle(dev)
         # the Parameter objects persist across .cuda() / load_state_dict (their data pointer / version change): keep the
         # list instead of walking the module tree on every forward
         plist = self.__dict__.get("_plist")
@@ -191,7 +200,53 @@ class ModelBiLSTM(nn.Module):
                                % (t.device, dev))
         return t.detach().reshape(shape).to(torch.float32).contiguous()
 
+    def _init_hidden_states(self, n, dev):
+        """``init_hidden`` for the seq, signal and comb stacks in the reference's order -> (6 device
+        pointers for the library, the tensors behind them)."""
+        has_seq = self.module != "signal_bilstm"
+        has_sig = self.module != "seq_bilstm"
+        keep = []
+        ptrs = (C.c_void_p * 6)()
+        groups = ((has_seq, self.num_layers2, getattr(self, "nhid_seq", 0)),
+                  (has_sig, self.num_layers2, getattr(self, "nhid_signal", 0)),
+                  (True, self.num_layers1, self.hidden_size))
+        for g, (used, layers, hid) in enumerate(groups):
+            if not used:
+                continue
+            h0, c0 = self.init_hidden(n, layers, hid)
+            h0 = h0.detach().to(dev, torch.float32).contiguous()
+            c0 = c0.detach().to(dev, torch.float32).contiguous()
+            if tuple(h0.shape) != (layers * 2, n, hid) or tuple(c0.shape) != (layers * 2, n, hid):
+                raise RuntimeError("init_hidden returned shape %s, expected %s"
+                                   % (tuple(h0.shape), (layers * 2, n, hid)))
+            keep += [h0, c0]
+            ptrs[2 * g], ptrs[2 * g + 1] = h0.data_ptr(), c0.data_ptr()
+        return ptrs, keep
+
+    def dropout_mask_shapes(self, n):
+        """Shapes of the dropout-mask slots of ``dsp_train_forward`` for n sites, ``None`` for a slot this
+        module never uses: nn.LSTM inter-layer dropout of lstm_seq, lstm_signal, lstm_comb (every layer's
+        output but the last), then the head's dropout before and after fc1 (models.py:234-237)."""
+        T, H = self.seq_len, self.hidden_size
+        has_seq = self.module != "signal_bilstm"
+        has_sig = self.module != "seq_bilstm"
+        shapes = [(n, T, 2 * self.nhid_seq) if has_seq else None] * (self.num_layers2 - 1)
+        shapes += [(n, T, 2 * self.nhid_signal) if has_sig else None] * (self.num_layers2 - 1)
+        shapes += [(n, T, 2 * H)] * (self.num_layers1 - 1)
+        return shapes + [(n, 2 * H), (n, H)]
+
+    def draw_dropout_masks(self, n, dev):
+        """keep / (1 - p) masks drawn with torch's CUDA generator (``torch.rand >= p``), as nn.Dropout
+        scales them; all ``None`` when ``dropout_rate`` is 0."""
+        p = self.dropout_rate
+        if p <= 0:
+            return [None] * len(self.dropout_mask_shapes(n))
+        return [None if shp is None else (torch.rand(shp, device=dev) >= p).to(torch.float32).div_(1.0 - p)
+                for shp in self.dropout_mask_shapes(n)]
+
     def forward(self, kmer, base_means, base_stds, base_signal_lens, signals):
+        if self.training and self.trainable:
+            return self._forward_train(kmer, base_means, base_stds, base_signal_lens, signals)
         if self.training:
             raise RuntimeError("deepsignal_plant_b200.ModelBiLSTM implements inference only; "
                                "call .eval() (training is outside the accelerated hot path)")
@@ -210,25 +265,7 @@ class ModelBiLSTM(nn.Module):
         n = (kmer if has_seq else sig).shape[0]
         with torch.cuda.device(dev):
             handle = self._ensure_handle(dev)
-            states_arg = None
-            keep = []
-            if self._uses_init_hidden():
-                ptrs = (C.c_void_p * 6)()
-                groups = ((has_seq, self.num_layers2, getattr(self, "nhid_seq", 0)),
-                          (has_sig, self.num_layers2, getattr(self, "nhid_signal", 0)),
-                          (True, self.num_layers1, self.hidden_size))
-                for g, (used, layers, hid) in enumerate(groups):
-                    if not used:
-                        continue
-                    h0, c0 = self.init_hidden(n, layers, hid)
-                    h0 = h0.detach().to(dev, torch.float32).contiguous()
-                    c0 = c0.detach().to(dev, torch.float32).contiguous()
-                    if tuple(h0.shape) != (layers * 2, n, hid) or tuple(c0.shape) != (layers * 2, n, hid):
-                        raise RuntimeError("init_hidden returned shape %s, expected %s"
-                                           % (tuple(h0.shape), (layers * 2, n, hid)))
-                    keep += [h0, c0]
-                    ptrs[2 * g], ptrs[2 * g + 1] = h0.data_ptr(), c0.data_ptr()
-                states_arg = ptrs
+            states_arg, keep = self._init_hidden_states(n, dev) if self._uses_init_hidden() else (None, [])
             logits = torch.empty((n, self.num_classes), dtype=torch.float32, device=dev)
             probs = torch.empty((n, self.num_classes), dtype=torch.float32, device=dev)
             labels = torch.empty((n,), dtype=torch.int32, device=dev)
@@ -244,6 +281,33 @@ class ModelBiLSTM(nn.Module):
                 t.record_stream(torch.cuda.current_stream(dev))
         self.last_labels = labels
         return logits, probs
+
+    def _forward_train(self, kmer, base_means, base_stds, base_signal_lens, signals):
+        dev = self._param_device()
+        if dev.type != "cuda":
+            raise RuntimeError("ModelBiLSTM parameters are on %s; move the model to a CUDA device "
+                               "(.cuda(device)) -- this implementation has no CPU fallback" % dev)
+        T, S = self.seq_len, self.signal_len
+        has_seq = self.module != "signal_bilstm"
+        has_sig = self.module != "seq_bilstm"
+        inputs = (self._prep(kmer, dev, (-1, T)) if has_seq else None,
+                  self._prep(base_means, dev, (-1, T)) if has_seq else None,
+                  self._prep(base_stds, dev, (-1, T)) if has_seq else None,
+                  self._prep(base_signal_lens, dev, (-1, T)) if has_seq else None,
+                  self._prep(signals, dev, (-1, T, S)) if has_sig else None)
+        n = (inputs[0] if has_seq else inputs[4]).shape[0]
+        with torch.cuda.device(dev):
+            handle = self._create_handle(dev)
+            states_arg, keep = self._init_hidden_states(n, dev) if self._uses_init_hidden() else (None, [])
+            masks = self.draw_dropout_masks(n, dev)
+            self.last_dropout_masks = masks
+            self._calls += 1
+            params = [p for p in self.state_dict(keep_vars=True).values()]
+            for p in params:
+                if p.dtype != torch.float32 or not p.is_contiguous():
+                    raise RuntimeError("training needs contiguous float32 parameters")
+            logits = _TrainStep.apply(handle, inputs, states_arg, keep, masks, (self.seed << 20) + self._calls, *params)
+        return logits, torch.softmax(logits, 1)
 
     # ---- host-buffer entry (the FloatTensor/.cpu() boundary of _call_mods) ---------------
     def forward_host(self, kmer, base_means, base_stds, base_signal_lens, signals):
@@ -320,3 +384,47 @@ class ModelBiLSTM(nn.Module):
 
     def launch_count(self):
         return int(_native.lib().dsp_launch_count(self._handle)) if self._handle else 0
+
+
+def _ptr_array(tensors):
+    arr = (C.c_void_p * max(1, len(tensors)))()
+    for i, t in enumerate(tensors):
+        arr[i] = None if t is None else t.data_ptr()
+    return arr
+
+
+class _TrainStep(torch.autograd.Function):
+    """logits = ModelBiLSTM forward in train() mode on the fp32 training kernels; backward hands dlogits to
+    ``dsp_train_backward``.  The activation arena is a torch tensor kept in the context, so several forwards
+    may precede one backward and the memory returns to torch's allocator with the graph."""
+
+    @staticmethod
+    def forward(ctx, handle, inputs, states_arg, keep, masks, seed, *params):
+        L = _native.lib()
+        n = (inputs[0] if inputs[0] is not None else inputs[4]).shape[0]
+        dev = params[0].device
+        C_ = params[-1].shape[0]
+        arena = torch.empty(int(L.dsp_train_arena_bytes(handle, n)), dtype=torch.uint8, device=dev)
+        logits = torch.empty((n, C_), dtype=torch.float32, device=dev)
+        pp, mp = _ptr_array(params), _ptr_array(masks)
+        ptr = lambda t: None if t is None else t.data_ptr()
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _native.check(L.dsp_train_forward(handle, pp, len(params), *(ptr(t) for t in inputs), states_arg, seed, mp, n,
+                                          arena.data_ptr(), logits.data_ptr(), stream), "dsp_train_forward")
+        ctx.handle, ctx.n, ctx.arena, ctx.masks = handle, n, arena, masks
+        ctx.save_for_backward(*params)
+        return logits
+
+    @staticmethod
+    def backward(ctx, dlogits):
+        L = _native.lib()
+        params = ctx.saved_tensors
+        dev = params[0].device
+        dlogits = dlogits.to(torch.float32).contiguous()
+        ws = torch.empty(int(L.dsp_train_workspace_bytes(ctx.handle, ctx.n)), dtype=torch.uint8, device=dev)
+        grads = [torch.empty_like(p) for p in params]
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _native.check(L.dsp_train_backward(ctx.handle, _ptr_array(params), len(params), _ptr_array(ctx.masks),
+                                           ctx.arena.data_ptr(), dlogits.data_ptr(), ctx.n, ws.data_ptr(),
+                                           _ptr_array(grads), stream), "dsp_train_backward")
+        return (None,) * 6 + tuple(grads)

@@ -128,6 +128,50 @@ int dsp_forward_host_submit(dsp_handle h,
                             float* logits, float* probs, int32_t* labels, int64_t* ticket);
 int dsp_forward_host_wait(dsp_handle h, int64_t ticket);
 
+/* ---- training (train.py:104-128: model.train(), forward, loss.backward()) ------------------------
+ * fp32 on the CUDA cores whatever cfg->precision says; the handle contributes its configuration only
+ * (no dsp_set_param / dsp_pack_weights needed).  All pointers are DEVICE pointers; work is enqueued on
+ * `stream`; nothing is allocated inside forward or backward.
+ *
+ * params: the module's parameters in state_dict order (models.py:131-161): embed.weight (unless
+ *   signal_bilstm), lstm_seq.{weight_ih,weight_hh,bias_ih,bias_hh}_l{k}[_reverse] per layer, fc_seq.{weight,bias},
+ *   the same for lstm_signal / fc_signal, lstm_comb, fc1, fc2 -- torch's row-major float32 layouts.
+ *   dsp_train_shape gives their count and the number of dropout-mask slots.
+ * dropout_masks: n_masks slots, each NULL (no dropout there) or a float32 tensor holding keep / (1 - p):
+ *   slots [0, L2-1): lstm_seq inter-layer (n, seq_len, 2*nhid_seq) after layer l;  [L2-1, 2(L2-1)):
+ *   lstm_signal likewise;  then L1-1 slots of lstm_comb (n, seq_len, 2*hidden);  then the head:
+ *   (n, 2*hidden) before fc1 and (n, hidden) after fc1 (models.py:234-237).  L1 = num_layers1,
+ *   L2 = num_layers2.  Backward must get the same masks as the forward whose arena it reads.
+ * states: as for dsp_forward (6 pointers or NULL = Philox from `seed`); they are copied into the arena.
+ *
+ * Arena (saved activations of one forward, read by its backward; sections 256-byte aligned), per
+ * LSTM stack of `layers` layers, hidden H, first-layer input K0:
+ *   h0, c0: layers*2*n*H floats each; per layer l: y (n*T*2H), dropout output (n*T*2H, all but the last
+ *   layer), gates i,f,g,o (n*T*8H), cell states (n*T*2H), the layer's weights in the forward kernel's
+ *   layout 2 * ((ru(K,4) + ru(H,4))*4H + 4H) with K = K0 for l = 0, 2H otherwise;
+ * then xseq (n*T*kseq) + kmer codes (n*T int32) when the module has the seq branch, signals (n*T*S)
+ * when it has the signal branch, comb input (n*T*hidden), head: dropout(last states) (n*2*hidden),
+ * fc1 output (n*hidden), relu(dropout(fc1)) (n*hidden).  dsp_train_arena_bytes returns the total:
+ * for both_bilstm 13 x 16, hidden 256, 3 + 1 layers about 0.73 MB per site plus 19 MB of weights.
+ * The workspace of dsp_train_backward is scratch only (dsp_train_workspace_bytes; ~0.3 MB per site for
+ * the same model plus the split-K partial sums).
+ *
+ * dsp_train_forward writes logits (n, num_classes).  dsp_train_backward takes dlogits (n, num_classes),
+ * the gradient of the loss w.r.t. the logits, and WRITES (does not add) every parameter's gradient to
+ * grads[i] (same order and shapes as params; bias_ih and bias_hh receive the same values).  Sums over
+ * sites use a fixed split and order: repeating a backward gives bit-identical gradients. */
+int dsp_train_shape(dsp_handle h, int32_t* n_params, int32_t* n_masks);
+int64_t dsp_train_arena_bytes(dsp_handle h, int64_t n);
+int64_t dsp_train_workspace_bytes(dsp_handle h, int64_t n);
+int dsp_train_forward(dsp_handle h, const float* const* params, int32_t n_params,
+                      const float* kmer, const float* base_means, const float* base_stds,
+                      const float* base_signal_lens, const float* signals,
+                      const float* const* states, uint64_t seed, const float* const* dropout_masks,
+                      int64_t n, void* arena, float* logits, void* stream);
+int dsp_train_backward(dsp_handle h, const float* const* params, int32_t n_params,
+                       const float* const* dropout_masks, const void* arena, const float* dlogits,
+                       int64_t n, void* workspace, float* const* grads, void* stream);
+
 /* Number of kernels this library launched on behalf of `h` since creation. */
 int64_t dsp_launch_count(dsp_handle h);
 /* Milliseconds (CUDA events on the launching stream) spent in kernels of class `which`
