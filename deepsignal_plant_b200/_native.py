@@ -20,7 +20,7 @@ SYMBOLS = (
     "dsp_parse_features", "dsp_format_calls", "dsp_freq_release_cache", "dsp_extract_features", "dsp_format_sampleinfo", "dsp_find_sites", "dsp_extract_features_f64",
     "dsp_format_features", "dsp_parse_calls", "dsp_format_freq",
     "dsp_comm_create", "dsp_comm_export", "dsp_comm_connect", "dsp_comm_destroy", "dsp_freq_aggregate_distributed",
-    "dsp_comm_route_rows", "dsp_comm_last_timing", "dsp_freq_aggregate_host", "dsp_device_warmup",
+    "dsp_comm_route_rows", "dsp_comm_last_timing", "dsp_comm_allreduce_f32", "dsp_freq_aggregate_host", "dsp_device_warmup",
     "dsp_train_shape", "dsp_train_arena_bytes", "dsp_train_workspace_bytes", "dsp_train_forward", "dsp_train_backward",
 )
 
@@ -104,6 +104,7 @@ def lib():
                                                  C.POINTER(i64), C.POINTER(i64), vp, vp]
     L.dsp_comm_route_rows.argtypes = [vp, vp, i64, i32, i32, vp, vp, i64, C.POINTER(i64), vp]
     L.dsp_comm_last_timing.argtypes = [vp, vp]
+    L.dsp_comm_allreduce_f32.argtypes = [vp, C.POINTER(vp), C.POINTER(i64), C.c_int32, vp]
     L.dsp_train_shape.argtypes = [vp, C.POINTER(i32), C.POINTER(i32)]
     L.dsp_train_arena_bytes.argtypes = [vp, i64]
     L.dsp_train_arena_bytes.restype = i64

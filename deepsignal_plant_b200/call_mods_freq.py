@@ -807,22 +807,9 @@ def call_mods_frequency_to_file(args):
     contigs = parse_contigs_arg(getattr(args, "contigs", None))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world > 1:
-        import torch
         import torch.distributed as dist
         from . import freq_dist
-        local = int(os.environ.get("LOCAL_RANK", "0"))
-        ndev = torch.cuda.device_count()
-        if ndev == 0:
-            raise RuntimeError("call_freq aggregation needs a CUDA device; there is no CPU path")
-        if not dist.is_initialized():
-            # one GPU per rank: NCCL carries the (tiny) control plane; ranks sharing a GPU fall back to gloo for it --
-            # the records travel through CUDA IPC windows either way
-            if ndev >= world:
-                dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-            else:
-                dist.init_process_group("gloo")
-        device = local % ndev
-        torch.cuda.set_device(device)
+        device = freq_dist.join_torchrun("call_freq aggregation")
         print("read the input files..")
         table, considered, path = freq_dist.call_freq_distributed(sorted(mods_files) if getattr(args, "sort_files", False) else mods_files,
                                                                   args.prob_cf, args.result_file, args.sort, args.bed, args.gzip,

@@ -11,10 +11,12 @@ reference's flag names and defaults.
     python -m deepsignal_plant_b200 pack_features -i features.tsv -o features.dspf             # an existing text file -> binary
     python -m deepsignal_plant_b200 train --train_file train.dspf --valid_file valid.dspf --model_dir models/
 
-Multi-GPU: launch ``call_mods`` or ``call_freq`` under torchrun, one process per GPU.  ``call_mods`` cuts the feature
-file (or the reads archive) into contiguous shards and concatenates the output in file order, no collective on the
-data path; ``call_freq`` parses contiguous byte shards, exchanges the records by site key over NVLink peer memory and
-every rank writes its slice of the table (freq_dist.py).  ``extract`` here takes reads that are already decoded
+Multi-GPU: launch ``call_mods``, ``call_freq`` or ``train`` under torchrun, one process per GPU.  ``call_mods`` cuts the
+feature file (or the reads archive) into contiguous shards and concatenates the output in file order, no collective on
+the data path; ``call_freq`` parses contiguous byte shards, exchanges the records by site key over NVLink peer memory and
+every rank writes its slice of the table (freq_dist.py); ``train`` keeps ``--batch_size`` as the global batch, every
+rank trains on a slice of each step and the gradients are summed by a deterministic all-reduce over NVLink peer
+memory, so the replicas stay bit-identical and rank 0 writes the checkpoints (train_dist.py).  ``extract`` here takes reads that are already decoded
 (reading fast5 needs h5py: outside this implementation); ``train`` runs the reference's training loop on the fp32 training kernels (train.py); ``denoise`` stays with the
 reference."""
 from __future__ import annotations

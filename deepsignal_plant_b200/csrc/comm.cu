@@ -1,5 +1,6 @@
 // Multi-GPU call_freq: the one exchange step of the path (SURVEY.md 8(e)), as kernels over NVLink
-// peer memory instead of a library all-to-all.
+// peer memory instead of a library all-to-all.  The same windows also carry the deterministic gradient
+// all-reduce of multi-GPU training (dsp_comm_allreduce_f32, below the splitters).
 //
 // One process per GPU.  Every rank owns two receive WINDOWS and a small control block in device
 // memory, exported to the other ranks of the box with CUDA IPC (dsp_comm_export / _connect), so a
@@ -22,7 +23,9 @@
 #include "freq.cuh"
 #include "route.cuh"
 #include <unistd.h>
+#include <algorithm>
 #include <cstring>
+#include <vector>
 
 namespace dsp {
 
@@ -40,6 +43,7 @@ struct Ctrl {                                   // device memory; peers write, t
     uint64_t samples[2][MAXW][256];             // splitter selection: every rank's sample of its rows' sort field
     int32_t nsamples[2][MAXW];
     unsigned long long flag_smp[MAXW];
+    unsigned long long flag_ar[2][MAXW];         // all-reduce: [0] slots of source landed here, [1] its summed range landed here
 };
 constexpr int NSAMP = 256;
 
@@ -181,6 +185,131 @@ __global__ void __launch_bounds__(1024) splitters_kernel(const Ctrl* local, int 
         bounds[t] = v;
     }
     if (t == 0 && s_bad) res->err = s_bad;
+}
+
+// ---- deterministic fp32 all-reduce of a tensor list (dsp_comm_allreduce_f32) -------------------------------------
+// The list is one flat vector of E floats, the tensors back to back in argument order.  Rank r owns the range
+// [r * chunk, min(E, (r + 1) * chunk)), chunk = ceil(E / world) rounded up to a multiple of 4 (16-byte aligned).
+//   pack:          every rank stores the part of its vector that rank r owns into slot [me] of r's window 0
+//   signal + wait  on flag_ar[0]
+//   reduce:        the owner adds its world slots in rank order, fl(fl(s0 + s1) + s2)..., and stores the sums into
+//                  every rank's window 1 at the range's offset
+//   signal + wait  on flag_ar[1]
+//   unpack:        window 1 -> the tensors
+// One rank computes each element, with plain adds in a fixed order, so every rank gets the same bits on every call,
+// whatever the chunking and timing.  The kernels that move data never spin; only the one-warp signal kernels wait,
+// so ranks that share a GPU make progress under time-slicing.
+//
+// No window is overwritten while a peer may still read it:
+// * slot writes of call k+1 into owner r's window 0, against r's reduction of call k: a rank packs call k+1 only after
+//   its call-k wait on flag_ar[1] saw every rank's flag, and r raises that flag in the kernel after its reduction, so
+//   r has finished reading window 0 for call k.
+// * window-1 writes of call k+1 by owner r into rank p's window 1, against p's unpack of call k: r reduces call k+1
+//   only after its wait on flag_ar[0] saw p's flag of call k+1, which p raises after its pack of call k+1, and p's
+//   stream runs that pack after its unpack of call k.
+constexpr int AR_MAXT = 64;                     // tensors per pack / unpack launch (kernel parameter space)
+constexpr int AR_THREADS = 256;
+
+struct ArList {
+    float* ptr[AR_MAXT];
+    int64_t off[AR_MAXT + 1];                   // flat offsets of the tensors; off[count] = end of the group
+    int count;
+};
+
+__host__ __device__ __forceinline__ int64_t ar_chunk(int64_t e, int world) { return ((e + world - 1) / world + 3) & ~(int64_t)3; }
+
+// the tensor that holds flat index j: the last one starting at or before j (empty tensors share their successor's start)
+__device__ __forceinline__ int ar_find(const int64_t* off, int count, int64_t j) {
+    int lo = 0, hi = count - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (off[mid] <= j) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(AR_THREADS) allreduce_pack_kernel(ArList l, Windows win0, int me, int64_t chunk) {
+    __shared__ float* s_ptr[AR_MAXT];
+    __shared__ int64_t s_off[AR_MAXT + 1];
+    __shared__ float* s_win[MAXW];               // tables indexed at run time: shared memory, not a stack copy of the parameters
+    for (int i = threadIdx.x; i <= l.count; i += AR_THREADS) {
+        s_off[i] = l.off[i];
+        if (i < l.count) s_ptr[i] = l.ptr[i];
+    }
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int r = 0; r < MAXW; ++r) s_win[r] = static_cast<float*>(win0.win[r]);
+    }
+    __syncthreads();
+    const int64_t base = s_off[0], n = s_off[l.count] - base;
+    for (int64_t i = (int64_t)blockIdx.x * AR_THREADS + threadIdx.x; i < n; i += (int64_t)gridDim.x * AR_THREADS) {
+        const int64_t j = base + i;
+        const int t = ar_find(s_off, l.count, j);
+        const float v = s_ptr[t][j - s_off[t]];
+        const int64_t r = j / chunk;
+        s_win[r][me * chunk + (j - r * chunk)] = v;
+    }
+}
+
+__global__ void __launch_bounds__(AR_THREADS) allreduce_reduce_kernel(const float* __restrict__ slots, Windows win1, int world,
+                                                                      int64_t chunk, int64_t lo, int64_t len,
+                                                                      const int* __restrict__ abort_flag) {
+    __shared__ float* s_win[MAXW];
+    if (*abort_flag) return;
+    if (threadIdx.x == 0) {
+#pragma unroll
+        for (int r = 0; r < MAXW; ++r) s_win[r] = static_cast<float*>(win1.win[r]);
+    }
+    __syncthreads();
+    const int64_t nv = len >> 2, stride = (int64_t)gridDim.x * AR_THREADS;
+    for (int64_t v = (int64_t)blockIdx.x * AR_THREADS + threadIdx.x; v < nv; v += stride) {
+        float4 a = reinterpret_cast<const float4*>(slots)[v];
+        for (int s = 1; s < world; ++s) {
+            const float4 b = reinterpret_cast<const float4*>(slots + s * chunk)[v];
+            a.x = __fadd_rn(a.x, b.x); a.y = __fadd_rn(a.y, b.y); a.z = __fadd_rn(a.z, b.z); a.w = __fadd_rn(a.w, b.w);
+        }
+        for (int p = 0; p < world; ++p) reinterpret_cast<float4*>(s_win[p] + lo)[v] = a;
+    }
+    if (blockIdx.x == 0 && threadIdx.x < (len & 3)) {                  // the last range may end off a multiple of 4
+        const int64_t i = (nv << 2) + threadIdx.x;
+        float a = slots[i];
+        for (int s = 1; s < world; ++s) a = __fadd_rn(a, slots[s * chunk + i]);
+        for (int p = 0; p < world; ++p) s_win[p][lo + i] = a;
+    }
+}
+
+__global__ void __launch_bounds__(AR_THREADS) allreduce_unpack_kernel(ArList l, const float* __restrict__ win1,
+                                                                      const int* __restrict__ abort_flag) {
+    __shared__ float* s_ptr[AR_MAXT];
+    __shared__ int64_t s_off[AR_MAXT + 1];
+    if (*abort_flag) return;
+    for (int i = threadIdx.x; i <= l.count; i += AR_THREADS) {
+        s_off[i] = l.off[i];
+        if (i < l.count) s_ptr[i] = l.ptr[i];
+    }
+    __syncthreads();
+    const int64_t base = s_off[0], n = s_off[l.count] - base;
+    for (int64_t i = (int64_t)blockIdx.x * AR_THREADS + threadIdx.x; i < n; i += (int64_t)gridDim.x * AR_THREADS) {
+        const int64_t j = base + i;
+        const int t = ar_find(s_off, l.count, j);
+        s_ptr[t][j - s_off[t]] = win1[j];
+    }
+}
+
+// One warp: "my stores of this phase have landed" to every peer, then wait for every peer's.  After a time-out the
+// rank raises no further flag, so its peers time out too instead of unpacking a range that was never summed.
+__global__ void allreduce_signal_wait_kernel(Ctrl* local, Peers peers, int me, int world, int phase, unsigned long long epoch,
+                                             int* abort_flag, Result* res) {
+    const int t = threadIdx.x;
+    if (*reinterpret_cast<volatile int*>(abort_flag)) return;
+    __threadfence_system();                      // the previous kernel's peer stores before the flag
+    if (t < world) *reinterpret_cast<volatile unsigned long long*>(&peers.ctrl[t]->flag_ar[phase][me]) = epoch;
+    const bool ok = t >= world || wait_flag(&local->flag_ar[phase][t], epoch);
+    __threadfence_system();
+    if (!__all_sync(0xffffffffu, ok) && t == 0) {
+        res->err |= 2;
+        *abort_flag = 1;
+    }
 }
 
 }  // namespace
@@ -491,6 +620,60 @@ int dsp_freq_aggregate_distributed(dsp_comm c, const uint64_t* key, const double
     DSP_CUDA(cudaEventRecord(c->ev[4], st));
     DSP_CUDA(cudaStreamSynchronize(st));
     for (int i = 0; i < 4; ++i) cudaEventElapsedTime(&c->last_ms[i], c->ev[i], c->ev[i + 1]);
+    return DSP_OK;
+}
+
+int dsp_comm_allreduce_f32(dsp_comm c, float* const* bufs, const int64_t* numel, int32_t n_bufs, void* stream) {
+    DSP_REQUIRE(n_bufs >= 0, DSP_ERR_INVALID, "dsp_comm_allreduce_f32: n_bufs=%d", (int)n_bufs);
+    DSP_REQUIRE(n_bufs == 0 || (bufs && numel), DSP_ERR_INVALID, "dsp_comm_allreduce_f32: null buffer or size list");
+    int64_t e = 0;
+    for (int32_t i = 0; i < n_bufs; ++i) {
+        DSP_REQUIRE(numel[i] >= 0 && numel[i] <= ((int64_t)1 << 40) - e, DSP_ERR_INVALID,
+                    "dsp_comm_allreduce_f32: numel[%d]=%lld out of range", (int)i, (long long)numel[i]);
+        DSP_REQUIRE(numel[i] == 0 || bufs[i], DSP_ERR_INVALID, "dsp_comm_allreduce_f32: bufs[%d] is null", (int)i);
+        e += numel[i];
+    }
+    DSP_REQUIRE(c, DSP_ERR_INVALID, "dsp_comm_allreduce_f32: null communicator");
+    DSP_REQUIRE(c->connected, DSP_ERR_STATE, "dsp_comm_allreduce_f32: not connected (dsp_comm_connect after exchanging the export blobs)");
+    const int world = c->world, me = c->rank;
+    const int64_t chunk = ar_chunk(e, world);
+    DSP_REQUIRE(chunk * world * 4 <= c->window_bytes, DSP_ERR_NOMEM,
+                "dsp_comm_allreduce_f32: %lld floats need windows of %lld bytes, the communicator has %lld",
+                (long long)e, (long long)(chunk * world * 4), (long long)c->window_bytes);
+    if (e == 0 || world == 1) return DSP_OK;
+    DevGuard g(c->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned long long epoch = ++c->epoch;
+    Peers peers{}; Windows w0{}, w1{};
+    for (int r = 0; r < world; ++r) { peers.ctrl[r] = c->peer_ctrl[r]; w0.win[r] = c->peer_win[0][r]; w1.win[r] = c->peer_win[1][r]; }
+    auto blocks = [&](int64_t items, int per_sm) { return (int)std::max<int64_t>(1, std::min<int64_t>((items + AR_THREADS - 1) / AR_THREADS, (int64_t)c->n_sm * per_sm)); };
+    DSP_CUDA(cudaMemsetAsync(c->d_abort, 0, sizeof(int), st));
+    DSP_CUDA(cudaMemsetAsync(c->d_res, 0, sizeof(Result), st));
+    std::vector<ArList> groups;
+    int64_t o = 0;
+    for (int32_t i0 = 0; i0 < n_bufs; i0 += AR_MAXT) {
+        ArList l{};
+        l.count = std::min<int32_t>(AR_MAXT, n_bufs - i0);
+        for (int k = 0; k < l.count; ++k) { l.ptr[k] = bufs[i0 + k]; l.off[k] = o; o += numel[i0 + k]; }
+        l.off[l.count] = o;
+        groups.push_back(l);
+    }
+    for (const ArList& l : groups)
+        if (l.off[l.count] > l.off[0]) allreduce_pack_kernel<<<blocks(l.off[l.count] - l.off[0], 8), AR_THREADS, 0, st>>>(l, w0, me, chunk);
+    allreduce_signal_wait_kernel<<<1, 32, 0, st>>>(c->ctrl, peers, me, world, 0, epoch, c->d_abort, c->d_res);
+    const int64_t lo = std::min<int64_t>(e, me * chunk), len = std::min<int64_t>(e, lo + chunk) - lo;
+    if (len > 0)
+        allreduce_reduce_kernel<<<blocks(len / 4 + 1, 4), AR_THREADS, 0, st>>>(static_cast<const float*>(c->win[0]), w1, world, chunk,
+                                                                                 lo, len, c->d_abort);
+    allreduce_signal_wait_kernel<<<1, 32, 0, st>>>(c->ctrl, peers, me, world, 1, epoch, c->d_abort, c->d_res);
+    for (const ArList& l : groups)
+        if (l.off[l.count] > l.off[0])
+            allreduce_unpack_kernel<<<blocks(l.off[l.count] - l.off[0], 8), AR_THREADS, 0, st>>>(l, static_cast<const float*>(c->win[1]),
+                                                                                               c->d_abort);
+    DSP_CUDA(cudaGetLastError());
+    DSP_CUDA(cudaMemcpyAsync(c->h_res, c->d_res, sizeof(Result), cudaMemcpyDeviceToHost, st));
+    DSP_CUDA(cudaStreamSynchronize(st));
+    DSP_REQUIRE(!(c->h_res->err & 2), DSP_ERR_CUDA, "dsp_comm_allreduce_f32: rank %d timed out waiting for a peer (call %llu)", me, epoch);
     return DSP_OK;
 }
 

@@ -82,6 +82,28 @@ def read_units(units):
 
 
 # ---- device backend ----------------------------------------------------------------------------------
+def open_comm(rank, world, device, window_bytes, all_gather_object):
+    """A connected ``dsp_comm`` handle on ``device`` with two windows of ``window_bytes``: create, export, gather the
+    blobs of all ranks through ``all_gather_object`` (collective), connect."""
+    import torch
+    L = _native.lib()
+    h = C.c_void_p()
+    with torch.cuda.device(torch.device("cuda", device)):
+        _native.check(L.dsp_comm_create(C.byref(h), device, rank, world, int(window_bytes)), "dsp_comm_create")
+        try:
+            blob = np.zeros(512, np.uint8)
+            nb = C.c_int64(0)
+            _native.check(L.dsp_comm_export(h, blob.ctypes.data, blob.size, C.byref(nb)), "dsp_comm_export")
+            blobs = all_gather_object(blob[:nb.value].tobytes())
+            if world > 1:
+                joined = np.frombuffer(b"".join(blobs), np.uint8).copy()
+                _native.check(L.dsp_comm_connect(h, joined.ctypes.data, nb.value), "dsp_comm_connect")
+        except BaseException:
+            L.dsp_comm_destroy(h)
+            raise
+    return h
+
+
 class DeviceBackend:
     """``dsp_comm_*`` / ``dsp_freq_aggregate_distributed`` behind the two calls the driver needs."""
 
@@ -95,15 +117,7 @@ class DeviceBackend:
         self.L = _native.lib()
         self.h = C.c_void_p()
         self.window_bytes = int(window_bytes)
-        with torch.cuda.device(self.dev):
-            _native.check(self.L.dsp_comm_create(C.byref(self.h), device, rank, world, self.window_bytes), "dsp_comm_create")
-            blob = np.zeros(512, np.uint8)
-            nb = C.c_int64(0)
-            _native.check(self.L.dsp_comm_export(self.h, blob.ctypes.data, blob.size, C.byref(nb)), "dsp_comm_export")
-            blobs = all_gather_object(blob[:nb.value].tobytes())
-            if world > 1:
-                joined = np.frombuffer(b"".join(blobs), np.uint8).copy()
-                _native.check(self.L.dsp_comm_connect(self.h, joined.ctypes.data, nb.value), "dsp_comm_connect")
+        self.h = open_comm(rank, world, device, self.window_bytes, all_gather_object)
 
     def close(self):
         if self.h:
@@ -173,6 +187,27 @@ class DeviceBackend:
 
 
 # ---- control plane ------------------------------------------------------------------------------------
+def join_torchrun(what):
+    """Under torchrun: join the default process group (if not yet joined), make this rank's GPU (LOCAL_RANK modulo the
+    device count) current and return its index.  One GPU per rank: NCCL carries the (tiny) control plane; ranks sharing a
+    GPU fall back to gloo for it -- the bulk data travels through CUDA IPC windows either way."""
+    import torch
+    import torch.distributed as dist
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    local = int(os.environ.get("LOCAL_RANK", "0"))
+    ndev = torch.cuda.device_count()
+    if ndev == 0:
+        raise RuntimeError("%s needs a CUDA device; there is no CPU path" % what)
+    if not dist.is_initialized():
+        if ndev >= world:
+            dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+        else:
+            dist.init_process_group("gloo")
+    device = local % ndev
+    torch.cuda.set_device(device)
+    return device
+
+
 class TorchGroup:
     """The few small collectives of the control plane, on ``torch.distributed`` (any backend)."""
 

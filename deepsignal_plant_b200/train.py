@@ -14,7 +14,10 @@ Loop, as the reference runs it:
 Data: the training and validation sets (``.dspf`` or the 12-column text feature file) are read once and
 kept on the device (1 040 B per site for 13 x 16, plus the label); each epoch draws its order with
 ``torch.randperm`` from a CPU generator seeded with ``--tseed``, and every step gathers its batch on
-the device.  A set that does not fit in free device memory is refused; there is no streaming."""
+the device.  A set that does not fit in free device memory is refused; there is no streaming.
+
+Under torchrun (WORLD_SIZE > 1) the same loop runs on every rank's GPU with a deterministic gradient all-reduce
+(train_dist.py)."""
 from __future__ import annotations
 
 import os
@@ -103,11 +106,12 @@ def evaluate(model, data, criterion, batch_size):
     return float(np.mean(losses)), correct / n
 
 
-def build_model(args, dev):
+def build_model(args, dev, seed=0):
+    """``seed``: the module's Philox seed for the initial LSTM states (one per rank under torchrun)."""
     from .models import ModelBiLSTM
     model = ModelBiLSTM(args.seq_len, args.signal_len, args.layernum1, args.layernum2, args.class_num,
                         args.dropout_rate, args.hid_rnn, args.n_vocab, args.n_embed, str2bool(args.is_base),
-                        str2bool(args.is_signallen), args.model_type, device=dev.index, trainable=True)
+                        str2bool(args.is_signallen), args.model_type, device=dev.index, seed=seed, trainable=True)
     if args.init_model is not None:
         para = torch.load(args.init_model, map_location=torch.device("cpu"))
         d = model.state_dict()
@@ -117,6 +121,9 @@ def build_model(args, dev):
 
 
 def train(args, log=print):
+    if int(os.environ.get("WORLD_SIZE", "1")) > 1:          # torchrun: one process per GPU (train_dist.py)
+        from .train_dist import train_distributed
+        return train_distributed(args, log)
     if not torch.cuda.is_available():
         raise RuntimeError("train needs a CUDA device; this implementation has no CPU path")
     t0 = time.time()

@@ -272,6 +272,18 @@ int dsp_comm_route_rows(dsp_comm c, const void* rows, int64_t n, int32_t row_byt
  * waiting for every rank's stores. */
 int dsp_comm_last_timing(dsp_comm c, float* ms12);
 
+/* ---- multi-GPU training: deterministic gradient all-reduce --------------------------------------------------
+ * Sums n_bufs float32 DEVICE buffers (bufs[i] holds numel[i] floats; HOST arrays of pointers and sizes) in place
+ * across the ranks of `c`: on return element i of every rank's list holds fl(...fl(fl(g0_i + g1_i) + g2_i)... +
+ * g{w-1}_i), the float32 sum in rank order -- the same bits on every rank, on every call, however the work is
+ * chunked or timed.  The list is one flat vector of E = sum(numel) floats: a reduce-scatter (rank r sums the 16-byte
+ * aligned range [r * chunk, (r + 1) * chunk), chunk = ceil(E / world) rounded up to a multiple of 4) followed by an
+ * all-gather, both through the communicator's windows.  Every rank passes the same numel list (collective
+ * semantics).  Needs window_bytes >= 4 * world * chunk; otherwise DSP_ERR_NOMEM before anything is launched, and
+ * negative sizes or a null buffer of non-zero size give DSP_ERR_INVALID.  A peer that never arrives fails after
+ * 30 s with DSP_ERR_CUDA on every rank.  Synchronises `stream`. */
+int dsp_comm_allreduce_f32(dsp_comm c, float* const* bufs, const int64_t* numel, int32_t n_bufs, void* stream);
+
 /* dsp_parse_calls: ModRecord.__init__ (utils/txt_formater.py:8-21) for a whole call_mods file held in memory
  * (HOST pointers): every line is strip()-ed and split on tabs; columns 1, 3, 8 are parsed like int(), 6 and 7
  * like float() (correctly rounded to float64), chromosome names (column 0) are interned -- chrom_code[i] indexes
