@@ -120,13 +120,18 @@ struct LayerParams {
 
 enum { MODE_LSTM = 0, MODE_FC = 1, MODE_HEAD = 2 };
 constexpr int HEAD_MAX_CLASSES = 8;
-// weight ring: NST stages of STG half slabs (one mbarrier pair per stage)
-template <int KSX, int MODE> struct RingCfg {
+template <int KSX, int H, int MODE, int NOUT> struct LayerCfg {
+    static constexpr int NCH = MODE != MODE_LSTM ? NOUT / 128 : H / 32;   // 128-column chunks per step
+    // weight ring: NST stages of STG half slabs (one mbarrier pair per stage)
     static constexpr int STG = KSX >= 8 ? 2 : 4;
     static constexpr int NST = KSX >= 8 ? (MODE == 2 ? 4 : 5) : (MODE == 1 ? 2 : 4);
     // x_t buffers: the per-timestep dense layers are HBM-bound streams of x_t, so where shared memory allows
     // they double-buffer it (load of step t+1 overlaps the MMAs and stores of step t)
     static constexpr int XB = (MODE == 1 && KSX <= 4) ? 2 : 1;
+    // dynamic shared memory, as offsets from its 1 KB-aligned base: XB x KSX x_t slabs at 0, the ring, the biases
+    static constexpr size_t W = (size_t)KSX * XB * SLAB_BYTES;
+    static constexpr size_t BIAS = W + (size_t)NST * STG * HSLAB_BYTES;
+    static constexpr size_t BYTES = BIAS + (size_t)NCH * 128 * sizeof(float) + 1024;     // + the alignment slack
 };
 
 // Philox4x32-10 (Salmon et al., SC'11) + Box-Muller: four N(0,1) values per counter.  Used to
@@ -284,9 +289,10 @@ template <int KSX, int H, int MODE, int NOUT>
 __global__ void __launch_bounds__(NTHREADS, 1)
 layer_kernel(const LayerParams p) {
     constexpr bool IS_FC = MODE != MODE_LSTM;              // no recurrence: x part only
-    constexpr int STG = RingCfg<KSX, MODE>::STG, NST = RingCfg<KSX, MODE>::NST, XB = RingCfg<KSX, MODE>::XB;
+    using Cfg = LayerCfg<KSX, H, MODE, NOUT>;
+    constexpr int STG = Cfg::STG, NST = Cfg::NST, XB = Cfg::XB;
     constexpr int NXS = KSX * XB;                          // x slabs resident in shared memory
-    constexpr int NCH = IS_FC ? NOUT / 128 : H / 32;       // 128-column chunks per step
+    constexpr int NCH = Cfg::NCH;
     constexpr int KSH = IS_FC ? 0 : H / 64;                // h slabs (K of the recurrent part)
     constexpr int KS = KSX + KSH;
     constexpr int W_STEP = NCH * KS;                       // half slabs streamed per step
@@ -299,8 +305,8 @@ layer_kernel(const LayerParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     uint8_t* s_x = smem;                                   // NXS slabs
-    uint8_t* s_w = smem + (size_t)NXS * SLAB_BYTES;        // NST ring stages of STG half slabs
-    float* s_bias = reinterpret_cast<float*>(s_w + (size_t)NST * STG * HSLAB_BYTES);
+    uint8_t* s_w = smem + Cfg::W;                          // NST ring stages of STG half slabs
+    float* s_bias = reinterpret_cast<float*>(smem + Cfg::BIAS);
     __shared__ __align__(8) uint64_t bars[2 * NST + 2 * NXS + 5];
     __shared__ uint32_t tmem_base_s;
     const uint32_t b_wfull = smem_u32(&bars[0]), b_wempty = smem_u32(&bars[NST]);
@@ -739,42 +745,100 @@ layer_kernel(const LayerParams p) {
 // 8 epilogue warps per chain, one MMA issuer alternating between the chains.  Everything else
 // (CTA pair, half-operand staging, barrier protocol) is as in layer_kernel.
 constexpr int BR_H = 128, BR_NW = 64, BR_NCH = BR_H / 16, BR_KSH = BR_H / 64;
+constexpr int BR_KSX = 1;                                 // x slabs per step: only a branch's first layer (K <= 64) runs here
+constexpr int BR_YS = 2 * BR_H / 64;                      // slabs of a y row [h_fwd | h_bwd] (also the K of the fused fc)
 constexpr int QSLAB_BYTES = 32 * SLAB_ROW_BYTES;          // 4 KB: one CTA's share (32 rows) of a 64-column B slab
 constexpr int BR_STG = 4, BR_NST = 6;                     // ring: 6 stages of 16 KB
+constexpr int BR_PAIR_UNITS = 4 * BR_KSX + 4 * BR_KSH;    // X(0,c) X(0,c+1) X(1,c) X(1,c+1) H(0,c) H(0,c+1) H(1,c) H(1,c+1)
+constexpr int BR_W_STEP = (BR_NCH / 2) * BR_PAIR_UNITS;   // ring units streamed per step
+constexpr int BR_NBIAS = 2 * BR_NCH * BR_NW;
+static_assert(BR_W_STEP % BR_STG == 0, "a step must be a whole number of ring stages");
 
-template <int KSX>
-__global__ void __launch_bounds__(NTHREADS, 1)
-branch_kernel(const LayerParams p) {
-    constexpr int KS = KSX + BR_KSH;
-    constexpr int PAIR_UNITS = 4 * KSX + 4 * BR_KSH;      // X(0,c) X(0,c+1) X(1,c) X(1,c+1) H(0,c) H(0,c+1) H(1,c) H(1,c+1)
-    constexpr int W_STEP = (BR_NCH / 2) * PAIR_UNITS;     // ring units streamed per step
-    constexpr int NBIAS = 2 * BR_NCH * BR_NW;
+// Dynamic shared memory of the branch kernels, as offsets from its 1 KB-aligned base: x slabs [dir][BR_KSX] at 0,
+// the weight ring, the LSTM biases.  FC_TAIL adds the fc weights and biases, resident for the whole kernel, and
+// double-buffers y(t) over the x + ring space, which the recurrence has finished with by then.
+template <bool FC_TAIL> struct BranchSmem {
+    static constexpr size_t W = (size_t)2 * BR_KSX * SLAB_BYTES;
+    static constexpr size_t WFC = W + (size_t)BR_NST * BR_STG * QSLAB_BYTES;
+    static constexpr size_t BIAS = WFC + (FC_TAIL ? (size_t)BR_YS * HSLAB_BYTES : 0);
+    static constexpr size_t FCB = BIAS + (size_t)BR_NBIAS * sizeof(float);
+    static constexpr size_t BYTES = FCB + (FC_TAIL ? 128 * sizeof(float) : 0) + 1024;     // + the alignment slack
+    static_assert(!FC_TAIL || WFC == (size_t)2 * BR_YS * SLAB_BYTES, "tail A buffers alias x + ring exactly");
+};
+
+// One hidden-128 bidirectional layer, as the two-chain recurrence reads it.
+struct BranchLayer {
+    const uint8_t* x_img;      // [tiles][T][BR_KSX] slabs
+    const uint8_t* w_img;      // [cta rank][stream unit] quarter slabs (TcLstmPack::w_img_dual)
+    const float* bias;         // [dir][BR_NCH * 64] in chunk column order
+    const float* h0;           // [dir][n][128] fp32; null: draw N(0,1) in-kernel (Philox)
+    const float* c0;
+    int64_t state_dir_stride;
+    uint32_t rng_slot;         // state slot id of this layer, dir is added in-kernel
+    int xk16;
+    uint8_t* y_img;            // [tiles][T][BR_YS] slabs: [h_fwd | h_bwd] of every t
+    uint64_t seed;
+    uint32_t rng_call;
+    int64_t site_base;
+    int64_t n;
+    int T;
+};
+
+// The per-timestep dense layer branch_fused_kernel runs behind the recurrence: relu(y(t) W^T + b), N = 128.
+struct FcTail {
+    const uint8_t* w_img;      // [cta rank][BR_YS] half slabs (TcDensePack layout)
+    const float* bias;         // 128 floats
+    uint8_t* y_img;            // [tiles][T][4] slabs
+    int col0;                  // first column of y_img this layer writes
+};
+
+// The two-chain recurrence of one CTA pair, the body of both branch_kernel and branch_fused_kernel (the entry points
+// only pick the layer and the tile).  FC_TAIL adds the fc tail phase of branch_fused_kernel and nothing else: the fc
+// weight preload, the tail barriers and their relay, the y(t) read-back over the x + ring space, the fc MMAs and the
+// fence.proxy.async + relu epilogue.
+template <bool FC_TAIL>
+__device__ __forceinline__ void branch_body(const BranchLayer& L, const FcTail& fc, const int tile) {
+    using S = BranchSmem<FC_TAIL>;
     constexpr uint32_t IDESC = make_idesc_f16(256, BR_NW);
-    static_assert(W_STEP % BR_STG == 0 && KS * 2 == PAIR_UNITS / 2, "stream layout");
+    constexpr uint32_t IDESC_FC = make_idesc_f16(256, 128);
 
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    uint8_t* s_x = smem;                                   // [dir][KSX] slabs
-    uint8_t* s_w = smem + (size_t)2 * KSX * SLAB_BYTES;
-    float* s_bias = reinterpret_cast<float*>(s_w + (size_t)BR_NST * BR_STG * QSLAB_BYTES);
-    __shared__ __align__(8) uint64_t bars[2 * BR_NST + 4 * KSX + 10];
+    uint8_t* s_x = smem;                                   // [dir][BR_KSX] slabs          } recurrent phase
+    uint8_t* s_w = smem + S::W;                            // weight ring                  }
+    uint8_t* s_a = smem;                                   // tail: 2 x BR_YS slabs of y(t), aliasing the two above
+    uint8_t* s_wfc = smem + S::WFC;                        // tail: this CTA's half of the fc weights (BR_YS half slabs)
+    float* s_bias = reinterpret_cast<float*>(smem + S::BIAS);
+    float* s_fcb = reinterpret_cast<float*>(smem + S::FCB);
+    __shared__ __align__(8) uint64_t bars[2 * BR_NST + 4 * BR_KSX + 10 + (FC_TAIL ? 10 : 0)];
     __shared__ uint32_t tmem_base_s;
     const uint32_t b_wfull = smem_u32(&bars[0]), b_wempty = smem_u32(&bars[BR_NST]);
-    const uint32_t b_xfull = smem_u32(&bars[2 * BR_NST]), b_xempty = b_xfull + 8 * 2 * KSX;       // [dir][KSX]
-    const uint32_t b_accfull = b_xempty + 8 * 2 * KSX, b_accempty = b_accfull + 32;               // [dir][2]
+    const uint32_t b_xfull = smem_u32(&bars[2 * BR_NST]), b_xempty = b_xfull + 8 * 2 * BR_KSX;    // [dir][BR_KSX]
+    const uint32_t b_accfull = b_xempty + 8 * 2 * BR_KSX, b_accempty = b_accfull + 32;            // [dir][2]
     const uint32_t b_hready = b_accempty + 32;                                                  // [dir]
+    const uint32_t b_tail = b_hready + 16;                 // all epilogue warps of THIS CTA are past the last y store
+    const uint32_t b_wfc = b_tail + 8;                     // fc weights landed (both CTAs)
+    const uint32_t b_afull = b_wfc + 8, b_aempty = b_afull + 16;                                  // [2]
+    const uint32_t b_faccfull = b_aempty + 16, b_faccempty = b_faccfull + 16;                     // [2]
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int tile = blockIdx.x;
-    const int T = p.T;
+    const int T = L.T;
     const uint32_t crank = cluster_ctarank();
 
     if (tid == 0) {
         const uint32_t both = crank == 0 ? 2u : 1u;
         for (int i = 0; i < BR_NST; ++i) { mbar_init(b_wfull + 8 * i, both); mbar_init(b_wempty + 8 * i, 1); }
-        for (int i = 0; i < 2 * KSX; ++i) { mbar_init(b_xfull + 8 * i, both); mbar_init(b_xempty + 8 * i, 1); }
+        for (int i = 0; i < 2 * BR_KSX; ++i) { mbar_init(b_xfull + 8 * i, both); mbar_init(b_xempty + 8 * i, 1); }
         for (int i = 0; i < 4; ++i) { mbar_init(b_accfull + 8 * i, 1); mbar_init(b_accempty + 8 * i, EPI_WARPS); }   // 8 warps x 2 CTAs
         for (int i = 0; i < 2; ++i) mbar_init(b_hready + 8 * i, EPI_WARPS);
+        if constexpr (FC_TAIL) {
+            mbar_init(b_tail, EPI_WARPS);
+            mbar_init(b_wfc, both);
+            for (int i = 0; i < 2; ++i) {
+                mbar_init(b_afull + 8 * i, both); mbar_init(b_aempty + 8 * i, 1);
+                mbar_init(b_faccfull + 8 * i, 1); mbar_init(b_faccempty + 8 * i, 2 * EPI_WARPS);
+            }
+        }
         mbar_fence_init();
     }
     if (warp == 3) tmem_alloc_pair(smem_u32(&tmem_base_s), 512);
@@ -792,11 +856,16 @@ branch_kernel(const LayerParams p) {
         asm volatile("setmaxnreg.dec.sync.aligned.u32 32;");
         if (warp == 0) {
             if (elect_one()) {
-                const uint8_t* wsrc = p.w_img + (size_t)crank * W_STEP * QSLAB_BYTES;
+                if constexpr (FC_TAIL) {
+                    // fc weights first: they stay put for the whole kernel
+                    mbar_arrive_expect_tx(b_wfc, BR_YS * HSLAB_BYTES);
+                    bulk_g2s(smem_u32(s_wfc), fc.w_img + (size_t)crank * BR_YS * HSLAB_BYTES, BR_YS * HSLAB_BYTES, b_wfc);
+                }
+                const uint8_t* wsrc = L.w_img + (size_t)crank * BR_W_STEP * QSLAB_BYTES;
                 uint32_t stage = 0, phase = 0;
                 for (int step = 0; step < T; ++step) {
                     const uint8_t* src = wsrc;
-                    for (int s = 0; s < W_STEP; s += BR_STG) {
+                    for (int s = 0; s < BR_W_STEP; s += BR_STG) {
                         mbar_wait(b_wempty + 8 * stage, phase ^ 1);
                         mbar_arrive_expect_tx(b_wfull + 8 * stage, BR_STG * QSLAB_BYTES);
                         bulk_g2s(smem_u32(s_w + (size_t)stage * BR_STG * QSLAB_BYTES), src, BR_STG * QSLAB_BYTES, b_wfull + 8 * stage);
@@ -811,33 +880,55 @@ branch_kernel(const LayerParams p) {
                 for (int step = 0; step < T; ++step)
                     for (int d = 0; d < 2; ++d) {
                         const int t = d ? (T - 1 - step) : step;
-                        const uint8_t* xsrc = p.x_img + ((size_t)tile * T + t) * KSX * SLAB_BYTES;
-                        for (int j = 0; j < KSX; ++j) {
-                            const uint32_t o = 8u * (uint32_t)(d * KSX + j);
+                        const uint8_t* xsrc = L.x_img + ((size_t)tile * T + t) * BR_KSX * SLAB_BYTES;
+                        for (int j = 0; j < BR_KSX; ++j) {
+                            const uint32_t o = 8u * (uint32_t)(d * BR_KSX + j);
                             mbar_wait(b_xempty + o, (step & 1) ^ 1);
                             mbar_arrive_expect_tx(b_xfull + o, SLAB_BYTES);
-                            bulk_g2s(smem_u32(s_x + (size_t)(d * KSX + j) * SLAB_BYTES), xsrc + (size_t)j * SLAB_BYTES, SLAB_BYTES, b_xfull + o);
+                            bulk_g2s(smem_u32(s_x + (size_t)(d * BR_KSX + j) * SLAB_BYTES), xsrc + (size_t)j * SLAB_BYTES, SLAB_BYTES, b_xfull + o);
                         }
                     }
+                if constexpr (FC_TAIL) {
+                    // ---- tail: y(t) of the own tile back from L2, double buffered over the idle x + ring space ----
+                    mbar_wait(b_tail, 0);    // every y store of this CTA is done and fenced towards the async proxy;
+                                             // it also implies all recurrent MMAs (the last readers of x + ring) completed
+                    for (int t = 0; t < T; ++t) {
+                        const uint32_t buf = (uint32_t)t & 1u;
+                        mbar_wait(b_aempty + 8 * buf, ((uint32_t)(t >> 1) & 1u) ^ 1u);
+                        mbar_arrive_expect_tx(b_afull + 8 * buf, BR_YS * SLAB_BYTES);
+                        bulk_g2s(smem_u32(s_a + (size_t)buf * BR_YS * SLAB_BYTES), L.y_img + ((size_t)tile * T + t) * BR_YS * SLAB_BYTES,
+                                 BR_YS * SLAB_BYTES, b_afull + 8 * buf);
+                    }
+                }
             }
         } else if (warp == 1 && crank != 0) {
             const uint32_t r_wfull = mapa_u32(b_wfull, 0), r_xfull = mapa_u32(b_xfull, 0);
             uint32_t stage = 0, phase = 0;
             for (int step = 0; step < T; ++step) {
-                for (int i = 0; i < 2 * KSX; ++i) {
+                for (int i = 0; i < 2 * BR_KSX; ++i) {
                     mbar_wait(b_xfull + 8 * i, step & 1);
                     if (lane == 0) mbar_arrive_cluster(r_xfull + 8 * i);
                 }
-                for (int s = 0; s < W_STEP; s += BR_STG) {
+                for (int s = 0; s < BR_W_STEP; s += BR_STG) {
                     mbar_wait(b_wfull + 8 * stage, phase);
                     if (lane == 0) mbar_arrive_cluster(r_wfull + 8 * stage);
                     if (++stage == BR_NST) { stage = 0; phase ^= 1; }
                 }
             }
+            if constexpr (FC_TAIL) {
+                const uint32_t r_wfc = mapa_u32(b_wfc, 0), r_afull = mapa_u32(b_afull, 0);
+                mbar_wait(b_wfc, 0);
+                if (lane == 0) mbar_arrive_cluster(r_wfc);
+                for (int t = 0; t < T; ++t) {
+                    const uint32_t buf = (uint32_t)t & 1u;
+                    mbar_wait(b_afull + 8 * buf, (uint32_t)(t >> 1) & 1u);
+                    if (lane == 0) mbar_arrive_cluster(r_afull + 8 * buf);
+                }
+            }
         } else if (warp == 1) {
             const bool leader = elect_one();
             const uint32_t a_lo0 = smem_desc_lo(smem_u32(s_x)), b_lo0 = smem_desc_lo(smem_u32(s_w));
-            const int xk16 = p.xk16;
+            const int xk16 = L.xk16;
             uint32_t stage = 0, phase = 0, in_stage = 0;
             auto w_acquire = [&]() -> uint32_t {
                 if (in_stage == 0) { mbar_wait_cluster(b_wfull + 8 * stage, phase); tc_fence_after(); }
@@ -861,13 +952,13 @@ branch_kernel(const LayerParams p) {
                             mbar_wait_cluster(b_accempty + 8 * (d * 2 + e), (use & 1u) ^ 1u);
                             tc_fence_after();
 #pragma unroll
-                            for (int j = 0; j < KSX; ++j) {
-                                const uint32_t xo = 8u * (uint32_t)(d * KSX + j);
+                            for (int j = 0; j < BR_KSX; ++j) {
+                                const uint32_t xo = 8u * (uint32_t)(d * BR_KSX + j);
                                 if (pr == 0 && e == 0) { mbar_wait_cluster(b_xfull + xo, step & 1); tc_fence_after(); }
                                 const uint32_t bl = w_acquire();
                                 if (leader) {
-                                    const uint32_t al = a_lo0 + (uint32_t)(d * KSX + j) * (SLAB_BYTES >> 4);
-                                    const int nk = (KSX * 4 == xk16) ? 4 : min(4, xk16 - 4 * j);
+                                    const uint32_t al = a_lo0 + (uint32_t)(d * BR_KSX + j) * (SLAB_BYTES >> 4);
+                                    const int nk = (BR_KSX * 4 == xk16) ? 4 : min(4, xk16 - 4 * j);
 #pragma unroll
                                     for (int k = 0; k < 4; ++k) {
                                         if (k < nk) {
@@ -902,6 +993,33 @@ branch_kernel(const LayerParams p) {
                     }
                 }
             }
+            if constexpr (FC_TAIL) {
+                // ---- tail: fc = y(t) * W_fc^T, accumulators = the (now idle) columns of chain 0 / chain 1 ----
+                const uint32_t fa_lo0 = smem_desc_lo(smem_u32(s_a)), fb_lo0 = smem_desc_lo(smem_u32(s_wfc));
+                mbar_wait_cluster(b_wfc, 0);
+                tc_fence_after();
+                for (int t = 0; t < T; ++t) {
+                    const uint32_t buf = (uint32_t)t & 1u, use = (uint32_t)(t >> 1);
+                    mbar_wait_cluster(b_faccempty + 8 * buf, (use & 1u) ^ 1u);
+                    mbar_wait_cluster(b_afull + 8 * buf, use & 1u);
+                    tc_fence_after();
+                    if (leader) {
+#pragma unroll
+                        for (int j = 0; j < BR_YS; ++j) {
+                            const uint32_t al = fa_lo0 + (buf * BR_YS + (uint32_t)j) * (SLAB_BYTES >> 4);
+                            const uint32_t bl = fb_lo0 + (uint32_t)j * (HSLAB_BYTES >> 4);
+#pragma unroll
+                            for (int k = 0; k < 4; ++k) {
+                                if (j == 0 && k == 0) mma2_ss_lo<0>(tmem + buf * 128u, al, bl, IDESC_FC);
+                                else mma2_ss_lo<1>(tmem + buf * 128u, al + k * 2, bl + k * 2, IDESC_FC);
+                            }
+                        }
+                        mma2_commit(b_aempty + 8 * buf, PAIR_MASK);
+                        mma2_commit(b_faccfull + 8 * buf, PAIR_MASK);
+                    }
+                    __syncwarp();
+                }
+            }
         }
     } else {
         asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
@@ -911,31 +1029,33 @@ branch_kernel(const LayerParams p) {
         const int half = (ew >> 2) & 1;              // which 32 of the chunk's 64 columns (8 hidden units)
         const int row = q * 32 + lane;
         const int64_t site = (int64_t)tile * TILE + row;
-        const bool valid = site < p.n;
+        const bool valid = site < L.n;
         const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
         const uint32_t r_accempty = mapa_u32(b_accempty, 0) + 16u * (uint32_t)d, r_hready = mapa_u32(b_hready, 0) + 8u * (uint32_t)d;
         const uint32_t b_myfull = b_accfull + 16u * (uint32_t)d;
 
-        for (int i = tid - 128; i < NBIAS; i += EPI_WARPS * 32) s_bias[i] = p.bias[i];
+        for (int i = tid - 128; i < BR_NBIAS; i += EPI_WARPS * 32) s_bias[i] = L.bias[i];
+        if constexpr (FC_TAIL)
+            for (int i = tid - 128; i < 128; i += EPI_WARPS * 32) s_fcb[i] = fc.bias[i];
         asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
 
         constexpr int UPT = 8;
         float2 c2[BR_NCH][UPT / 2];
-        const bool draw = p.h0 == nullptr;
-        const uint64_t gs = (uint64_t)(p.site_base + site);
-        const uint32_t k0 = (uint32_t)p.seed, k1 = (uint32_t)(p.seed >> 32);
-        const uint32_t slot0 = (p.rng_slot + (uint32_t)d) << 16;
+        const bool draw = L.h0 == nullptr;
+        const uint64_t gs = (uint64_t)(L.site_base + site);
+        const uint32_t k0 = (uint32_t)L.seed, k1 = (uint32_t)(L.seed >> 32);
+        const uint32_t slot0 = (L.rng_slot + (uint32_t)d) << 16;
         if (draw) {
 #pragma unroll 1
             for (int i = 0; i < BR_NCH * (UPT / 4); ++i) {
                 const int unit = (i >> 1) * 16 + half * UPT + (i & 1) * 4;
-                const float4 hq = philox_normal4((uint32_t)gs, (uint32_t)(gs >> 32), slot0 | (uint32_t)(unit >> 2), p.rng_call, k0, k1);
+                const float4 hq = philox_normal4((uint32_t)gs, (uint32_t)(gs >> 32), slot0 | (uint32_t)(unit >> 2), L.rng_call, k0, k1);
                 tmem_st2(t_h(d, 0) + lane_addr + (uint32_t)(unit >> 1), pack_half2(hq.x, hq.y), pack_half2(hq.z, hq.w));
             }
             tmem_st_wait();
         } else {
-            const float* h0 = p.h0 + (size_t)d * p.state_dir_stride + (size_t)site * BR_H;
-            const float* c0 = p.c0 + (size_t)d * p.state_dir_stride + (size_t)site * BR_H;
+            const float* h0 = L.h0 + (size_t)d * L.state_dir_stride + (size_t)site * BR_H;
+            const float* c0 = L.c0 + (size_t)d * L.state_dir_stride + (size_t)site * BR_H;
 #pragma unroll
             for (int ch = 0; ch < BR_NCH; ++ch) {
                 const int u0 = ch * 16 + half * UPT;
@@ -959,7 +1079,7 @@ branch_kernel(const LayerParams p) {
 #pragma unroll 1
             for (int i = 0; i < BR_NCH * (UPT / 4); ++i) {
                 const int unit = (i >> 1) * 16 + half * UPT + (i & 1) * 4;
-                const float4 cv = philox_normal4((uint32_t)gs, (uint32_t)(gs >> 32), slot0 | (uint32_t)(unit >> 2) | 0x8000u, p.rng_call, k0, k1);
+                const float4 cv = philox_normal4((uint32_t)gs, (uint32_t)(gs >> 32), slot0 | (uint32_t)(unit >> 2) | 0x8000u, L.rng_call, k0, k1);
                 tmem_st2(t_park + (uint32_t)(unit >> 1), pack_half2(cv.x, cv.y), pack_half2(cv.z, cv.w));
             }
             tmem_st_wait();
@@ -978,7 +1098,7 @@ branch_kernel(const LayerParams p) {
         const uint32_t s_bias_u32 = smem_u32(s_bias) + (uint32_t)((d * BR_NCH * BR_NW + half * 32) * 4);
         for (int step = 0; step < T; ++step) {
             const int t = d ? (T - 1 - step) : step;
-            uint8_t* ybase = p.y_img + ((size_t)tile * T + t) * p.y_slabs * SLAB_BYTES + row * SLAB_ROW_BYTES;
+            uint8_t* ybase = L.y_img + ((size_t)tile * T + t) * BR_YS * SLAB_BYTES + row * SLAB_ROW_BYTES;
             const uint32_t t_hnext = t_h(d, (step + 1) & 1) + lane_addr;
 #pragma unroll
             for (int ch = 0; ch < BR_NCH; ++ch) {
@@ -1024,6 +1144,41 @@ branch_kernel(const LayerParams p) {
             __syncwarp();
             if (lane == 0) mbar_arrive_cluster(r_hready);
         }
+        if constexpr (FC_TAIL) {
+            // ---- tail: this CTA's y image is complete; hand it to the async proxy (the bulk copies of warp 2) ----
+            asm volatile("fence.proxy.async.global;" ::: "memory");
+            __syncwarp();
+            if (lane == 0) mbar_arrive(b_tail);
+            const int sl = ew >> 2;                  // 32-column slice of the 128 fc outputs
+            const uint32_t r_faccempty = mapa_u32(b_faccempty, 0);
+            const int col0 = fc.col0 + sl * 32;
+            const float* bs = s_fcb + sl * 32;
+            for (int t = 0; t < T; ++t) {
+                const uint32_t buf = (uint32_t)t & 1u, use = (uint32_t)(t >> 1);
+                mbar_wait(b_faccfull + 8 * buf, use & 1u);
+                tc_fence_after();
+                uint32_t v[32];
+                tmem_ld32(tmem + buf * 128u + lane_addr + (uint32_t)(sl * 32), v);
+                tmem_ld_wait();
+                tc_fence_before();
+                __syncwarp();
+                if (lane == 0) mbar_arrive_cluster(r_faccempty + 8 * buf);
+                uint8_t* yslab = fc.y_img + (((size_t)tile * T + t) * BR_YS + (size_t)(col0 >> 6)) * SLAB_BYTES + row * SLAB_ROW_BYTES;
+#pragma unroll
+                for (int c8 = 0; c8 < 4; ++c8) {
+                    uint32_t o[4];
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) {
+                        const int j = c8 * 8 + e * 2;
+                        const float a = fmaxf(__uint_as_float(v[j]) + bs[j], 0.f);
+                        const float b = fmaxf(__uint_as_float(v[j + 1]) + bs[j + 1], 0.f);
+                        o[e] = pack_half2(a, b);
+                    }
+                    const int chunk = ((col0 & 63) >> 3) + c8;
+                    *reinterpret_cast<uint4*>(yslab + ((chunk ^ (row & 7)) << 4)) = make_uint4(o[0], o[1], o[2], o[3]);
+                }
+            }
+        }
     }
     tc_fence_before();
     __syncthreads();
@@ -1031,12 +1186,19 @@ branch_kernel(const LayerParams p) {
     if (warp == 3) tmem_dealloc_pair(tmem, 512);
 }
 
+// The hidden-128 layers of a branch, one launch per layer (DSP_B200_BRANCH_DUAL=1, or where the wave cost favours it).
+__global__ void __launch_bounds__(NTHREADS, 1)
+branch_kernel(const LayerParams p) {
+    branch_body<false>({p.x_img, p.w_img, p.bias, p.h0, p.c0, p.state_dir_stride, p.rng_slot, p.xk16, p.y_img,
+                        p.seed, p.rng_call, p.site_base, p.n, p.T}, FcTail{}, (int)blockIdx.x);
+}
+
 // ---------------------------------------------------------------------------------------------
 // both_bilstm's two branches in ONE launch, with their per-timestep dense layers fused behind them
 // (models.py:196-201 and :212-217, then the concat of :225).  Grid = 2 x tile pairs of CTA pairs: cluster
 // 2k runs lstm_seq + fc_seq, cluster 2k+1 lstm_signal + fc_signal for the same two site tiles, so the
 // launch has one tail instead of four and both halves of a tile's lstm_comb input are produced in the same
-// wave.  The recurrent phase is branch_kernel's (two direction chains per CTA pair).  fc needs h_fwd(t) and
+// wave.  The recurrent phase is branch_kernel's, the same branch_body.  fc needs h_fwd(t) and
 // h_bwd(t) of the same t, which the two chains produce T-1-2t steps apart, so it runs as a TAIL phase of the
 // same CTA pair once step T-1 is done: the pair streams its own y image back (written minutes of
 // microseconds ago by its own epilogue warps: L2 hits, no second kernel re-reading it from HBM), multiplies
@@ -1067,391 +1229,11 @@ struct FusedBranchParams {
 
 __global__ void __launch_bounds__(NTHREADS, 1)
 branch_fused_kernel(const FusedBranchParams p) {
-    constexpr int KSX = 1;
-    constexpr int KS = KSX + BR_KSH;
-    constexpr int PAIR_UNITS = 4 * KSX + 4 * BR_KSH;
-    constexpr int W_STEP = (BR_NCH / 2) * PAIR_UNITS;
-    constexpr int NBIAS = 2 * BR_NCH * BR_NW;
-    constexpr uint32_t IDESC = make_idesc_f16(256, BR_NW);
-    constexpr uint32_t IDESC_FC = make_idesc_f16(256, 128);
-    constexpr int FC_KS = 4;                                 // K = 256 = [h_fwd | h_bwd]
-    static_assert(W_STEP % BR_STG == 0 && KS * 2 == PAIR_UNITS / 2, "stream layout");
-    static_assert(2 * KSX * SLAB_BYTES + BR_NST * BR_STG * QSLAB_BYTES == 2 * FC_KS * SLAB_BYTES, "tail A buffers alias x + ring exactly");
-
-    extern __shared__ __align__(1024) uint8_t smem_raw[];
-    uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-    uint8_t* s_x = smem;                                   // [dir][KSX] slabs          } recurrent phase
-    uint8_t* s_w = smem + (size_t)2 * KSX * SLAB_BYTES;    // weight ring               }
-    uint8_t* s_a = smem;                                   // tail: 2 x 4 slabs of y(t), aliasing the two above
-    uint8_t* s_wfc = smem + (size_t)2 * FC_KS * SLAB_BYTES;   // this CTA's half of the fc weights (4 half slabs), resident
-    float* s_bias = reinterpret_cast<float*>(s_wfc + (size_t)FC_KS * HSLAB_BYTES);
-    float* s_fcb = s_bias + NBIAS;
-    __shared__ __align__(8) uint64_t bars[2 * BR_NST + 4 * KSX + 10 + 10];
-    __shared__ uint32_t tmem_base_s;
-    const uint32_t b_wfull = smem_u32(&bars[0]), b_wempty = smem_u32(&bars[BR_NST]);
-    const uint32_t b_xfull = smem_u32(&bars[2 * BR_NST]), b_xempty = b_xfull + 8 * 2 * KSX;       // [dir][KSX]
-    const uint32_t b_accfull = b_xempty + 8 * 2 * KSX, b_accempty = b_accfull + 32;               // [dir][2]
-    const uint32_t b_hready = b_accempty + 32;                                                  // [dir]
-    const uint32_t b_tail = b_hready + 16;                 // all epilogue warps of THIS CTA are past the last y store
-    const uint32_t b_wfc = b_tail + 8;                     // fc weights landed (both CTAs)
-    const uint32_t b_afull = b_wfc + 8, b_aempty = b_afull + 16;                                  // [2]
-    const uint32_t b_faccfull = b_aempty + 16, b_faccempty = b_faccfull + 16;                     // [2]
-
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int br = (int)((blockIdx.x >> 1) & 1u);                                   // 0 seq, 1 signal
     const int tile = (int)(((blockIdx.x >> 2) << 1) | (blockIdx.x & 1u));
-    const int T = p.T;
-    const uint32_t crank = cluster_ctarank();
-
-    if (tid == 0) {
-        const uint32_t both = crank == 0 ? 2u : 1u;
-        for (int i = 0; i < BR_NST; ++i) { mbar_init(b_wfull + 8 * i, both); mbar_init(b_wempty + 8 * i, 1); }
-        for (int i = 0; i < 2 * KSX; ++i) { mbar_init(b_xfull + 8 * i, both); mbar_init(b_xempty + 8 * i, 1); }
-        for (int i = 0; i < 4; ++i) { mbar_init(b_accfull + 8 * i, 1); mbar_init(b_accempty + 8 * i, EPI_WARPS); }
-        for (int i = 0; i < 2; ++i) mbar_init(b_hready + 8 * i, EPI_WARPS);
-        mbar_init(b_tail, EPI_WARPS);
-        mbar_init(b_wfc, both);
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(b_afull + 8 * i, both); mbar_init(b_aempty + 8 * i, 1);
-            mbar_init(b_faccfull + 8 * i, 1); mbar_init(b_faccempty + 8 * i, 2 * EPI_WARPS);
-        }
-        mbar_fence_init();
-    }
-    if (warp == 3) tmem_alloc_pair(smem_u32(&tmem_base_s), 512);
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();
-    tc_fence_after();
-    const uint32_t tmem = tmem_base_s;
-    griddep_launch_dependents();
-    auto t_acc = [&](int d, int e) -> uint32_t { return tmem + (uint32_t)(d * 128 + e * 64); };
-    auto t_h = [&](int d, int b) -> uint32_t { return tmem + 256u + (uint32_t)(d * 128 + b * 64); };
-    const uint8_t* x_img = p.x_img[br];
-    uint8_t* y_img = p.y_img[br];
-
-    if (warp < 4) {
-        asm volatile("setmaxnreg.dec.sync.aligned.u32 32;");
-        if (warp == 0) {
-            if (elect_one()) {
-                // fc weights first: they stay put for the whole kernel
-                mbar_arrive_expect_tx(b_wfc, FC_KS * HSLAB_BYTES);
-                bulk_g2s(smem_u32(s_wfc), p.fcw_img[br] + (size_t)crank * FC_KS * HSLAB_BYTES, FC_KS * HSLAB_BYTES, b_wfc);
-                const uint8_t* wsrc = p.w_img[br] + (size_t)crank * W_STEP * QSLAB_BYTES;
-                uint32_t stage = 0, phase = 0;
-                for (int step = 0; step < T; ++step) {
-                    const uint8_t* src = wsrc;
-                    for (int s = 0; s < W_STEP; s += BR_STG) {
-                        mbar_wait(b_wempty + 8 * stage, phase ^ 1);
-                        mbar_arrive_expect_tx(b_wfull + 8 * stage, BR_STG * QSLAB_BYTES);
-                        bulk_g2s(smem_u32(s_w + (size_t)stage * BR_STG * QSLAB_BYTES), src, BR_STG * QSLAB_BYTES, b_wfull + 8 * stage);
-                        src += (size_t)BR_STG * QSLAB_BYTES;
-                        if (++stage == BR_NST) { stage = 0; phase ^= 1; }
-                    }
-                }
-            }
-        } else if (warp == 2) {
-            if (elect_one()) {
-                griddep_wait();              // the layer input is the previous kernel's output
-                for (int step = 0; step < T; ++step)
-                    for (int d = 0; d < 2; ++d) {
-                        const int t = d ? (T - 1 - step) : step;
-                        const uint8_t* xsrc = x_img + ((size_t)tile * T + t) * KSX * SLAB_BYTES;
-                        for (int j = 0; j < KSX; ++j) {
-                            const uint32_t o = 8u * (uint32_t)(d * KSX + j);
-                            mbar_wait(b_xempty + o, (step & 1) ^ 1);
-                            mbar_arrive_expect_tx(b_xfull + o, SLAB_BYTES);
-                            bulk_g2s(smem_u32(s_x + (size_t)(d * KSX + j) * SLAB_BYTES), xsrc + (size_t)j * SLAB_BYTES, SLAB_BYTES, b_xfull + o);
-                        }
-                    }
-                // ---- tail: y(t) of the own tile back from L2, double buffered over the idle x + ring space ----
-                mbar_wait(b_tail, 0);        // every y store of this CTA is done and fenced towards the async proxy;
-                                             // it also implies all recurrent MMAs (the last readers of x + ring) completed
-                for (int t = 0; t < T; ++t) {
-                    const uint32_t buf = (uint32_t)t & 1u;
-                    mbar_wait(b_aempty + 8 * buf, ((uint32_t)(t >> 1) & 1u) ^ 1u);
-                    mbar_arrive_expect_tx(b_afull + 8 * buf, FC_KS * SLAB_BYTES);
-                    bulk_g2s(smem_u32(s_a + (size_t)buf * FC_KS * SLAB_BYTES), y_img + ((size_t)tile * T + t) * FC_KS * SLAB_BYTES,
-                             FC_KS * SLAB_BYTES, b_afull + 8 * buf);
-                }
-            }
-        } else if (warp == 1 && crank != 0) {
-            const uint32_t r_wfull = mapa_u32(b_wfull, 0), r_xfull = mapa_u32(b_xfull, 0);
-            uint32_t stage = 0, phase = 0;
-            for (int step = 0; step < T; ++step) {
-                for (int i = 0; i < 2 * KSX; ++i) {
-                    mbar_wait(b_xfull + 8 * i, step & 1);
-                    if (lane == 0) mbar_arrive_cluster(r_xfull + 8 * i);
-                }
-                for (int s = 0; s < W_STEP; s += BR_STG) {
-                    mbar_wait(b_wfull + 8 * stage, phase);
-                    if (lane == 0) mbar_arrive_cluster(r_wfull + 8 * stage);
-                    if (++stage == BR_NST) { stage = 0; phase ^= 1; }
-                }
-            }
-            const uint32_t r_wfc = mapa_u32(b_wfc, 0), r_afull = mapa_u32(b_afull, 0);
-            mbar_wait(b_wfc, 0);
-            if (lane == 0) mbar_arrive_cluster(r_wfc);
-            for (int t = 0; t < T; ++t) {
-                const uint32_t buf = (uint32_t)t & 1u;
-                mbar_wait(b_afull + 8 * buf, (uint32_t)(t >> 1) & 1u);
-                if (lane == 0) mbar_arrive_cluster(r_afull + 8 * buf);
-            }
-        } else if (warp == 1) {
-            const bool leader = elect_one();
-            const uint32_t a_lo0 = smem_desc_lo(smem_u32(s_x)), b_lo0 = smem_desc_lo(smem_u32(s_w));
-            const int xk16 = p.xk16[br];
-            uint32_t stage = 0, phase = 0, in_stage = 0;
-            auto w_acquire = [&]() -> uint32_t {
-                if (in_stage == 0) { mbar_wait_cluster(b_wfull + 8 * stage, phase); tc_fence_after(); }
-                return b_lo0 + (stage * BR_STG + in_stage) * (uint32_t)(QSLAB_BYTES >> 4);
-            };
-            auto w_release = [&]() {
-                if (++in_stage == BR_STG) {
-                    if (leader) mma2_commit(b_wempty + 8 * stage, PAIR_MASK);
-                    in_stage = 0;
-                    if (++stage == BR_NST) { stage = 0; phase ^= 1; }
-                }
-                __syncwarp();
-            };
-            for (int step = 0; step < T; ++step) {
-                for (int pr = 0; pr < BR_NCH / 2; ++pr) {
-                    const uint32_t use = (uint32_t)(step * (BR_NCH / 2) + pr);
-#pragma unroll
-                    for (int d = 0; d < 2; ++d)
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            mbar_wait_cluster(b_accempty + 8 * (d * 2 + e), (use & 1u) ^ 1u);
-                            tc_fence_after();
-#pragma unroll
-                            for (int j = 0; j < KSX; ++j) {
-                                const uint32_t xo = 8u * (uint32_t)(d * KSX + j);
-                                if (pr == 0 && e == 0) { mbar_wait_cluster(b_xfull + xo, step & 1); tc_fence_after(); }
-                                const uint32_t bl = w_acquire();
-                                if (leader) {
-                                    const uint32_t al = a_lo0 + (uint32_t)(d * KSX + j) * (SLAB_BYTES >> 4);
-                                    const int nk = (KSX * 4 == xk16) ? 4 : min(4, xk16 - 4 * j);
-#pragma unroll
-                                    for (int k = 0; k < 4; ++k) {
-                                        if (k < nk) {
-                                            if (j == 0 && k == 0) mma2_ss_lo<0>(t_acc(d, e), al, bl, IDESC);
-                                            else mma2_ss_lo<1>(t_acc(d, e), al + k * 2, bl + k * 2, IDESC);
-                                        }
-                                    }
-                                    if (pr == BR_NCH / 2 - 1 && e == 1) mma2_commit(b_xempty + xo, PAIR_MASK);
-                                }
-                                w_release();
-                            }
-                        }
-#pragma unroll
-                    for (int d = 0; d < 2; ++d) {
-                        if (pr == 0) { mbar_wait_cluster(b_hready + 8 * d, step & 1); tc_fence_after(); }
-                        const uint32_t a_t = t_h(d, step & 1);
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-#pragma unroll
-                            for (int j = 0; j < BR_KSH; ++j) {
-                                const uint32_t bl = w_acquire();
-                                if (leader) {
-#pragma unroll
-                                    for (int k = 0; k < 4; ++k)
-                                        mma2_ts_lo<1>(t_acc(d, e), a_t + (uint32_t)(j * 32 + k * 8), bl + k * 2, IDESC);
-                                }
-                                w_release();
-                            }
-                            if (leader) mma2_commit(b_accfull + 8 * (d * 2 + e), PAIR_MASK);
-                            __syncwarp();
-                        }
-                    }
-                }
-            }
-            // ---- tail: fc = y(t) * W_fc^T, accumulators = the (now idle) columns of chain 0 / chain 1 ----
-            const uint32_t fa_lo0 = smem_desc_lo(smem_u32(s_a)), fb_lo0 = smem_desc_lo(smem_u32(s_wfc));
-            mbar_wait_cluster(b_wfc, 0);
-            tc_fence_after();
-            for (int t = 0; t < T; ++t) {
-                const uint32_t buf = (uint32_t)t & 1u, use = (uint32_t)(t >> 1);
-                mbar_wait_cluster(b_faccempty + 8 * buf, (use & 1u) ^ 1u);
-                mbar_wait_cluster(b_afull + 8 * buf, use & 1u);
-                tc_fence_after();
-                if (leader) {
-#pragma unroll
-                    for (int j = 0; j < FC_KS; ++j) {
-                        const uint32_t al = fa_lo0 + (buf * FC_KS + (uint32_t)j) * (SLAB_BYTES >> 4);
-                        const uint32_t bl = fb_lo0 + (uint32_t)j * (HSLAB_BYTES >> 4);
-#pragma unroll
-                        for (int k = 0; k < 4; ++k) {
-                            if (j == 0 && k == 0) mma2_ss_lo<0>(tmem + buf * 128u, al, bl, IDESC_FC);
-                            else mma2_ss_lo<1>(tmem + buf * 128u, al + k * 2, bl + k * 2, IDESC_FC);
-                        }
-                    }
-                    mma2_commit(b_aempty + 8 * buf, PAIR_MASK);
-                    mma2_commit(b_faccfull + 8 * buf, PAIR_MASK);
-                }
-                __syncwarp();
-            }
-        }
-    } else {
-        asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
-        const int ew = warp - 4;
-        const int d = ew >> 3;                       // chain = direction
-        const int q = warp & 3;                      // TMEM lane quarter
-        const int half = (ew >> 2) & 1;              // which 32 of the chunk's 64 columns (8 hidden units)
-        const int row = q * 32 + lane;
-        const int64_t site = (int64_t)tile * TILE + row;
-        const bool valid = site < p.n;
-        const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-        const uint32_t r_accempty = mapa_u32(b_accempty, 0) + 16u * (uint32_t)d, r_hready = mapa_u32(b_hready, 0) + 8u * (uint32_t)d;
-        const uint32_t b_myfull = b_accfull + 16u * (uint32_t)d;
-
-        for (int i = tid - 128; i < NBIAS; i += EPI_WARPS * 32) s_bias[i] = p.bias[br][i];
-        for (int i = tid - 128; i < 128; i += EPI_WARPS * 32) s_fcb[i] = p.fcb[br][i];
-        asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
-
-        constexpr int UPT = 8;
-        float2 c2[BR_NCH][UPT / 2];
-        const bool draw = p.h0[br] == nullptr;
-        const uint64_t gs = (uint64_t)(p.site_base + site);
-        const uint32_t k0 = (uint32_t)p.seed, k1 = (uint32_t)(p.seed >> 32);
-        const uint32_t slot0 = (p.rng_slot[br] + (uint32_t)d) << 16;
-        if (draw) {
-#pragma unroll 1
-            for (int i = 0; i < BR_NCH * (UPT / 4); ++i) {
-                const int unit = (i >> 1) * 16 + half * UPT + (i & 1) * 4;
-                const float4 hq = philox_normal4((uint32_t)gs, (uint32_t)(gs >> 32), slot0 | (uint32_t)(unit >> 2), p.rng_call, k0, k1);
-                tmem_st2(t_h(d, 0) + lane_addr + (uint32_t)(unit >> 1), pack_half2(hq.x, hq.y), pack_half2(hq.z, hq.w));
-            }
-            tmem_st_wait();
-        } else {
-            const float* h0 = p.h0[br] + (size_t)d * p.state_dir_stride[br] + (size_t)site * BR_H;
-            const float* c0 = p.c0[br] + (size_t)d * p.state_dir_stride[br] + (size_t)site * BR_H;
-#pragma unroll
-            for (int ch = 0; ch < BR_NCH; ++ch) {
-                const int u0 = ch * 16 + half * UPT;
-                float4 cv0 = make_float4(0.f, 0.f, 0.f, 0.f), cv1 = cv0, hq0 = cv0, hq1 = cv0;
-                if (valid) {
-                    cv0 = *reinterpret_cast<const float4*>(c0 + u0); cv1 = *reinterpret_cast<const float4*>(c0 + u0 + 4);
-                    hq0 = *reinterpret_cast<const float4*>(h0 + u0); hq1 = *reinterpret_cast<const float4*>(h0 + u0 + 4);
-                }
-                c2[ch][0] = make_float2(cv0.x, cv0.y); c2[ch][1] = make_float2(cv0.z, cv0.w);
-                c2[ch][2] = make_float2(cv1.x, cv1.y); c2[ch][3] = make_float2(cv1.z, cv1.w);
-                tmem_st4(t_h(d, 0) + lane_addr + (uint32_t)(u0 >> 1), pack_half2(hq0.x, hq0.y), pack_half2(hq0.z, hq0.w),
-                         pack_half2(hq1.x, hq1.y), pack_half2(hq1.z, hq1.w));
-            }
-            tmem_st_wait();
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(r_hready);
-        if (draw) {          // c0 behind the first MMAs, parked in this thread's columns of h buffer 1 (see layer_kernel)
-            const uint32_t t_park = t_h(d, 1) + lane_addr;
-#pragma unroll 1
-            for (int i = 0; i < BR_NCH * (UPT / 4); ++i) {
-                const int unit = (i >> 1) * 16 + half * UPT + (i & 1) * 4;
-                const float4 cv = philox_normal4((uint32_t)gs, (uint32_t)(gs >> 32), slot0 | (uint32_t)(unit >> 2) | 0x8000u, p.rng_call, k0, k1);
-                tmem_st2(t_park + (uint32_t)(unit >> 1), pack_half2(cv.x, cv.y), pack_half2(cv.z, cv.w));
-            }
-            tmem_st_wait();
-#pragma unroll
-            for (int ch = 0; ch < BR_NCH; ++ch) {
-                uint32_t v[4];
-                tmem_ld4(t_park + (uint32_t)((ch * 16 + half * UPT) >> 1), v);
-                tmem_ld_wait();
-#pragma unroll
-                for (int j = 0; j < UPT / 2; ++j) {
-                    const __half2 hh = *reinterpret_cast<const __half2*>(&v[j]);
-                    c2[ch][j] = make_float2(__low2float(hh), __high2float(hh));
-                }
-            }
-        }
-        const uint32_t s_bias_u32 = smem_u32(s_bias) + (uint32_t)((d * BR_NCH * BR_NW + half * 32) * 4);
-        for (int step = 0; step < T; ++step) {
-            const int t = d ? (T - 1 - step) : step;
-            uint8_t* ybase = y_img + ((size_t)tile * T + t) * FC_KS * SLAB_BYTES + row * SLAB_ROW_BYTES;
-            const uint32_t t_hnext = t_h(d, (step + 1) & 1) + lane_addr;
-#pragma unroll
-            for (int ch = 0; ch < BR_NCH; ++ch) {
-                const int e = ch & 1;
-                const uint32_t use = (uint32_t)(step * (BR_NCH / 2) + (ch >> 1));
-                mbar_wait(b_myfull + 8 * e, use & 1u);
-                tc_fence_after();
-                const int u0 = ch * 16 + half * UPT;
-                float2 h2[UPT / 2];
-#pragma unroll
-                for (int part = 0; part < 2; ++part) {
-                    uint32_t v[16];
-                    tmem_ld16(t_acc(d, e) + lane_addr + (uint32_t)(half * 32 + part * 16), v);
-                    float4 bq[4];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) bq[i] = lds128(s_bias_u32 + (uint32_t)((ch * BR_NW + part * 16 + i * 4) * 4));
-                    tmem_ld_wait();
-                    if (part == 1) {
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive_cluster(r_accempty + 8 * e);
-                    }
-#pragma unroll
-                    for (int qq = 0; qq < 2; ++qq) {
-                        const float4 b0 = bq[2 * qq], b1 = bq[2 * qq + 1];
-                        const float2 ai = add2(make_float2(__uint_as_float(v[qq * 8 + 0]), __uint_as_float(v[qq * 8 + 1])), make_float2(b0.x, b0.y));
-                        const float2 af = add2(make_float2(__uint_as_float(v[qq * 8 + 2]), __uint_as_float(v[qq * 8 + 3])), make_float2(b0.z, b0.w));
-                        const float2 ag = add2(make_float2(__uint_as_float(v[qq * 8 + 4]), __uint_as_float(v[qq * 8 + 5])), make_float2(b1.x, b1.y));
-                        const float2 ao = add2(make_float2(__uint_as_float(v[qq * 8 + 6]), __uint_as_float(v[qq * 8 + 7])), make_float2(b1.z, b1.w));
-                        lstm_cell2<DSP_POLY_MASK_BRANCH>(ai, af, ag, ao, c2[ch][part * 2 + qq], h2[part * 2 + qq]);
-                    }
-                }
-                uint32_t pk[UPT / 2];
-#pragma unroll
-                for (int j = 0; j < UPT / 2; ++j) pk[j] = pack_half2(h2[j].x, h2[j].y);
-                tmem_st4(t_hnext + (uint32_t)(u0 >> 1), pk[0], pk[1], pk[2], pk[3]);
-                const int col = d * BR_H + u0;                             // multiple of 8
-                uint8_t* yslab = ybase + (size_t)(col >> 6) * SLAB_BYTES;
-                *reinterpret_cast<uint4*>(yslab + ((((col & 63) >> 3) ^ (row & 7)) << 4)) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-            }
-            tmem_st_wait();
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive_cluster(r_hready);
-        }
-        // ---- tail: this CTA's y image is complete; hand it to the async proxy (the bulk copies of warp 2) ----
-        asm volatile("fence.proxy.async.global;" ::: "memory");
-        __syncwarp();
-        if (lane == 0) mbar_arrive(b_tail);
-        {
-            const int sl = ew >> 2;                  // 32-column slice of the 128 fc outputs
-            const uint32_t r_faccempty = mapa_u32(b_faccempty, 0);
-            const int col0 = br * 128 + sl * 32;     // column of lstm_comb's input image: [fc_seq | fc_signal]
-            const float* bs = s_fcb + sl * 32;
-            for (int t = 0; t < T; ++t) {
-                const uint32_t buf = (uint32_t)t & 1u, use = (uint32_t)(t >> 1);
-                mbar_wait(b_faccfull + 8 * buf, use & 1u);
-                tc_fence_after();
-                uint32_t v[32];
-                tmem_ld32(tmem + buf * 128u + lane_addr + (uint32_t)(sl * 32), v);
-                tmem_ld_wait();
-                tc_fence_before();
-                __syncwarp();
-                if (lane == 0) mbar_arrive_cluster(r_faccempty + 8 * buf);
-                uint8_t* yslab = p.comb_img + (((size_t)tile * T + t) * FC_KS + (size_t)(col0 >> 6)) * SLAB_BYTES + row * SLAB_ROW_BYTES;
-#pragma unroll
-                for (int c8 = 0; c8 < 4; ++c8) {
-                    uint32_t o[4];
-#pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        const int j = c8 * 8 + e * 2;
-                        const float a = fmaxf(__uint_as_float(v[j]) + bs[j], 0.f);
-                        const float b = fmaxf(__uint_as_float(v[j + 1]) + bs[j + 1], 0.f);
-                        o[e] = pack_half2(a, b);
-                    }
-                    const int chunk = ((col0 & 63) >> 3) + c8;
-                    *reinterpret_cast<uint4*>(yslab + ((chunk ^ (row & 7)) << 4)) = make_uint4(o[0], o[1], o[2], o[3]);
-                }
-            }
-        }
-    }
-    tc_fence_before();
-    __syncthreads();
-    cluster_sync_all();
-    if (warp == 3) tmem_dealloc_pair(tmem, 512);
+    branch_body<true>({p.x_img[br], p.w_img[br], p.bias[br], p.h0[br], p.c0[br], p.state_dir_stride[br], p.rng_slot[br],
+                       p.xk16[br], p.y_img[br], p.seed, p.rng_call, p.site_base, p.n, p.T},
+                      {p.fcw_img[br], p.fcb[br], p.comb_img, br * 128}, tile);    // comb columns: [fc_seq | fc_signal]
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1583,20 +1365,12 @@ int tc_alloc(Model* m, void** p, size_t bytes) {
     return DSP_OK;
 }
 
-template <int KSX, int H, int MODE, int NOUT>
-int launch_layer(Model* m, const LayerParams& p, int64_t tiles, cudaStream_t st) {
-    constexpr int NCH = MODE != MODE_LSTM ? NOUT / 128 : H / 32;
-    const size_t smem = (size_t)KSX * RingCfg<KSX, MODE>::XB * SLAB_BYTES + (size_t)RingCfg<KSX, MODE>::NST * RingCfg<KSX, MODE>::STG * HSLAB_BYTES
-                        + (size_t)NCH * 128 * sizeof(float) + 1024;
-    auto kern = layer_kernel<KSX, H, MODE, NOUT>;
+// CTA-pair kernels: clusters of 2 along x, programmatic dependent launch unless DSP_B200_PDL=0 turned it off.
+template <class Params>
+int launch_pair(Model* m, void (*kern)(Params), const Params& p, dim3 grid, size_t smem, cudaStream_t st) {
     DSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     cudaLaunchConfig_t cfg{};
-    const unsigned tiles2 = (unsigned)((tiles + 1) / 2 * 2);                          // CTA pairs: the workspace is padded too
-#if DSP_DIR_INTERLEAVE
-    cfg.gridDim = dim3(MODE != MODE_LSTM ? tiles2 : 2 * tiles2, 1);
-#else
-    cfg.gridDim = dim3(tiles2, MODE != MODE_LSTM ? 1 : 2);
-#endif
+    cfg.gridDim = grid;
     cfg.blockDim = dim3(NTHREADS);
     cfg.dynamicSmemBytes = smem;
     cfg.stream = st;
@@ -1612,47 +1386,24 @@ int launch_layer(Model* m, const LayerParams& p, int64_t tiles, cudaStream_t st)
     return DSP_OK;
 }
 
-template <int KSX>
+template <int KSX, int H, int MODE, int NOUT>
+int launch_layer(Model* m, const LayerParams& p, int64_t tiles, cudaStream_t st) {
+    const unsigned tiles2 = (unsigned)((tiles + 1) / 2 * 2);                          // CTA pairs: the workspace is padded too
+#if DSP_DIR_INTERLEAVE
+    const dim3 grid(MODE != MODE_LSTM ? tiles2 : 2 * tiles2, 1);
+#else
+    const dim3 grid(tiles2, MODE != MODE_LSTM ? 1 : 2);
+#endif
+    return launch_pair(m, layer_kernel<KSX, H, MODE, NOUT>, p, grid, LayerCfg<KSX, H, MODE, NOUT>::BYTES, st);
+}
+
 int launch_branch(Model* m, const LayerParams& p, int64_t tiles, cudaStream_t st) {
-    const size_t smem = (size_t)2 * KSX * SLAB_BYTES + (size_t)BR_NST * BR_STG * QSLAB_BYTES + (size_t)2 * BR_NCH * BR_NW * sizeof(float) + 1024;
-    auto kern = branch_kernel<KSX>;
-    DSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)((tiles + 1) / 2 * 2), 1);
-    cfg.blockDim = dim3(NTHREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = ((TcState*)m->tc_state)->pdl ? 2 : 1;
-    DSP_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
-    m->launches++;
-    return DSP_OK;
+    return launch_pair(m, branch_kernel, p, dim3((unsigned)((tiles + 1) / 2 * 2), 1), BranchSmem<false>::BYTES, st);
 }
 
 int launch_branch_fused(Model* m, const FusedBranchParams& p, int64_t tiles, cudaStream_t st) {
-    const size_t smem = (size_t)2 * 4 * SLAB_BYTES + (size_t)4 * HSLAB_BYTES + (size_t)(2 * BR_NCH * BR_NW + 128) * sizeof(float) + 1024;
-    auto kern = branch_fused_kernel;
-    DSP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)(2 * ((tiles + 1) / 2 * 2)), 1);       // (tile pair, branch, rank in pair)
-    cfg.blockDim = dim3(NTHREADS);
-    cfg.dynamicSmemBytes = smem;
-    cfg.stream = st;
-    cudaLaunchAttribute attr[2];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-    attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = ((TcState*)m->tc_state)->pdl ? 2 : 1;
-    DSP_CUDA(cudaLaunchKernelEx(&cfg, kern, p));
-    m->launches++;
-    return DSP_OK;
+    // (tile pair, branch, rank in pair)
+    return launch_pair(m, branch_fused_kernel, p, dim3((unsigned)(2 * ((tiles + 1) / 2 * 2)), 1), BranchSmem<true>::BYTES, st);
 }
 
 int launch_lstm(Model* m, int KSX, int H, const LayerParams& p, int64_t tiles, cudaStream_t st) {
@@ -1773,21 +1524,22 @@ int tc_pack_lstm_layer(Model* m, LstmLayer& L,
     pk->xk16 = (K + 15) / 16;
     const float* wih[2] = {wih0, wih1}; const float* whh[2] = {whh0, whh1};
     const float* bih[2] = {bih0, bih1}; const float* bhh[2] = {bhh0, bhh1};
-    if (H == BR_H && KSX == 1) {
-        // branch_kernel: [rank][stream unit][32 rows x 128 B]; per chunk pair (c, c+1) the stream is
+    // branch_kernel / branch_fused_kernel stage BR_KSX x slabs per direction: the first layer of a branch, whose input
+    // tc_create limits to 64 columns (signal_len <= 64, <= 16 sequence features), gets their weight image
+    static_assert(BR_KSX == 1, "a branch's first-layer input is one slab wide");
+    if (H == BR_H && KSX == BR_KSX) {
+        // [rank][stream unit][32 rows x 128 B]; per chunk pair (c, c+1) the stream is
         // X(0,c) X(0,c+1) X(1,c) X(1,c+1) H(0,c) H(0,c+1) H(1,c) H(1,c+1) (first index = direction)
-        const int pair_units = 4 * KSX + 4 * KSH;
-        const size_t per_rank = (size_t)(BR_NCH / 2) * pair_units;
-        std::vector<uint8_t> img((size_t)2 * per_rank * QSLAB_BYTES, 0);
-        std::vector<float> bias((size_t)2 * BR_NCH * BR_NW);
+        std::vector<uint8_t> img((size_t)2 * BR_W_STEP * QSLAB_BYTES, 0);
+        std::vector<float> bias((size_t)BR_NBIAS);
         auto put = [&](int rank, size_t unit, int row, int k, float v) {
             __half h = __float2half_rn(v);
-            memcpy(&img[((size_t)rank * per_rank + unit) * QSLAB_BYTES + slab_offset_bytes((uint32_t)row, (uint32_t)k)], &h, 2);
+            memcpy(&img[((size_t)rank * BR_W_STEP + unit) * QSLAB_BYTES + slab_offset_bytes((uint32_t)row, (uint32_t)k)], &h, 2);
         };
         for (int d = 0; d < 2; ++d)
             for (int ch = 0; ch < BR_NCH; ++ch) {
-                const size_t pair_base = (size_t)(ch >> 1) * pair_units;
-                const size_t sx = pair_base + (size_t)(d * 2 + (ch & 1)) * KSX, sh = pair_base + 4 * KSX + (size_t)(d * 2 + (ch & 1)) * KSH;
+                const size_t pair_base = (size_t)(ch >> 1) * BR_PAIR_UNITS;
+                const size_t sx = pair_base + (size_t)(d * 2 + (ch & 1)) * BR_KSX, sh = pair_base + 4 * BR_KSX + (size_t)(d * 2 + (ch & 1)) * BR_KSH;
                 for (int n = 0; n < BR_NW; ++n) {
                     const int g = (n >> 1) & 3;
                     const int unit = ch * 16 + (n >> 3) * 2 + (n & 1);
@@ -1956,7 +1708,7 @@ int tc_forward_chunk(Model* m, const float* kmer, const float* means, const floa
                 if (s->force_dual >= 0) dual = s->force_dual != 0;
             }
             if (dual) { p.w_img = pk->w_img_dual; p.bias = pk->bias_dual; }
-            int rc = dual ? launch_branch<1>(m, p, tiles, st) : launch_lstm(m, pk->KSX, hid, p, tiles, st);
+            int rc = dual ? launch_branch(m, p, tiles, st) : launch_lstm(m, pk->KSX, hid, p, tiles, st);
             if (rc) return rc;
             x = s->ybuf[l & 1];
         }
