@@ -17,8 +17,9 @@ the data path; ``call_freq`` parses contiguous byte shards, exchanges the record
 every rank writes its slice of the table (freq_dist.py); ``train`` keeps ``--batch_size`` as the global batch, every
 rank trains on a slice of each step and the gradients are summed by a deterministic all-reduce over NVLink peer
 memory, so the replicas stay bit-identical and rank 0 writes the checkpoints (train_dist.py).  ``extract`` here takes reads that are already decoded
-(reading fast5 needs h5py: outside this implementation); ``train`` runs the reference's training loop on the fp32 training kernels (train.py); ``denoise`` stays with the
-reference."""
+(reading fast5 needs h5py: outside this implementation); ``train`` runs the reference's training loop on the fp32 training kernels (train.py), with
+``--optim_type Adam|RMSprop|SGD|Ranger`` (Ranger's step is one fused kernel per parameter group, optim.py); ``denoise``
+stays with the reference."""
 from __future__ import annotations
 
 import argparse
@@ -48,7 +49,8 @@ def add_train_parser(sub):
     g.add_argument("--is_signallen", type=str, default="yes", required=False)
     g.add_argument("--hid_rnn", type=int, default=256, required=False)
     g = tp.add_argument_group("TRAINING")
-    g.add_argument("--optim_type", type=str, default="Adam", choices=["Adam", "RMSprop", "SGD"], required=False)
+    g.add_argument("--optim_type", type=str, default="Adam", choices=["Adam", "RMSprop", "SGD", "Ranger"],
+                   required=False)
     g.add_argument("--batch_size", type=int, default=512, required=False)
     g.add_argument("--lr", type=float, default=0.001, required=False)
     g.add_argument("--max_epoch_num", type=int, default=10, required=False)

@@ -2,7 +2,8 @@
 training kernels.
 
 Loop, as the reference runs it:
-* CrossEntropyLoss with class weights [1, pos_weight]; Adam / RMSprop / SGD(momentum 0.8) at ``--lr``;
+* CrossEntropyLoss with class weights [1, pos_weight]; Adam / RMSprop / SGD(momentum 0.8) / Ranger (``optim.py``: the
+  reference's ``utils/ranger2020.py`` as one fused kernel per step) at ``--lr``;
   StepLR(step_size=2, gamma=0.1) stepped once per epoch; ``clip_grad_norm_(model.parameters(), 0.5)``.
 * Every ``step_interval`` steps and at the last step of an epoch the model is validated under
   ``eval()`` (the inference path).  When the validation accuracy beats the best of this epoch and comes
@@ -87,7 +88,10 @@ def make_optimizer(name, params, lr):
         return torch.optim.RMSprop(params, lr=lr)
     if name == "SGD":
         return torch.optim.SGD(params, lr=lr, momentum=0.8)
-    raise ValueError("--optim_type must be Adam, RMSprop or SGD (Ranger is not available here)")
+    if name == "Ranger":
+        from .optim import Ranger
+        return Ranger(params, lr=lr, betas=(0.95, 0.999), eps=1e-5)
+    raise ValueError("--optim_type must be Adam, RMSprop, SGD or Ranger")
 
 
 def evaluate(model, data, criterion, batch_size):

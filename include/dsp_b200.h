@@ -172,6 +172,32 @@ int dsp_train_backward(dsp_handle h, const float* const* params, int32_t n_param
                        const float* const* dropout_masks, const void* arena, const float* dlogits,
                        int64_t n, void* workspace, float* const* grads, void* stream);
 
+/* dsp_ranger_step: one step of Ranger (RAdam + Lookahead + gradient centralisation, the reference's
+ * utils/ranger2020.py) for the n_tensors tensors of one parameter group, in place, on the current device.
+ * Per tensor i, all DEVICE pointers to numel[i] contiguous float32 elements: params[i] (p), grads[i] (g),
+ * exp_avg[i] (m), exp_avg_sq[i] (v), slow_buffer[i] (the Lookahead weights); row_len[i] = numel / size(0)
+ * for a tensor of more than one dimension, numel (or 1 when numel is 0) otherwise.  The caller works out
+ * the per-tensor scalars from the tensor's own step count t (so tensors at different steps update exactly):
+ *   neg_step_lr[i] = (float)(-step_size(t) * lr);
+ *   flags[i]: DSP_RANGER_RECTIFY (N_sma(t) > N_sma_threshhold), DSP_RANGER_LOOKAHEAD (t % k == 0),
+ *             DSP_RANGER_CENTRALIZE (gradient centralisation applies to this tensor).
+ * Per element, in fp32 and the published order: with gc_loc = 1 and CENTRALIZE, g -= mean of g over its row,
+ * WRITTEN BACK to grads[i] (as the published code centralises p.grad in place); v = v*beta2 + (1-beta2)*g*g;
+ * m = m*beta1 + (1-beta1)*g; G = m / (sqrt(v) + eps) if RECTIFY else m; G += weight_decay * p; with gc_loc = 0
+ * and CENTRALIZE, G -= mean of G over its row; un-rectified, G is m and m receives those changes;
+ * p += neg_step_lr * G; on LOOKAHEAD slow += alpha * (p - slow), p = slow.  slow_buffer is read only on
+ * LOOKAHEAD steps.  Every row mean is summed in a fixed order and every element is computed by one thread, so
+ * the same inputs give the same bits on every call and on every GPU.  Negative sizes, a row_len that does not
+ * divide numel, unknown flags or a null pointer give DSP_ERR_INVALID before anything is launched.  One launch
+ * per 56 tensors on `stream`; does not synchronise. */
+#define DSP_RANGER_RECTIFY 1
+#define DSP_RANGER_LOOKAHEAD 2
+#define DSP_RANGER_CENTRALIZE 4
+int dsp_ranger_step(int32_t n_tensors, float* const* params, float* const* grads, float* const* exp_avg,
+                    float* const* exp_avg_sq, float* const* slow_buffer, const int64_t* numel,
+                    const int64_t* row_len, const float* neg_step_lr, const int32_t* flags, double beta1,
+                    double beta2, double eps, double weight_decay, double alpha, int32_t gc_loc, void* stream);
+
 /* Number of kernels this library launched on behalf of `h` since creation. */
 int64_t dsp_launch_count(dsp_handle h);
 /* Milliseconds (CUDA events on the launching stream) spent in kernels of class `which`

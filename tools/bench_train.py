@@ -27,6 +27,7 @@ import torch  # noqa: E402
 import torch.nn.functional as F  # noqa: E402
 
 from deepsignal_plant_b200.models import ModelBiLSTM  # noqa: E402
+from deepsignal_plant_b200.train import make_optimizer  # noqa: E402
 
 
 def forward_flop_per_site(m):
@@ -72,7 +73,7 @@ def torch_forward(m, kmer, means, stds, lens, signals, p):
     return m.fc2(x)
 
 
-def run_arm(arm, batch, seconds, warmup, p, dev, log):
+def run_arm(arm, batch, seconds, warmup, p, dev, log, optim="Adam"):
     torch.manual_seed(1234)
     m = ModelBiLSTM(dropout_rate=p, trainable=True).cuda(dev).train()
     n = batch
@@ -82,7 +83,7 @@ def run_arm(arm, batch, seconds, warmup, p, dev, log):
          torch.randn(n, 13, 16, device=dev, generator=g)]
     y = torch.randint(0, 2, (n,), device=dev, generator=g)
     crit = torch.nn.CrossEntropyLoss()
-    opt = torch.optim.Adam(m.parameters(), lr=1e-3)
+    opt = make_optimizer(optim, m.parameters(), 1e-3)
     fwd = (lambda: m(*x)[0]) if arm == "b200_kernels" else (lambda: torch_forward(m, *x, p))
 
     def step(ev=None):
@@ -114,11 +115,11 @@ def run_arm(arm, batch, seconds, warmup, p, dev, log):
     wall = time.perf_counter() - t0
     split = [sum(e[i].elapsed_time(e[i + 1]) for e in evs) / 1e3 for i in range(3)]
     flop = 3 * forward_flop_per_site(m)
-    r = {"arm": arm, "batch": batch, "steps": steps, "seconds": wall, "sites_per_s": steps * n / wall,
+    r = {"arm": arm, "optim": optim, "batch": batch, "steps": steps, "seconds": wall, "sites_per_s": steps * n / wall,
          "forward_s": split[0], "backward_s": split[1], "optimizer_s": split[2],
          "flop_per_site": flop, "achieved_tflops": steps * n * flop / wall / 1e12}
-    log("%-12s batch %5d: %6d steps in %.2f s = %9.0f sites/s, %.2f TFLOP/s; fwd %.1f%% bwd %.1f%% opt %.1f%%" % (
-        arm, batch, steps, wall, r["sites_per_s"], r["achieved_tflops"], 100 * split[0] / sum(split),
+    log("%-12s %-6s batch %5d: %6d steps in %.2f s = %9.0f sites/s, %.2f TFLOP/s; fwd %.1f%% bwd %.1f%% opt %.1f%%" % (
+        arm, optim, batch, steps, wall, r["sites_per_s"], r["achieved_tflops"], 100 * split[0] / sum(split),
         100 * split[1] / sum(split), 100 * split[2] / sum(split)))
     del m, opt
     torch.cuda.empty_cache()
