@@ -22,8 +22,10 @@ SYMBOLS = (
     "dsp_comm_create", "dsp_comm_export", "dsp_comm_connect", "dsp_comm_destroy", "dsp_freq_aggregate_distributed",
     "dsp_comm_route_rows", "dsp_comm_last_timing", "dsp_comm_allreduce_f32", "dsp_freq_aggregate_host", "dsp_device_warmup",
     "dsp_train_shape", "dsp_train_arena_bytes", "dsp_train_workspace_bytes", "dsp_train_forward", "dsp_train_backward",
-    "dsp_ranger_step",
+    "dsp_ranger_step", "dsp_train_forward_batch", "dsp_train_backward_batch",
 )
+
+TRAIN_MAX_MODELS = 8    # DSP_TRAIN_MAX_MODELS
 
 MODULES = {"both_bilstm": 0, "seq_bilstm": 1, "signal_bilstm": 2}
 PRECISIONS = {"fp32": 0, "fp16": 1}
@@ -114,6 +116,10 @@ def lib():
     L.dsp_train_forward.argtypes = [vp, C.POINTER(vp), i32, fp, fp, fp, fp, fp, C.POINTER(vp), u64, C.POINTER(vp), i64, vp,
                                     fp, vp]
     L.dsp_train_backward.argtypes = [vp, C.POINTER(vp), i32, C.POINTER(vp), vp, fp, i64, vp, C.POINTER(vp), vp]
+    L.dsp_train_forward_batch.argtypes = [vp, i32, C.POINTER(vp), i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(u64),
+                                          C.POINTER(vp), i64, C.POINTER(vp), C.POINTER(vp), vp]
+    L.dsp_train_backward_batch.argtypes = [vp, i32, C.POINTER(vp), i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), i64,
+                                           C.POINTER(vp), C.POINTER(vp), vp]
     d = C.c_double
     L.dsp_ranger_step.argtypes = [i32] + [C.POINTER(vp)] * 5 + [C.POINTER(i64), C.POINTER(i64), C.POINTER(C.c_float),
                                                                  C.POINTER(i32), d, d, d, d, d, i32, vp]

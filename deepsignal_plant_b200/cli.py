@@ -9,6 +9,7 @@ reference's flag names and defaults.
     python -m deepsignal_plant_b200 extract   -i reads.npz -o features.dspf     # ... -> binary hand-off (feature_bin.py)
     python -m deepsignal_plant_b200 call_mods -i features.dspf -m model.ckpt -o calls.tsv      # same calls, no text parsing
     python -m deepsignal_plant_b200 pack_features -i features.tsv -o features.dspf             # an existing text file -> binary
+    python -m deepsignal_plant_b200 denoise --train_file samples.tsv      # -> samples.denoise_fp<k>.tsv, then train on it
     python -m deepsignal_plant_b200 train --train_file train.dspf --valid_file valid.dspf --model_dir models/
 
 Multi-GPU: launch ``call_mods``, ``call_freq`` or ``train`` under torchrun, one process per GPU.  ``call_mods`` cuts the
@@ -19,7 +20,8 @@ rank trains on a slice of each step and the gradients are summed by a determinis
 memory, so the replicas stay bit-identical and rank 0 writes the checkpoints (train_dist.py).  ``extract`` here takes reads that are already decoded
 (reading fast5 needs h5py: outside this implementation); ``train`` runs the reference's training loop on the fp32 training kernels (train.py), with
 ``--optim_type Adam|RMSprop|SGD|Ranger`` (Ranger's step is one fused kernel per parameter group, optim.py); ``denoise``
-stays with the reference."""
+removes unsupported positive samples before ``train``, training each iteration's cross-validation models together in
+model-batched steps (denoise.py).  ``denoise`` runs on one GPU; under torchrun it is refused."""
 from __future__ import annotations
 
 import argparse
@@ -62,6 +64,46 @@ def add_train_parser(sub):
     return tp
 
 
+def add_denoise_parser(sub):
+    """The reference's ``denoise`` flags and defaults (``deepsignal_plant.py`` denoise parser)."""
+    dp = sub.add_parser("denoise", description="remove positive training samples whose label the data does not support "
+                                               "(labelled features: .dspf or the reference's text file)")
+    g = dp.add_argument_group("INPUT")
+    g.add_argument("--train_file", type=str, required=True)
+    g = dp.add_argument_group("FILTER")
+    g.add_argument("--is_filter_fn", type=str, default="no", required=False,
+                   help="also remove negative samples the models score as positive; default no")
+    g = dp.add_argument_group("MODEL_HYPER")
+    g.add_argument("--model_type", type=str, default="signal_bilstm",
+                   choices=["both_bilstm", "seq_bilstm", "signal_bilstm"], required=False)
+    g.add_argument("--seq_len", type=int, default=13, required=False)
+    g.add_argument("--signal_len", type=int, default=16, required=False)
+    g.add_argument("--layernum1", type=int, default=3, required=False)
+    g.add_argument("--layernum2", type=int, default=1, required=False)
+    g.add_argument("--class_num", type=int, default=2, required=False)
+    g.add_argument("--dropout_rate", type=float, default=0.5, required=False)
+    g.add_argument("--n_vocab", type=int, default=16, required=False)
+    g.add_argument("--n_embed", type=int, default=4, required=False)
+    g.add_argument("--is_base", type=str, default="yes", required=False)
+    g.add_argument("--is_signallen", type=str, default="yes", required=False)
+    g.add_argument("--hid_rnn", type=int, default=256, required=False)
+    g = dp.add_argument_group("TRAINING")
+    g.add_argument("--pos_weight", type=float, default=1.0, required=False)
+    g.add_argument("--batch_size", type=int, default=512, required=False)
+    g.add_argument("--lr", type=float, default=0.001, required=False)
+    g.add_argument("--epoch_num", type=int, default=3, required=False)
+    g.add_argument("--step_interval", type=int, default=100, required=False)
+    g = dp.add_argument_group("DENOISE")
+    g.add_argument("--iterations", type=int, default=10, required=False)
+    g.add_argument("--rounds", type=int, default=3, required=False)
+    g.add_argument("--score_cf", type=float, default=0.5, required=False,
+                   help="score cutoff to keep a sample; default 0.5")
+    g.add_argument("--kept_ratio", type=float, default=0.99, required=False,
+                   help="stop once this fraction of the positive (and, with --is_filter_fn, negative) samples is kept")
+    g.add_argument("--tseed", type=int, default=1234, required=False)
+    return dp
+
+
 def build_parser():
     parser = argparse.ArgumentParser(prog="deepsignal_plant_b200",
                                      description="deepsignal-plant extract / call_mods / call_freq on B200 (sm_100a) kernels")
@@ -69,6 +111,7 @@ def build_parser():
     cm = sub.add_parser("call_mods", description="call modifications")
     cf = sub.add_parser("call_freq", description="call frequency of modifications at genome level")
     add_train_parser(sub)
+    add_denoise_parser(sub)
 
     ex = sub.add_parser("extract", description="extract features from decoded re-squiggled reads (an .npz archive written by "
                                                "extract_features.save_reads) into the reference's feature file")
@@ -229,6 +272,9 @@ def main(argv=None):
     elif args.module == "train":
         from .train import main as train_main
         train_main(args)
+    elif args.module == "denoise":
+        from .denoise import main as denoise_main
+        denoise_main(args)
     elif args.module == "call_freq":
         from .call_mods_freq import call_mods_frequency_to_file
         call_mods_frequency_to_file(args)

@@ -590,15 +590,62 @@ int dsp_train_shape(dsp_handle h, int32_t* n_params, int32_t* n_masks) {
 int64_t dsp_train_arena_bytes(dsp_handle h, int64_t n) { return (h && n >= 0) ? train_arena_bytes(h, n) : -1; }
 int64_t dsp_train_workspace_bytes(dsp_handle h, int64_t n) { return (h && n >= 0) ? train_workspace_bytes(h, n) : -1; }
 
-static int train_check(Model* m, const char* who, const float* const* params, int32_t n_params, const float* const* masks,
-                       const void* arena, int64_t n) {
+// Everything the training entries refuse before a launch; tables as in include/dsp_b200.h.
+static int train_check(Model* m, const char* who, int G, const float* const* params, int32_t n_params,
+                       const float* const* masks, const void* const* arenas, int64_t n) {
     int32_t np = 0, nm = 0;
     train_shape(m, &np, &nm);
-    DSP_REQUIRE(params && masks && arena, DSP_ERR_INVALID, "%s: null argument", who);
+    DSP_REQUIRE(G >= 1 && G <= DSP_TRAIN_MAX_MODELS, DSP_ERR_INVALID, "%s: %d models, must be 1..%d", who, G,
+                DSP_TRAIN_MAX_MODELS);
+    DSP_REQUIRE(params && masks && arenas, DSP_ERR_INVALID, "%s: null argument", who);
     DSP_REQUIRE(n_params == np, DSP_ERR_INVALID, "%s: %d parameters given, this configuration has %d", who, n_params, np);
-    for (int i = 0; i < np; ++i) DSP_REQUIRE(params[i], DSP_ERR_INVALID, "%s: parameter %d is null", who, i);
+    for (int i = 0; i < G * np; ++i)
+        DSP_REQUIRE(params[i], DSP_ERR_INVALID, "%s: parameter %d of model %d is null", who, i % np, i / np);
+    for (int i = 0; i < G; ++i) DSP_REQUIRE(arenas[i], DSP_ERR_INVALID, "%s: arena of model %d is null", who, i);
+    for (int i = 1; i < G; ++i)
+        for (int k = 0; k < nm; ++k)
+            DSP_REQUIRE(!masks[i * nm + k] == !masks[k], DSP_ERR_INVALID,
+                        "%s: dropout mask slot %d is null for some models and not for others", who, k);
     DSP_REQUIRE(n >= 1, DSP_ERR_INVALID, "%s: batch must hold at least one site", who);
     return DSP_OK;
+}
+
+static int train_forward_checked(Model* m, const char* who, int G, const float* const* params, int32_t n_params,
+                                 const float* const* inputs, const float* const* states, const uint64_t* seeds,
+                                 const float* const* masks, int64_t n, void* const* arenas, float* const* logits,
+                                 void* stream) {
+    int rc = train_check(m, who, G, params, n_params, masks, arenas, n);
+    if (rc) return rc;
+    DSP_REQUIRE(inputs && seeds && logits, DSP_ERR_INVALID, "%s: null argument", who);
+    for (int i = 0; i < G; ++i) {
+        const float* const* in = inputs + 5 * i;
+        DSP_REQUIRE(logits[i], DSP_ERR_INVALID, "%s: null output pointer (model %d)", who, i);
+        if (has_seq(m)) DSP_REQUIRE(in[0] && in[1] && in[2] && in[3], DSP_ERR_INVALID,
+                                    "%s: sequence features are required for this module (model %d)", who, i);
+        if (has_signal(m)) DSP_REQUIRE(in[4], DSP_ERR_INVALID, "%s: signals are required for this module (model %d)", who, i);
+        if (states)
+            for (int g = 0; g < 3; ++g) {
+                if ((g == 0 && !has_seq(m)) || (g == 1 && !has_signal(m))) continue;
+                DSP_REQUIRE(states[6 * i + 2 * g] && states[6 * i + 2 * g + 1], DSP_ERR_INVALID,
+                            "%s: states[%d] of model %d is null", who, 2 * g, i);
+            }
+    }
+    DeviceGuard guard(m->cfg.device);
+    return train_forward(m, G, params, inputs, states, seeds, masks, n, arenas, logits, (cudaStream_t)stream);
+}
+
+static int train_backward_checked(Model* m, const char* who, int G, const float* const* params, int32_t n_params,
+                                  const float* const* masks, const void* const* arenas, const float* const* dlogits,
+                                  int64_t n, void* const* workspaces, float* const* grads, void* stream) {
+    int rc = train_check(m, who, G, params, n_params, masks, arenas, n);
+    if (rc) return rc;
+    DSP_REQUIRE(dlogits && workspaces && grads, DSP_ERR_INVALID, "%s: null argument", who);
+    for (int i = 0; i < G; ++i)
+        DSP_REQUIRE(dlogits[i] && workspaces[i], DSP_ERR_INVALID, "%s: null argument (model %d)", who, i);
+    for (int i = 0; i < G * n_params; ++i)
+        DSP_REQUIRE(grads[i], DSP_ERR_INVALID, "%s: gradient %d of model %d is null", who, i % n_params, i / n_params);
+    DeviceGuard guard(m->cfg.device);
+    return train_backward(m, G, params, masks, arenas, dlogits, n, workspaces, grads, (cudaStream_t)stream);
 }
 
 int dsp_train_forward(dsp_handle h, const float* const* params, int32_t n_params, const float* kmer,
@@ -606,29 +653,35 @@ int dsp_train_forward(dsp_handle h, const float* const* params, int32_t n_params
                       const float* signals, const float* const* states, uint64_t seed,
                       const float* const* dropout_masks, int64_t n, void* arena, float* logits, void* stream) {
     DSP_REQUIRE(h, DSP_ERR_INVALID, "dsp_train_forward: null handle");
-    Model* m = h;
-    int rc = train_check(m, "dsp_train_forward", params, n_params, dropout_masks, arena, n);
-    if (rc) return rc;
-    DSP_REQUIRE(logits, DSP_ERR_INVALID, "dsp_train_forward: null output pointer");
-    if (has_seq(m)) DSP_REQUIRE(kmer && base_means && base_stds && base_signal_lens, DSP_ERR_INVALID,
-                                "dsp_train_forward: sequence features are required for this module");
-    if (has_signal(m)) DSP_REQUIRE(signals, DSP_ERR_INVALID, "dsp_train_forward: signals are required for this module");
-    DeviceGuard guard(m->cfg.device);
-    return train_forward(m, params, kmer, base_means, base_stds, base_signal_lens, signals, states, seed, dropout_masks, n,
-                         arena, logits, (cudaStream_t)stream);
+    const float* inputs[5] = {kmer, base_means, base_stds, base_signal_lens, signals};
+    return train_forward_checked(h, "dsp_train_forward", 1, params, n_params, inputs, states, &seed, dropout_masks, n,
+                                 &arena, &logits, stream);
 }
 
 int dsp_train_backward(dsp_handle h, const float* const* params, int32_t n_params, const float* const* dropout_masks,
                        const void* arena, const float* dlogits, int64_t n, void* workspace, float* const* grads,
                        void* stream) {
     DSP_REQUIRE(h, DSP_ERR_INVALID, "dsp_train_backward: null handle");
-    Model* m = h;
-    int rc = train_check(m, "dsp_train_backward", params, n_params, dropout_masks, arena, n);
-    if (rc) return rc;
-    DSP_REQUIRE(dlogits && workspace && grads, DSP_ERR_INVALID, "dsp_train_backward: null argument");
-    for (int i = 0; i < n_params; ++i) DSP_REQUIRE(grads[i], DSP_ERR_INVALID, "dsp_train_backward: gradient %d is null", i);
-    DeviceGuard guard(m->cfg.device);
-    return train_backward(m, params, dropout_masks, arena, dlogits, n, workspace, grads, (cudaStream_t)stream);
+    return train_backward_checked(h, "dsp_train_backward", 1, params, n_params, dropout_masks, &arena, &dlogits, n,
+                                  &workspace, grads, stream);
+}
+
+int dsp_train_forward_batch(dsp_handle h, int32_t n_models, const float* const* params, int32_t n_params,
+                            const float* const* inputs, const float* const* states, const uint64_t* seeds,
+                            const float* const* dropout_masks, int64_t n, void* const* arenas,
+                            float* const* logits, void* stream) {
+    DSP_REQUIRE(h, DSP_ERR_INVALID, "dsp_train_forward_batch: null handle");
+    return train_forward_checked(h, "dsp_train_forward_batch", n_models, params, n_params, inputs, states, seeds,
+                                 dropout_masks, n, arenas, logits, stream);
+}
+
+int dsp_train_backward_batch(dsp_handle h, int32_t n_models, const float* const* params, int32_t n_params,
+                             const float* const* dropout_masks, const void* const* arenas,
+                             const float* const* dlogits, int64_t n, void* const* workspaces,
+                             float* const* grads, void* stream) {
+    DSP_REQUIRE(h, DSP_ERR_INVALID, "dsp_train_backward_batch: null handle");
+    return train_backward_checked(h, "dsp_train_backward_batch", n_models, params, n_params, dropout_masks, arenas,
+                                  dlogits, n, workspaces, grads, stream);
 }
 
 int64_t dsp_launch_count(dsp_handle h) { return h ? h->launches : 0; }

@@ -148,11 +148,12 @@ int philox_normal(Model* m, float* out, int64_t count, uint64_t seed, uint64_t s
 int train_shape(const Model* m, int32_t* n_params, int32_t* n_masks);
 int64_t train_arena_bytes(const Model* m, int64_t n);
 int64_t train_workspace_bytes(const Model* m, int64_t n);
-int train_forward(Model* m, const float* const* params, const float* kmer, const float* means, const float* stds,
-                  const float* lens, const float* signals, const float* const* states6, uint64_t seed,
-                  const float* const* masks, int64_t n, void* arena, float* logits, cudaStream_t st);
-int train_backward(Model* m, const float* const* params, const float* const* masks, const void* arena,
-                   const float* dlogits, int64_t n, void* workspace, float* const* grads, cudaStream_t st);
+// G models of one configuration in one set of launches; tables as for dsp_train_forward_batch / _backward_batch
+int train_forward(Model* m, int G, const float* const* params, const float* const* inputs, const float* const* states6,
+                  const uint64_t* seeds, const float* const* masks, int64_t n, void* const* arenas, float* const* logits,
+                  cudaStream_t st);
+int train_backward(Model* m, int G, const float* const* params, const float* const* masks, const void* const* arenas,
+                   const float* const* dlogits, int64_t n, void* const* workspaces, float* const* grads, cudaStream_t st);
 
 }  // namespace dsp
 

@@ -7,6 +7,7 @@
 // (dataflow) and torch nn.LSTM (gate order i,f,g,o; reverse direction walks t = T-1..0).
 #include "common.cuh"
 #include <curand_kernel.h>
+#include "philox.cuh"
 
 namespace dsp {
 
@@ -263,22 +264,10 @@ head_f32_kernel(const float* __restrict__ ylast, int H, int T, int64_t n,
 }
 
 // ---------------------------------------------------------------------------------------
-// N(0,1) initial states (models.py:169-176 draws torch.randn): Philox4x32-10, one
-// subsequence per group of four outputs, Box-Muller via curand_normal4.
+// N(0,1) initial states: philox_normal_quad (philox.cuh), one thread per group of four outputs.
 __global__ void philox_normal_kernel(float* __restrict__ out, int64_t count, uint64_t seed,
                                      uint64_t stream_id) {
-    int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    int64_t base = q * 4;
-    if (base >= count) return;
-    curandStatePhilox4_32_10_t st;
-    curand_init(seed, (unsigned long long)q, stream_id * 4ull, &st);
-    float4 v = curand_normal4(&st);
-    if (base + 3 < count) {
-        *reinterpret_cast<float4*>(out + base) = v;
-    } else {
-        float tmp[4] = {v.x, v.y, v.z, v.w};
-        for (int i = 0; base + i < count; ++i) out[base + i] = tmp[i];
-    }
+    philox_normal_quad(out, count, seed, stream_id, (int64_t)blockIdx.x * blockDim.x + threadIdx.x);
 }
 
 }  // namespace

@@ -10,21 +10,55 @@
 // contraction is a time-batched GEMM over all n*T rows (gemm_f32_kernel).  Sums over sites are
 // split-K with a fixed split count and a second, fixed-order reduction pass: no float atomics, so a
 // repeated backward is bit-identical.
+//
+// Model batching (dsp_train_forward_batch / dsp_train_backward_batch): one launch of every kernel covers
+// G <= DSP_TRAIN_MAX_MODELS independent models of one configuration and one site count.  Each kernel is one
+// __device__ body with two entry points: `*_kernel` takes plain __restrict__ pointers and runs one model (G = 1,
+// dsp_train_forward / dsp_train_backward), `*_batch_kernel` takes tables of G per-model pointers (Per<T>, passed as
+// __grid_constant__ kernel parameters) and gets the model index from the grid: its own y dimension for the
+// one-dimensional kernels, folded into y (recurrent kernels: model * 2 + direction, column sums: model * splits +
+// split) or z (GEMM: model * splits + split) elsewhere.  A model's CTAs do exactly the work a one-model launch does, so
+// its results are bit-identical to a one-model call.
 #include "common.cuh"
+#include "philox.cuh"
 #include <algorithm>
 #include <array>
+#include <type_traits>
 
 namespace dsp {
 
 namespace {
 
 constexpr int TS = 16;   // sites (rows) per CTA of the recurrent kernels
+constexpr int MAXG = DSP_TRAIN_MAX_MODELS;
+
+// One pointer per model of a batched launch.  `+ off` moves every non-null entry; the null pattern is the
+// same for all models (the entry points check it), so `bool` tests model 0.
+template <class T>
+struct Per {
+    T* p[MAXG];
+    Per() { for (int i = 0; i < MAXG; ++i) p[i] = nullptr; }
+    template <class U, class = typename std::enable_if<std::is_convertible<U*, T*>::value>::type>
+    Per(const Per<U>& o) { for (int i = 0; i < MAXG; ++i) p[i] = o.p[i]; }
+    __device__ __forceinline__ T* operator[](int i) const { return p[i]; }
+    Per operator+(int64_t off) const {
+        Per r = *this;
+        for (int i = 0; i < MAXG; ++i) if (r.p[i]) r.p[i] += off;
+        return r;
+    }
+    explicit operator bool() const { return p[0] != nullptr; }
+};
+using PF = Per<float>;
+using PCF = Per<const float>;
+struct Seeds { uint64_t s[MAXG]; };
+// Kernel parameters indexed by the model: read in place from the parameter space (no per-thread copy).
+#define GC const __grid_constant__
 
 __device__ __forceinline__ float sigmoid_t(float x) { return 1.0f / (1.0f + expf(-x)); }
 
 // torch layout (W_ih [4H][K], W_hh [4H][H], b_ih, b_hh) -> the fp32 forward layout of common.cuh
 // (wt [(Kp + Hp)][4][H], bias [4H] = b_ih + b_hh).
-__global__ void repack_lstm_kernel(const float* __restrict__ wih, const float* __restrict__ whh,
+__device__ __forceinline__ void repack_lstm_body(const float* __restrict__ wih, const float* __restrict__ whh,
                                    const float* __restrict__ bih, const float* __restrict__ bhh,
                                    int K, int H, float* __restrict__ wt, float* __restrict__ bias) {
     const int Kp = (K + 3) & ~3, Hp = (H + 3) & ~3;
@@ -41,7 +75,7 @@ __global__ void repack_lstm_kernel(const float* __restrict__ wih, const float* _
 }
 
 // Feature assembly (models.py:182-195) that also keeps the embedding codes it gathered.
-__global__ void assemble_seq_train_kernel(const float* __restrict__ kmer, const float* __restrict__ means,
+__device__ __forceinline__ void assemble_seq_train_body(const float* __restrict__ kmer, const float* __restrict__ means,
                                           const float* __restrict__ stds, const float* __restrict__ lens,
                                           const float* __restrict__ embed, int E, int vocab, int use_len,
                                           int kseq, int64_t rows, float* __restrict__ x, int32_t* __restrict__ codes) {
@@ -63,8 +97,8 @@ __global__ void assemble_seq_train_kernel(const float* __restrict__ kmer, const 
 // gates i, f, g, o at gates[((site*T + t)*2 + dir)*4H + gate*H + j] and the cell state c_t at
 // cst[((site*T + t)*2 + dir)*H + j].
 template <int TS_>
-__global__ void __launch_bounds__(256, 2)
-lstm_train_fwd_kernel(const float* __restrict__ x, int x_row_stride, int x_t_stride, int K,
+__device__ __forceinline__ void
+lstm_train_fwd_body(int dir, const float* __restrict__ x, int x_row_stride, int x_t_stride, int K,
                       const float* __restrict__ wt0, const float* __restrict__ wt1,
                       const float* __restrict__ bias0, const float* __restrict__ bias1,
                       const float* __restrict__ h0, const float* __restrict__ c0,
@@ -75,7 +109,6 @@ lstm_train_fwd_kernel(const float* __restrict__ x, int x_row_stride, int x_t_str
     float* ax = smem;                    // [TS][Kp]
     float* ah = ax + TS_ * Kp;           // [2][TS][Hp]
     float* cs = ah + 2 * TS_ * Hp;       // [TS][Hp]
-    const int dir = blockIdx.y;
     const float* __restrict__ wt = dir ? wt1 : wt0;
     const float* __restrict__ bias = dir ? bias1 : bias0;
     const int64_t site0 = (int64_t)blockIdx.x * TS_;
@@ -172,15 +205,15 @@ lstm_train_fwd_kernel(const float* __restrict__ x, int x_row_stride, int x_t_str
     }
 }
 
-// Recurrent part of one bidirectional LSTM layer's backward.  grid = (ceil(n/TS), 2 directions).
+// Recurrent part of one bidirectional LSTM layer's backward (direction `dir`) for one tile of TS sites.
 // Walks the direction's time order backwards with dh_rec and dc of the site tile in shared memory:
 //   dh = dY[t] + dh_rec;  dc += dh*o*(1 - tanh^2 c);  dz = (dc*g*i(1-i), dc*c_prev*f(1-f), dc*i(1-g^2),
 //   dh*tanh(c)*o(1-o));  dc *= f;  dh_rec = W_hh^T dz.
 // Writes dz to dz[((site*T + t)*2 + dir)*4H + gate*H + j] and h_{t-1} (the previous output in the
 // direction's order, h0 at its first step) to hprev[(site*T + t)*2H + dir*H + j] for dW_hh.
 template <int TS_>
-__global__ void __launch_bounds__(256)
-lstm_train_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ gates, const float* __restrict__ cst,
+__device__ __forceinline__ void
+lstm_train_bwd_body(int dir, const float* __restrict__ dy, const float* __restrict__ gates, const float* __restrict__ cst,
                       const float* __restrict__ y, const float* __restrict__ h0, const float* __restrict__ c0,
                       int64_t state_dir_stride, const float* __restrict__ whh0, const float* __restrict__ whh1,
                       float* __restrict__ dz, float* __restrict__ hprev, int H, int T, int64_t n) {
@@ -188,7 +221,6 @@ lstm_train_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ ga
     float* dzs = smem;                   // [4H][TS]
     float* dhr = dzs + 4 * H * TS_;      // [TS][H]
     float* dcs = dhr + TS_ * H;          // [TS][H]
-    const int dir = blockIdx.y;
     const float* __restrict__ whh = dir ? whh1 : whh0;
     const int64_t site0 = (int64_t)blockIdx.x * TS_;
     const int tid = threadIdx.x, nthr = blockDim.x;
@@ -257,20 +289,20 @@ lstm_train_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ ga
 }
 
 // C[m][n] (+)= sum_k A(m,k) B(k,n) (+ bias[n], ReLU) with arbitrary element strides, fp32 FMA.
-// 64x64 tile, 16-deep k slices, 256 threads x 4x4 outputs.  blockIdx.z is the split-K index: with
+// 64x64 tile, 16-deep k slices, 256 threads x 4x4 outputs.  z is the split-K index: with
 // `partial` set, split z writes its sum over k in [z*kps, (z+1)*kps) to partial[z][M][N] and
 // splitk_reduce_kernel adds the splits in order.
 constexpr int GBM = 64, GBN = 64, GBK = 16;
 
-__global__ void __launch_bounds__(256)
-gemm_f32_kernel(int M, int N, int K, const float* __restrict__ A, int64_t sam, int64_t sak,
+__device__ __forceinline__ void
+gemm_f32_body(int z, int M, int N, int K, const float* __restrict__ A, int64_t sam, int64_t sak,
                 const float* __restrict__ B, int64_t sbk, int64_t sbn, float* __restrict__ C, int64_t ldc,
                 const float* __restrict__ bias, int relu, int beta, int kps, float* __restrict__ partial) {
     __shared__ float As[GBK][GBM + 4];
     __shared__ float Bs[GBK][GBN + 4];
     const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
     const int m0 = blockIdx.x * GBM, n0 = blockIdx.y * GBN;
-    const int kbeg = blockIdx.z * kps, kend = min(K, kbeg + kps);
+    const int kbeg = z * kps, kend = min(K, kbeg + kps);
     float acc[4][4] = {};
     for (int k0 = kbeg; k0 < kend; k0 += GBK) {
 #pragma unroll
@@ -307,7 +339,7 @@ gemm_f32_kernel(int M, int N, int K, const float* __restrict__ A, int64_t sam, i
             const int gn = n0 + tx * 4 + j;
             if (gn >= N) continue;
             if (partial) {
-                partial[((int64_t)blockIdx.z * M + gm) * N + gn] = acc[i][j];
+                partial[((int64_t)z * M + gm) * N + gn] = acc[i][j];
             } else {
                 float v = acc[i][j];
                 float* c = C + (int64_t)gm * ldc + gn;
@@ -320,7 +352,7 @@ gemm_f32_kernel(int M, int N, int K, const float* __restrict__ A, int64_t sam, i
     }
 }
 
-__global__ void splitk_reduce_kernel(const float* __restrict__ partial, int splits, int M, int N,
+__device__ __forceinline__ void splitk_reduce_body(const float* __restrict__ partial, int splits, int M, int N,
                                      float* __restrict__ C, int64_t ldc, int beta) {
     const int64_t total = (int64_t)M * N;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -333,19 +365,19 @@ __global__ void splitk_reduce_kernel(const float* __restrict__ partial, int spli
 }
 
 // partial[z][c] = sum of x[r][c] over the rows of split z, in row order.
-__global__ void colsum_partial_kernel(const float* __restrict__ x, int64_t ld, int64_t rows, int cols,
+__device__ __forceinline__ void colsum_partial_body(int z, const float* __restrict__ x, int64_t ld, int64_t rows, int cols,
                                       int64_t rps, float* __restrict__ partial) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= cols) return;
-    const int64_t r0 = (int64_t)blockIdx.y * rps, r1 = min(rows, r0 + rps);
+    const int64_t r0 = (int64_t)z * rps, r1 = min(rows, r0 + rps);
     float acc = 0.f;
     for (int64_t r = r0; r < r1; ++r) acc += x[r * ld + c];
-    partial[(int64_t)blockIdx.y * cols + c] = acc;
+    partial[(int64_t)z * cols + c] = acc;
 }
 
 // out[r][c] = g[r][c] * mask[r][c] (mask may be NULL), zeroed where act[r][c] <= 0 (act may be NULL),
 // then ReLU if `relu`.  Dropout forward/backward, ReLU backward, and the head's relu(dropout(z1)).
-__global__ void ew_kernel(float* __restrict__ out, int64_t ldo, const float* __restrict__ g, int64_t ldg,
+__device__ __forceinline__ void ew_body(float* __restrict__ out, int64_t ldo, const float* __restrict__ g, int64_t ldg,
                           const float* __restrict__ mask, int64_t ldm, const float* __restrict__ act, int64_t lda,
                           int relu, int64_t rows, int cols) {
     const int64_t total = rows * cols;
@@ -360,7 +392,7 @@ __global__ void ew_kernel(float* __restrict__ out, int64_t ldo, const float* __r
 }
 
 // models.py:229-233: [h_fwd(T-1) | h_bwd(0)] of the last comb layer, times the first head dropout mask.
-__global__ void pick_last_kernel(const float* __restrict__ y, int H, int T, int64_t n, const float* __restrict__ mask,
+__device__ __forceinline__ void pick_last_body(const float* __restrict__ y, int H, int T, int64_t n, const float* __restrict__ mask,
                                  float* __restrict__ out) {
     const int64_t total = n * 2 * H;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -374,7 +406,7 @@ __global__ void pick_last_kernel(const float* __restrict__ y, int H, int T, int6
 }
 
 // Its backward: dY of the last comb layer is dlast (times the mask) at t = T-1 forward / t = 0 reverse, 0 elsewhere.
-__global__ void scatter_last_kernel(const float* __restrict__ dlast, const float* __restrict__ mask, int H, int T,
+__device__ __forceinline__ void scatter_last_body(const float* __restrict__ dlast, const float* __restrict__ mask, int H, int T,
                                     int64_t n, float* __restrict__ dy) {
     const int64_t total = n * T * 2 * H;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
@@ -392,8 +424,8 @@ __global__ void scatter_last_kernel(const float* __restrict__ dlast, const float
 
 // Embedding gradient: one CTA per code; each thread sums the rows r = tid, tid + 256, ... in order, then a
 // fixed-shape tree over the 256 partial sums.
-__global__ void __launch_bounds__(256)
-embed_grad_kernel(const float* __restrict__ dx, int ldx, const int32_t* __restrict__ codes, int64_t rows, int E,
+__device__ __forceinline__ void
+embed_grad_body(const float* __restrict__ dx, int ldx, const int32_t* __restrict__ codes, int64_t rows, int E,
                   float* __restrict__ grad) {
     __shared__ float red[256];
     const int code = blockIdx.x;
@@ -412,8 +444,158 @@ embed_grad_kernel(const float* __restrict__ dx, int ldx, const int32_t* __restri
     }
 }
 
+
+// ---- entry points ---------------------------------------------------------------------------------------------
+// Each body above has two entry points.  `xxx_kernel` takes plain __restrict__ pointer parameters and runs one model
+// (the G = 1 case: the compiler sees exactly the parameters it did before batching existed, so the one-model step
+// keeps its read-only loads and its speed).  `xxx_batch_kernel` takes per-model tables and runs model `mi` of the
+// grid.  launch_models() picks the entry by G.
+__global__ void repack_lstm_kernel(const float* __restrict__ wih, const float* __restrict__ whh,
+                                   const float* __restrict__ bih, const float* __restrict__ bhh, int K, int H,
+                                   float* __restrict__ wt, float* __restrict__ bias) {
+    repack_lstm_body(wih, whh, bih, bhh, K, H, wt, bias);
+}
+__global__ void repack_lstm_batch_kernel(GC PCF wih, GC PCF whh, GC PCF bih, GC PCF bhh, int K, int H, GC PF wt,
+                                         GC PF bias) {
+    const int mi = blockIdx.y;
+    repack_lstm_body(wih[mi], whh[mi], bih[mi], bhh[mi], K, H, wt[mi], bias[mi]);
+}
+
+__global__ void assemble_seq_train_kernel(const float* __restrict__ kmer, const float* __restrict__ means,
+                                          const float* __restrict__ stds, const float* __restrict__ lens,
+                                          const float* __restrict__ embed, int E, int vocab, int use_len, int kseq,
+                                          int64_t rows, float* __restrict__ x, int32_t* __restrict__ codes) {
+    assemble_seq_train_body(kmer, means, stds, lens, embed, E, vocab, use_len, kseq, rows, x, codes);
+}
+__global__ void assemble_seq_train_batch_kernel(GC PCF kmer, GC PCF means, GC PCF stds, GC PCF lens, GC PCF embed,
+                                                int E, int vocab, int use_len, int kseq, int64_t rows, GC PF x,
+                                                GC Per<int32_t> codes) {
+    const int mi = blockIdx.y;
+    assemble_seq_train_body(kmer[mi], means[mi], stds[mi], lens[mi], embed[mi], E, vocab, use_len, kseq, rows, x[mi],
+                            codes[mi]);
+}
+
+// blockIdx.y = direction (batched: model * 2 + direction)
+template <int TS_>
+__global__ void __launch_bounds__(256, 2)
+lstm_train_fwd_kernel(const float* __restrict__ x, int x_row_stride, int x_t_stride, int K,
+                      const float* __restrict__ wt0, const float* __restrict__ wt1,
+                      const float* __restrict__ bias0, const float* __restrict__ bias1,
+                      const float* __restrict__ h0, const float* __restrict__ c0,
+                      int64_t state_dir_stride, float* __restrict__ y, float* __restrict__ gates,
+                      float* __restrict__ cst, int H, int T, int64_t n) {
+    lstm_train_fwd_body<TS_>(blockIdx.y, x, x_row_stride, x_t_stride, K, wt0, wt1, bias0, bias1, h0, c0,
+                             state_dir_stride, y, gates, cst, H, T, n);
+}
+template <int TS_>
+__global__ void __launch_bounds__(256, 2)
+lstm_train_fwd_batch_kernel(GC PCF x, int x_row_stride, int x_t_stride, int K, GC PCF wt0, GC PCF wt1, GC PCF bias0,
+                            GC PCF bias1, GC PCF h0, GC PCF c0, int64_t state_dir_stride, GC PF y, GC PF gates,
+                            GC PF cst, int H, int T, int64_t n) {
+    const int mi = blockIdx.y >> 1;
+    lstm_train_fwd_body<TS_>(blockIdx.y & 1, x[mi], x_row_stride, x_t_stride, K, wt0[mi], wt1[mi], bias0[mi], bias1[mi],
+                             h0[mi], c0[mi], state_dir_stride, y[mi], gates[mi], cst[mi], H, T, n);
+}
+
+// blockIdx.y = direction (batched: model * 2 + direction)
+template <int TS_>
+__global__ void __launch_bounds__(256)
+lstm_train_bwd_kernel(const float* __restrict__ dy, const float* __restrict__ gates, const float* __restrict__ cst,
+                      const float* __restrict__ y, const float* __restrict__ h0, const float* __restrict__ c0,
+                      int64_t state_dir_stride, const float* __restrict__ whh0, const float* __restrict__ whh1,
+                      float* __restrict__ dz, float* __restrict__ hprev, int H, int T, int64_t n) {
+    lstm_train_bwd_body<TS_>(blockIdx.y, dy, gates, cst, y, h0, c0, state_dir_stride, whh0, whh1, dz, hprev, H, T, n);
+}
+template <int TS_>
+__global__ void __launch_bounds__(256)
+lstm_train_bwd_batch_kernel(GC PCF dy, GC PCF gates, GC PCF cst, GC PCF y, GC PCF h0, GC PCF c0,
+                            int64_t state_dir_stride, GC PCF whh0, GC PCF whh1, GC PF dz, GC PF hprev, int H, int T,
+                            int64_t n) {
+    const int mi = blockIdx.y >> 1;
+    lstm_train_bwd_body<TS_>(blockIdx.y & 1, dy[mi], gates[mi], cst[mi], y[mi], h0[mi], c0[mi], state_dir_stride,
+                             whh0[mi], whh1[mi], dz[mi], hprev[mi], H, T, n);
+}
+
+// blockIdx.z = split (batched: model * splits + split)
+__global__ void __launch_bounds__(256)
+gemm_f32_kernel(int M, int N, int K, const float* __restrict__ A, int64_t sam, int64_t sak,
+                const float* __restrict__ B, int64_t sbk, int64_t sbn, float* __restrict__ C, int64_t ldc,
+                const float* __restrict__ bias, int relu, int beta, int kps, int splits, float* __restrict__ partial) {
+    gemm_f32_body(blockIdx.z, M, N, K, A, sam, sak, B, sbk, sbn, C, ldc, bias, relu, beta, kps, partial);
+}
+__global__ void __launch_bounds__(256)
+gemm_f32_batch_kernel(int M, int N, int K, GC PCF A, int64_t sam, int64_t sak, GC PCF B, int64_t sbk, int64_t sbn,
+                      GC PF C, int64_t ldc, GC PCF bias, int relu, int beta, int kps, int splits, GC PF partial) {
+    const int mi = blockIdx.z / splits;
+    gemm_f32_body(blockIdx.z - mi * splits, M, N, K, A[mi], sam, sak, B[mi], sbk, sbn, C[mi], ldc, bias[mi], relu, beta,
+                  kps, partial[mi]);
+}
+
+__global__ void splitk_reduce_kernel(const float* __restrict__ partial, int splits, int M, int N,
+                                     float* __restrict__ C, int64_t ldc, int beta) {
+    splitk_reduce_body(partial, splits, M, N, C, ldc, beta);
+}
+__global__ void splitk_reduce_batch_kernel(GC PCF partial, int splits, int M, int N, GC PF C, int64_t ldc, int beta) {
+    splitk_reduce_body(partial[blockIdx.y], splits, M, N, C[blockIdx.y], ldc, beta);
+}
+
+// blockIdx.y = split (batched: model * splits + split)
+__global__ void colsum_partial_kernel(const float* __restrict__ x, int64_t ld, int64_t rows, int cols, int64_t rps,
+                                      int splits, float* __restrict__ partial) {
+    colsum_partial_body(blockIdx.y, x, ld, rows, cols, rps, partial);
+}
+__global__ void colsum_partial_batch_kernel(GC PCF x, int64_t ld, int64_t rows, int cols, int64_t rps, int splits,
+                                            GC PF partial) {
+    const int mi = blockIdx.y / splits;
+    colsum_partial_body(blockIdx.y - mi * splits, x[mi], ld, rows, cols, rps, partial[mi]);
+}
+
+__global__ void ew_kernel(float* __restrict__ out, int64_t ldo, const float* __restrict__ g, int64_t ldg,
+                          const float* __restrict__ mask, int64_t ldm, const float* __restrict__ act, int64_t lda,
+                          int relu, int64_t rows, int cols) {
+    ew_body(out, ldo, g, ldg, mask, ldm, act, lda, relu, rows, cols);
+}
+__global__ void ew_batch_kernel(GC PF out, int64_t ldo, GC PCF g, int64_t ldg, GC PCF mask, int64_t ldm, GC PCF act,
+                                int64_t lda, int relu, int64_t rows, int cols) {
+    const int mi = blockIdx.y;
+    ew_body(out[mi], ldo, g[mi], ldg, mask[mi], ldm, act[mi], lda, relu, rows, cols);
+}
+
+__global__ void pick_last_kernel(const float* __restrict__ y, int H, int T, int64_t n, const float* __restrict__ mask,
+                                 float* __restrict__ out) {
+    pick_last_body(y, H, T, n, mask, out);
+}
+__global__ void pick_last_batch_kernel(GC PCF y, int H, int T, int64_t n, GC PCF mask, GC PF out) {
+    pick_last_body(y[blockIdx.y], H, T, n, mask[blockIdx.y], out[blockIdx.y]);
+}
+
+__global__ void scatter_last_kernel(const float* __restrict__ dlast, const float* __restrict__ mask, int H, int T,
+                                    int64_t n, float* __restrict__ dy) {
+    scatter_last_body(dlast, mask, H, T, n, dy);
+}
+__global__ void scatter_last_batch_kernel(GC PCF dlast, GC PCF mask, int H, int T, int64_t n, GC PF dy) {
+    scatter_last_body(dlast[blockIdx.y], mask[blockIdx.y], H, T, n, dy[blockIdx.y]);
+}
+
+__global__ void __launch_bounds__(256)
+embed_grad_kernel(const float* __restrict__ dx, int ldx, const int32_t* __restrict__ codes, int64_t rows, int E,
+                  float* __restrict__ grad) {
+    embed_grad_body(dx, ldx, codes, rows, E, grad);
+}
+__global__ void __launch_bounds__(256)
+embed_grad_batch_kernel(GC PCF dx, int ldx, GC Per<const int32_t> codes, int64_t rows, int E, GC PF grad) {
+    embed_grad_body(dx[blockIdx.y], ldx, codes[blockIdx.y], rows, E, grad[blockIdx.y]);
+}
+
+// N(0,1) initial states of model blockIdx.y from its own seed (the one-model case uses philox_normal_kernel).
+__global__ void philox_normal_batch_kernel(GC PF out, int64_t count, GC Seeds seed, uint64_t stream_id) {
+    philox_normal_quad(out[blockIdx.y], count, seed.s[blockIdx.y], stream_id,
+                       (int64_t)blockIdx.x * blockDim.x + threadIdx.x);
+}
+
 // ---------------------------------------------------------------------------------------------------
-// Host side.
+// Host side.  Every launch covers the G models of one call; a buffer is a Per<> table of G pointers at the
+// same offset in each model's region.
 
 unsigned ew_grid(int64_t total) {
     int64_t b = (total + 255) / 256;
@@ -450,30 +632,39 @@ Shape shape_of(const Model* m) {
     return s;
 }
 
-// Byte layout of a region: sections appended at 256-byte alignment.
+// Entry k of every model's slice of a flat [G][stride] pointer list.
+template <class T>
+Per<T> gather(T* const* list, int G, int stride, int k) {
+    Per<T> r;
+    for (int i = 0; i < G; ++i) r.p[i] = list[(int64_t)i * stride + k];
+    return r;
+}
+
+// Byte layout of a region: sections appended at 256-byte alignment.  With null bases only sizes are computed.
 struct Bump {
-    char* base; size_t off = 0;
-    explicit Bump(void* b) : base((char*)b) {}
-    template <class X> X* take(int64_t count) {
-        X* p = base ? (X*)(base + off) : nullptr;
+    Per<char> base; size_t off = 0;
+    explicit Bump(const Per<char>& b) : base(b) {}
+    template <class X> Per<X> take(int64_t count) {
+        Per<X> p;
+        for (int i = 0; i < MAXG; ++i) p.p[i] = base.p[i] ? (X*)(base.p[i] + off) : nullptr;
         off += ((size_t)count * sizeof(X) + 255) & ~(size_t)255;
         return p;
     }
 };
 
 struct LayerAct {            // saved activations of one LSTM layer
-    float* y; float* ym; float* gates; float* cst;
-    float* wt[2]; float* bias[2];
+    PF y; PF ym; PF gates; PF cst;
+    PF wt[2]; PF bias[2];
 };
 
-// The arena: everything backward needs from one forward.  With base == nullptr only sizes are computed.
+// The arena: everything backward needs from one forward.
 struct Arena {
     std::vector<LayerAct> layer[3];
-    float* h0[3] = {}; float* c0[3] = {};
-    float* xseq = nullptr; int32_t* codes = nullptr; float* sig = nullptr;
-    float* comb_in = nullptr; float* in1 = nullptr; float* z1 = nullptr; float* a2 = nullptr;
+    PF h0[3], c0[3];
+    PF xseq; Per<int32_t> codes; PF sig;
+    PF comb_in, in1, z1, a2;
     size_t bytes = 0;
-    Arena(const Shape& s, int64_t n, void* base) {
+    Arena(const Shape& s, int64_t n, const Per<char>& base) {
         Bump b(base);
         const int64_t NT = n * s.T;
         for (int g = 0; g < 3; ++g) {
@@ -485,7 +676,7 @@ struct Arena {
                 const int K = l ? 2 * k.H : k.K0;
                 LayerAct a;
                 a.y = b.take<float>(NT * 2 * k.H);
-                a.ym = (l + 1 < k.layers) ? b.take<float>(NT * 2 * k.H) : nullptr;
+                if (l + 1 < k.layers) a.ym = b.take<float>(NT * 2 * k.H);
                 a.gates = b.take<float>(NT * 2 * 4 * k.H);
                 a.cst = b.take<float>(NT * 2 * k.H);
                 for (int d = 0; d < 2; ++d) {
@@ -507,11 +698,11 @@ struct Arena {
 
 // Backward scratch.
 struct Work {
-    float* dy[2]; float* dz; float* hprev; float* dcomb; float* dfc; float* dxseq;
-    float* dlast; float* da2; float* dz1; float* dbias; float* partial;
+    PF dy[2]; PF dz; PF hprev; PF dcomb; PF dfc; PF dxseq;
+    PF dlast; PF da2; PF dz1; PF dbias; PF partial;
     int64_t partial_floats;
     size_t bytes;
-    Work(const Shape& s, int64_t n, void* base) {
+    Work(const Shape& s, int64_t n, const Per<char>& base) {
         Bump b(base);
         const int64_t NT = n * s.T;
         int64_t maxmn = 8 * (int64_t)s.H, hmax = s.H;
@@ -545,25 +736,26 @@ struct Work {
 
 // Parameter (or gradient) pointers in state_dict order (models.py:131-161 creation order):
 // embed, lstm_seq (8 per layer: weight_ih, weight_hh, bias_ih, bias_hh, then the same for _reverse), fc_seq,
-// lstm_signal, fc_signal, lstm_comb, fc1, fc2.
-template <class P>
+// lstm_signal, fc_signal, lstm_comb, fc1, fc2.  `list` holds G such lists back to back.
+template <class T>
 struct Slots {
-    P* embed = nullptr;
-    std::vector<std::array<P*, 8>> lstm[3];
-    P* fcw[2] = {}; P* fcb[2] = {};
-    P* head[4] = {};             // fc1.weight, fc1.bias, fc2.weight, fc2.bias
-    Slots(const Shape& s, P* list) {
+    Per<T> embed;
+    std::vector<std::array<Per<T>, 8>> lstm[3];
+    Per<T> fcw[2], fcb[2];
+    Per<T> head[4];              // fc1.weight, fc1.bias, fc2.weight, fc2.bias
+    Slots(const Shape& s, T* const* list, int G) {
         int i = 0;
-        if (s.seq) embed = &list[i++];
+        auto next = [&]() { return gather(list, G, s.n_params, i++); };
+        if (s.seq) embed = next();
         for (int g = 0; g < 3; ++g) {
             for (int l = 0; l < s.st[g].layers; ++l) {
-                std::array<P*, 8> a;
-                for (int q = 0; q < 8; ++q) a[q] = &list[i++];
+                std::array<Per<T>, 8> a;
+                for (int q = 0; q < 8; ++q) a[q] = next();
                 lstm[g].push_back(a);
             }
-            if (g < 2 && s.st[g].layers) { fcw[g] = &list[i++]; fcb[g] = &list[i++]; }
+            if (g < 2 && s.st[g].layers) { fcw[g] = next(); fcb[g] = next(); }
         }
-        for (int q = 0; q < 4; ++q) head[q] = &list[i++];
+        for (int q = 0; q < 4; ++q) head[q] = next();
     }
 };
 
@@ -574,8 +766,27 @@ void mask_bases(const Model* m, int base[3]) {
     base[2] = 2 * (m->cfg.num_layers2 - 1);
 }
 
-int launch_gemm(Model* m, int M, int N, int K, const float* A, int64_t sam, int64_t sak, const float* B, int64_t sbk,
-                int64_t sbn, float* C, int64_t ldc, const float* bias, int relu, int beta, const Work* w, cudaStream_t st) {
+// A table passes its model-0 entry to a one-model entry point; everything else passes through.
+template <class T> T* one(const Per<T>& t) { return t.p[0]; }
+template <class T> const T& one(const T& v) { return v; }
+
+// One launch for the G models of a call: the plain-parameter entry point for G = 1, the table entry point otherwise.
+template <class K1, class KG, class... Args>
+int launch_models(Model* m, int G, K1 k1, KG kg, dim3 grid, unsigned block, size_t smem, cudaStream_t st,
+                  const Args&... args) {
+    if (G == 1)
+        k1<<<grid, block, smem, st>>>(one(args)...);
+    else
+        kg<<<grid, block, smem, st>>>(args...);
+    m->launches++;
+    DSP_CUDA(cudaGetLastError());
+    return DSP_OK;
+}
+
+#define RC(x) do { int rc__ = (x); if (rc__) return rc__; } while (0)
+
+int launch_gemm(Model* m, int G, int M, int N, int K, PCF A, int64_t sam, int64_t sak, PCF B, int64_t sbk, int64_t sbn,
+                PF C, int64_t ldc, PCF bias, int relu, int beta, const Work* w, cudaStream_t st) {
     if (M == 0 || N == 0) return DSP_OK;
     int splits = 1, kps = K;
     if (w) {
@@ -584,49 +795,40 @@ int launch_gemm(Model* m, int M, int N, int K, const float* A, int64_t sam, int6
         splits = (K + kps - 1) / kps;
         if (splits < 1) splits = 1;
     }
-    float* partial = (w && splits > 1) ? w->partial : nullptr;
+    PF partial = (w && splits > 1) ? w->partial : PF();
     if (partial && (int64_t)splits * M * N > w->partial_floats) {
         set_error("training GEMM %dx%d needs more split-K scratch than reserved", M, N);
         return DSP_ERR_INVALID;
     }
-    dim3 grid((unsigned)((M + GBM - 1) / GBM), (unsigned)((N + GBN - 1) / GBN), (unsigned)splits);
-    gemm_f32_kernel<<<grid, 256, 0, st>>>(M, N, K, A, sam, sak, B, sbk, sbn, C, ldc, bias, relu, beta, kps, partial);
-    m->launches++;
-    DSP_CUDA(cudaGetLastError());
+    dim3 grid((unsigned)((M + GBM - 1) / GBM), (unsigned)((N + GBN - 1) / GBN), (unsigned)(splits * G));
+    RC(launch_models(m, G, gemm_f32_kernel, gemm_f32_batch_kernel, grid, 256, 0, st, M, N, K, A, sam, sak, B, sbk, sbn,
+                     C, ldc, bias, relu, beta, kps, splits, partial));
     if (partial) {
         DSP_REQUIRE(!bias && !relu, DSP_ERR_INVALID, "split-K GEMM has no bias/ReLU epilogue");
-        splitk_reduce_kernel<<<ew_grid((int64_t)M * N), 256, 0, st>>>(partial, splits, M, N, C, ldc, beta);
-        m->launches++;
-        DSP_CUDA(cudaGetLastError());
+        RC(launch_models(m, G, splitk_reduce_kernel, splitk_reduce_batch_kernel, dim3(ew_grid((int64_t)M * N), G), 256,
+                         0, st, PCF(partial), splits, M, N, C, ldc, beta));
     }
     return DSP_OK;
 }
 
 // out[c] = sum over rows of x[r][c], fixed-order split over rows.
-int launch_colsum(Model* m, const float* x, int64_t ld, int64_t rows, int cols, float* out, const Work& w, cudaStream_t st) {
+int launch_colsum(Model* m, int G, PCF x, int64_t ld, int64_t rows, int cols, PF out, const Work& w, cudaStream_t st) {
     const int64_t splits0 = splits_for(rows), rps = (rows + splits0 - 1) / splits0;
     const int splits = (int)((rows + rps - 1) / rps);
     DSP_REQUIRE((int64_t)splits * cols <= w.partial_floats, DSP_ERR_INVALID, "bias gradient scratch too small");
-    dim3 grid((unsigned)((cols + 255) / 256), (unsigned)splits);
-    colsum_partial_kernel<<<grid, 256, 0, st>>>(x, ld, rows, cols, rps, w.partial);
-    m->launches++;
-    DSP_CUDA(cudaGetLastError());
-    splitk_reduce_kernel<<<ew_grid(cols), 256, 0, st>>>(w.partial, splits, 1, cols, out, cols, 0);
-    m->launches++;
-    DSP_CUDA(cudaGetLastError());
-    return DSP_OK;
+    dim3 grid((unsigned)((cols + 255) / 256), (unsigned)(splits * G));
+    RC(launch_models(m, G, colsum_partial_kernel, colsum_partial_batch_kernel, grid, 256, 0, st, x, ld, rows, cols, rps,
+                     splits, w.partial));
+    return launch_models(m, G, splitk_reduce_kernel, splitk_reduce_batch_kernel, dim3(ew_grid(cols), G), 256, 0, st,
+                         PCF(w.partial), splits, 1, cols, out, (int64_t)cols, 0);
 }
 
-int launch_ew(Model* m, float* out, int64_t ldo, const float* g, int64_t ldg, const float* mask, int64_t ldm,
-              const float* act, int64_t lda, int relu, int64_t rows, int cols, cudaStream_t st) {
+int launch_ew(Model* m, int G, PF out, int64_t ldo, PCF g, int64_t ldg, PCF mask, int64_t ldm, PCF act, int64_t lda,
+              int relu, int64_t rows, int cols, cudaStream_t st) {
     if (rows * cols == 0) return DSP_OK;
-    ew_kernel<<<ew_grid(rows * cols), 256, 0, st>>>(out, ldo, g, ldg, mask, ldm, act, lda, relu, rows, cols);
-    m->launches++;
-    DSP_CUDA(cudaGetLastError());
-    return DSP_OK;
+    return launch_models(m, G, ew_kernel, ew_batch_kernel, dim3(ew_grid(rows * cols), G), 256, 0, st, out, ldo, g, ldg,
+                         mask, ldm, act, lda, relu, rows, cols);
 }
-
-#define RC(x) do { int rc__ = (x); if (rc__) return rc__; } while (0)
 
 }  // namespace
 
@@ -637,30 +839,45 @@ int train_shape(const Model* m, int32_t* n_params, int32_t* n_masks) {
     return DSP_OK;
 }
 
-int64_t train_arena_bytes(const Model* m, int64_t n) { return (int64_t)Arena(shape_of(m), n, nullptr).bytes; }
-int64_t train_workspace_bytes(const Model* m, int64_t n) { return (int64_t)Work(shape_of(m), n, nullptr).bytes; }
+int64_t train_arena_bytes(const Model* m, int64_t n) { return (int64_t)Arena(shape_of(m), n, Per<char>()).bytes; }
+int64_t train_workspace_bytes(const Model* m, int64_t n) { return (int64_t)Work(shape_of(m), n, Per<char>()).bytes; }
 
-int train_forward(Model* m, const float* const* params, const float* kmer, const float* means, const float* stds,
-                  const float* lens, const float* signals, const float* const* states6, uint64_t seed,
-                  const float* const* masks, int64_t n, void* arena, float* logits, cudaStream_t st) {
+int train_forward(Model* m, int G, const float* const* params, const float* const* inputs, const float* const* states6,
+                  const uint64_t* seeds, const float* const* masks, int64_t n, void* const* arenas, float* const* logits,
+                  cudaStream_t st) {
     const Shape s = shape_of(m);
-    Arena A(s, n, arena);
-    Slots<const float* const> P(s, params);
+    Arena A(s, n, gather((char* const*)arenas, G, 1, 0));
+    Slots<const float> P(s, params, G);
     const int T = s.T, H = s.H;
     const int64_t NT = n * T;
+    auto mask = [&](int k) { return gather(masks, G, s.n_masks, k); };
 
     // initial states: copied from the caller or drawn (Philox, one stream per group); backward reads them here
+    Seeds seed;
+    for (int i = 0; i < G; ++i) seed.s[i] = seeds[i];
     for (int g = 0; g < 3; ++g) {
         const Stack& k = s.st[g];
         if (!k.layers) continue;
         const int64_t cnt = (int64_t)k.layers * 2 * n * k.H;
         if (states6) {
-            DSP_REQUIRE(states6[2 * g] && states6[2 * g + 1], DSP_ERR_INVALID, "dsp_train_forward: states[%d] is null", 2 * g);
-            DSP_CUDA(cudaMemcpyAsync(A.h0[g], states6[2 * g], cnt * sizeof(float), cudaMemcpyDeviceToDevice, st));
-            DSP_CUDA(cudaMemcpyAsync(A.c0[g], states6[2 * g + 1], cnt * sizeof(float), cudaMemcpyDeviceToDevice, st));
+            for (int i = 0; i < G; ++i) {
+                DSP_CUDA(cudaMemcpyAsync(A.h0[g].p[i], states6[6 * i + 2 * g], cnt * sizeof(float), cudaMemcpyDeviceToDevice, st));
+                DSP_CUDA(cudaMemcpyAsync(A.c0[g].p[i], states6[6 * i + 2 * g + 1], cnt * sizeof(float),
+                                         cudaMemcpyDeviceToDevice, st));
+            }
         } else {
-            RC(philox_normal(m, A.h0[g], cnt, seed, 2 * g, st));
-            RC(philox_normal(m, A.c0[g], cnt, seed, 2 * g + 1, st));
+            for (int hc = 0; hc < 2; ++hc) {
+                PF out = hc ? A.c0[g] : A.h0[g];
+                if (G == 1) {
+                    RC(philox_normal(m, out.p[0], cnt, seeds[0], 2 * g + hc, st));
+                    continue;
+                }
+                const int64_t quads = (cnt + 3) / 4;
+                philox_normal_batch_kernel<<<dim3((unsigned)((quads + 255) / 256), G), 256, 0, st>>>(out, cnt, seed,
+                                                                                                     2 * g + hc);
+                m->launches++;
+                DSP_CUDA(cudaGetLastError());
+            }
         }
     }
     // weights of every LSTM layer -> the forward kernel's layout, in the arena
@@ -669,106 +886,112 @@ int train_forward(Model* m, const float* const* params, const float* kmer, const
             const int K = l ? 2 * s.st[g].H : s.st[g].K0, Hh = s.st[g].H;
             for (int d = 0; d < 2; ++d) {
                 const int64_t total = (int64_t)(ru(K, 4) + ru(Hh, 4)) * 4 * Hh;
-                repack_lstm_kernel<<<ew_grid(total), 256, 0, st>>>(
-                    *P.lstm[g][l][4 * d], *P.lstm[g][l][4 * d + 1], *P.lstm[g][l][4 * d + 2], *P.lstm[g][l][4 * d + 3],
-                    K, Hh, A.layer[g][l].wt[d], A.layer[g][l].bias[d]);
-                m->launches++;
-                DSP_CUDA(cudaGetLastError());
+                RC(launch_models(m, G, repack_lstm_kernel, repack_lstm_batch_kernel, dim3(ew_grid(total), G), 256, 0, st,
+                                 P.lstm[g][l][4 * d], P.lstm[g][l][4 * d + 1], P.lstm[g][l][4 * d + 2],
+                                 P.lstm[g][l][4 * d + 3], K, Hh, A.layer[g][l].wt[d], A.layer[g][l].bias[d]));
             }
         }
     DSP_CUDA(cudaFuncSetAttribute(lstm_train_fwd_kernel<TS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    DSP_CUDA(cudaFuncSetAttribute(lstm_train_fwd_batch_kernel<TS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  227 * 1024));
 
-    // one stack: layers in order, inter-layer dropout on every output but the last
+    // one stack: layers in order, inter-layer dropout on every output but the last; its output goes to `out`
     int mask_base[3];
     mask_bases(m, mask_base);
-    auto run_stack = [&](int g, const float* x, int xs, int xt) -> const float* {
+    auto run_stack = [&](int g, PCF x, int xs, int xt, PCF& out) -> int {
         const Stack& k = s.st[g];
         const int64_t sstride = n * k.H;
         for (int l = 0; l < k.layers; ++l) {
             const int K = l ? 2 * k.H : k.K0;
             LayerAct& a = A.layer[g][l];
             const size_t smem = sizeof(float) * TS * (size_t)(ru(K, 4) + 3 * ru(k.H, 4));
-            if (smem > 227 * 1024) { set_error("training LSTM layer K=%d H=%d exceeds shared memory", K, k.H); return nullptr; }
+            DSP_REQUIRE(smem <= 227 * 1024, DSP_ERR_INVALID, "training LSTM layer K=%d H=%d exceeds shared memory", K, k.H);
             const int threads = k.H >= 256 ? 256 : ru(k.H, 32);
-            lstm_train_fwd_kernel<TS><<<dim3((unsigned)((n + TS - 1) / TS), 2), threads, smem, st>>>(
-                x, xs, xt, K, a.wt[0], a.wt[1], a.bias[0], a.bias[1], A.h0[g] + (int64_t)l * 2 * sstride,
-                A.c0[g] + (int64_t)l * 2 * sstride, sstride, a.y, a.gates, a.cst, k.H, T, n);
-            m->launches++;
-            if (cudaGetLastError() != cudaSuccess) { set_error("lstm_train_fwd_kernel launch failed"); return nullptr; }
+            RC(launch_models(m, G, lstm_train_fwd_kernel<TS>, lstm_train_fwd_batch_kernel<TS>,
+                             dim3((unsigned)((n + TS - 1) / TS), 2 * G), threads, smem, st, x, xs, xt, K, a.wt[0], a.wt[1],
+                             a.bias[0], a.bias[1], A.h0[g] + (int64_t)l * 2 * sstride, A.c0[g] + (int64_t)l * 2 * sstride,
+                             sstride, a.y, a.gates, a.cst, k.H, T, n));
             x = a.y;
-            const float* mk = (l + 1 < k.layers) ? masks[mask_base[g] + l] : nullptr;
+            const PCF mk = (l + 1 < k.layers) ? mask(mask_base[g] + l) : PCF();
             if (mk) {
-                if (launch_ew(m, a.ym, 2 * k.H, a.y, 2 * k.H, mk, 2 * k.H, nullptr, 0, 0, NT, 2 * k.H, st)) return nullptr;
+                RC(launch_ew(m, G, a.ym, 2 * k.H, a.y, 2 * k.H, mk, 2 * k.H, PCF(), 0, 0, NT, 2 * k.H, st));
                 x = a.ym;
             }
             xs = T * 2 * k.H; xt = 2 * k.H;
         }
-        return x;
+        out = x;
+        return DSP_OK;
     };
 
     int comb_off = 0;
     if (s.seq) {
-        assemble_seq_train_kernel<<<(unsigned)((NT + 255) / 256), 256, 0, st>>>(
-            kmer, means, stds, lens, *P.embed, s.E, m->cfg.vocab_size, m->cfg.is_signallen, s.kseq, NT, A.xseq, A.codes);
-        m->launches++;
-        DSP_CUDA(cudaGetLastError());
-        const float* y = run_stack(0, A.xseq, T * s.kseq, s.kseq);
-        if (!y) return DSP_ERR_CUDA;
+        RC(launch_models(m, G, assemble_seq_train_kernel, assemble_seq_train_batch_kernel,
+                         dim3((unsigned)((NT + 255) / 256), G), 256, 0, st, gather(inputs, G, 5, 0), gather(inputs, G, 5, 1),
+                         gather(inputs, G, 5, 2), gather(inputs, G, 5, 3), P.embed, s.E, m->cfg.vocab_size,
+                         m->cfg.is_signallen, s.kseq, NT, A.xseq, A.codes));
+        PCF y;
+        RC(run_stack(0, A.xseq, T * s.kseq, s.kseq, y));
         const int hs = s.st[0].H;
-        RC(launch_gemm(m, (int)NT, hs, 2 * hs, y, 2 * hs, 1, *P.fcw[0], 1, 2 * hs, A.comb_in, H, *P.fcb[0], 1, 0, nullptr, st));
+        RC(launch_gemm(m, G, (int)NT, hs, 2 * hs, y, 2 * hs, 1, P.fcw[0], 1, 2 * hs, A.comb_in, H, P.fcb[0], 1, 0, nullptr,
+                       st));
         comb_off = hs;
     }
     if (s.sig) {
-        DSP_CUDA(cudaMemcpyAsync(A.sig, signals, NT * s.S * sizeof(float), cudaMemcpyDeviceToDevice, st));
-        const float* y = run_stack(1, A.sig, T * s.S, s.S);
-        if (!y) return DSP_ERR_CUDA;
+        for (int i = 0; i < G; ++i)
+            DSP_CUDA(cudaMemcpyAsync(A.sig.p[i], inputs[5 * i + 4], NT * s.S * sizeof(float), cudaMemcpyDeviceToDevice, st));
+        PCF y;
+        RC(run_stack(1, A.sig, T * s.S, s.S, y));
         const int hs = s.st[1].H;
-        RC(launch_gemm(m, (int)NT, hs, 2 * hs, y, 2 * hs, 1, *P.fcw[1], 1, 2 * hs, A.comb_in + comb_off, H, *P.fcb[1], 1, 0,
-                       nullptr, st));
+        RC(launch_gemm(m, G, (int)NT, hs, 2 * hs, y, 2 * hs, 1, P.fcw[1], 1, 2 * hs, A.comb_in + comb_off, H, P.fcb[1], 1,
+                       0, nullptr, st));
     }
-    const float* y = run_stack(2, A.comb_in, T * H, H);
-    if (!y) return DSP_ERR_CUDA;
+    PCF y;
+    RC(run_stack(2, A.comb_in, T * H, H, y));
     // head: dropout -> fc1 -> dropout -> ReLU -> fc2 (models.py:229-238)
-    const float* m1 = masks[s.n_masks - 2];
-    const float* m2 = masks[s.n_masks - 1];
-    pick_last_kernel<<<ew_grid(n * 2 * H), 256, 0, st>>>(y, H, T, n, m1, A.in1);
-    m->launches++;
-    DSP_CUDA(cudaGetLastError());
-    RC(launch_gemm(m, (int)n, H, 2 * H, A.in1, 2 * H, 1, *P.head[0], 1, 2 * H, A.z1, H, *P.head[1], 0, 0, nullptr, st));
-    RC(launch_ew(m, A.a2, H, A.z1, H, m2, H, nullptr, 0, 1, n, H, st));
-    RC(launch_gemm(m, (int)n, s.C, H, A.a2, H, 1, *P.head[2], 1, H, logits, s.C, *P.head[3], 0, 0, nullptr, st));
+    const PCF m1 = mask(s.n_masks - 2);
+    const PCF m2 = mask(s.n_masks - 1);
+    RC(launch_models(m, G, pick_last_kernel, pick_last_batch_kernel, dim3(ew_grid(n * 2 * H), G), 256, 0, st, y, H, T, n,
+                     m1, A.in1));
+    RC(launch_gemm(m, G, (int)n, H, 2 * H, A.in1, 2 * H, 1, P.head[0], 1, 2 * H, A.z1, H, P.head[1], 0, 0, nullptr, st));
+    RC(launch_ew(m, G, A.a2, H, A.z1, H, m2, H, PCF(), 0, 1, n, H, st));
+    RC(launch_gemm(m, G, (int)n, s.C, H, A.a2, H, 1, P.head[2], 1, H, gather(logits, G, 1, 0), s.C, P.head[3], 0, 0,
+                   nullptr, st));
     return DSP_OK;
 }
 
-int train_backward(Model* m, const float* const* params, const float* const* masks, const void* arena,
-                   const float* dlogits, int64_t n, void* workspace, float* const* grads, cudaStream_t st) {
+int train_backward(Model* m, int G, const float* const* params, const float* const* masks, const void* const* arenas,
+                   const float* const* dlogits_, int64_t n, void* const* workspaces, float* const* grads, cudaStream_t st) {
     const Shape s = shape_of(m);
-    Arena A(s, n, const_cast<void*>(arena));
-    Work W(s, n, workspace);
-    Slots<const float* const> P(s, params);
-    Slots<float* const> G(s, grads);
+    Arena A(s, n, gather((char* const*)arenas, G, 1, 0));
+    Work W(s, n, gather((char* const*)workspaces, G, 1, 0));
+    Slots<const float> P(s, params, G);
+    Slots<float> Gr(s, grads, G);
     const int T = s.T, H = s.H, C = s.C;
     const int64_t NT = n * T;
-    const float* m1 = masks[s.n_masks - 2];
-    const float* m2 = masks[s.n_masks - 1];
+    auto mask = [&](int k) { return gather(masks, G, s.n_masks, k); };
+    const PCF m1 = mask(s.n_masks - 2);
+    const PCF m2 = mask(s.n_masks - 1);
+    const PCF dlogits = gather(dlogits_, G, 1, 0);
+    const PCF none;
 
     // head (models.py:234-238)
-    RC(launch_gemm(m, C, H, (int)n, dlogits, 1, C, A.a2, H, 1, *G.head[2], H, nullptr, 0, 0, &W, st));      // dW2
-    RC(launch_colsum(m, dlogits, C, n, C, *G.head[3], W, st));                                               // db2
-    RC(launch_gemm(m, (int)n, H, C, dlogits, C, 1, *P.head[2], H, 1, W.da2, H, nullptr, 0, 0, nullptr, st)); // da2
-    RC(launch_ew(m, W.dz1, H, W.da2, H, m2, H, A.a2, H, 0, n, H, st));
-    RC(launch_gemm(m, H, 2 * H, (int)n, W.dz1, 1, H, A.in1, 2 * H, 1, *G.head[0], 2 * H, nullptr, 0, 0, &W, st)); // dW1
-    RC(launch_colsum(m, W.dz1, H, n, H, *G.head[1], W, st));                                                        // db1
-    RC(launch_gemm(m, (int)n, 2 * H, H, W.dz1, H, 1, *P.head[0], 2 * H, 1, W.dlast, 2 * H, nullptr, 0, 0, nullptr, st));
-    scatter_last_kernel<<<ew_grid(NT * 2 * H), 256, 0, st>>>(W.dlast, m1, H, T, n, W.dy[0]);
-    m->launches++;
-    DSP_CUDA(cudaGetLastError());
+    RC(launch_gemm(m, G, C, H, (int)n, dlogits, 1, C, A.a2, H, 1, Gr.head[2], H, none, 0, 0, &W, st));      // dW2
+    RC(launch_colsum(m, G, dlogits, C, n, C, Gr.head[3], W, st));                                           // db2
+    RC(launch_gemm(m, G, (int)n, H, C, dlogits, C, 1, P.head[2], H, 1, W.da2, H, none, 0, 0, nullptr, st)); // da2
+    RC(launch_ew(m, G, W.dz1, H, W.da2, H, m2, H, A.a2, H, 0, n, H, st));
+    RC(launch_gemm(m, G, H, 2 * H, (int)n, W.dz1, 1, H, A.in1, 2 * H, 1, Gr.head[0], 2 * H, none, 0, 0, &W, st)); // dW1
+    RC(launch_colsum(m, G, W.dz1, H, n, H, Gr.head[1], W, st));                                                    // db1
+    RC(launch_gemm(m, G, (int)n, 2 * H, H, W.dz1, H, 1, P.head[0], 2 * H, 1, W.dlast, 2 * H, none, 0, 0, nullptr, st));
+    RC(launch_models(m, G, scatter_last_kernel, scatter_last_batch_kernel, dim3(ew_grid(NT * 2 * H), G), 256, 0, st,
+                     PCF(W.dlast), m1, H, T, n, W.dy[0]));
 
     DSP_CUDA(cudaFuncSetAttribute(lstm_train_bwd_kernel<TS>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    DSP_CUDA(cudaFuncSetAttribute(lstm_train_bwd_batch_kernel<TS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  227 * 1024));
     int mask_base[3];
     mask_bases(m, mask_base);
     // one stack top-down; dY of its last layer is in W.dy[0]; dX of layer 0 goes to dx0 (ld = K0) unless dx0 is null
-    auto back_stack = [&](int g, const float* x0, int ldx0, float* dx0) -> int {
+    auto back_stack = [&](int g, PCF x0, int ldx0, PF dx0) -> int {
         const Stack& k = s.st[g];
         const int64_t sstride = n * k.H;
         const int Hh = k.H;
@@ -776,39 +999,41 @@ int train_backward(Model* m, const float* const* params, const float* const* mas
         for (int l = k.layers - 1; l >= 0; --l) {
             const LayerAct& a = A.layer[g][l];
             const int K = l ? 2 * Hh : k.K0;
-            const float* x = l ? (A.layer[g][l - 1].ym && masks[mask_base[g] + l - 1] ? A.layer[g][l - 1].ym
-                                                                                       : A.layer[g][l - 1].y)
-                               : x0;
+            const PCF x = l ? (A.layer[g][l - 1].ym && mask(mask_base[g] + l - 1) ? A.layer[g][l - 1].ym
+                                                                                   : A.layer[g][l - 1].y)
+                            : x0;
             const int ldx = l ? 2 * Hh : ldx0;
             const size_t smem = sizeof(float) * TS * (size_t)(4 * Hh + 2 * Hh);
             DSP_REQUIRE(smem <= 227 * 1024, DSP_ERR_INVALID, "training LSTM backward H=%d exceeds shared memory", Hh);
             const int threads = Hh >= 256 ? 256 : ru(Hh, 32);
-            lstm_train_bwd_kernel<TS><<<dim3((unsigned)((n + TS - 1) / TS), 2), threads, smem, st>>>(
-                W.dy[cur], a.gates, a.cst, a.y, A.h0[g] + (int64_t)l * 2 * sstride, A.c0[g] + (int64_t)l * 2 * sstride,
-                sstride, *P.lstm[g][l][1], *P.lstm[g][l][5], W.dz, W.hprev, Hh, T, n);
-            m->launches++;
-            DSP_CUDA(cudaGetLastError());
+            RC(launch_models(m, G, lstm_train_bwd_kernel<TS>, lstm_train_bwd_batch_kernel<TS>,
+                             dim3((unsigned)((n + TS - 1) / TS), 2 * G), threads, smem, st, PCF(W.dy[cur]), PCF(a.gates),
+                             PCF(a.cst), PCF(a.y), PCF(A.h0[g] + (int64_t)l * 2 * sstride),
+                             PCF(A.c0[g] + (int64_t)l * 2 * sstride), sstride, P.lstm[g][l][1], P.lstm[g][l][5], W.dz,
+                             W.hprev, Hh, T, n));
             for (int d = 0; d < 2; ++d) {
-                const float* dzd = W.dz + d * 4 * Hh;
-                RC(launch_gemm(m, 4 * Hh, K, (int)NT, dzd, 1, 8 * Hh, x, ldx, 1, *G.lstm[g][l][4 * d], K, nullptr, 0, 0, &W, st));
-                RC(launch_gemm(m, 4 * Hh, Hh, (int)NT, dzd, 1, 8 * Hh, W.hprev + d * Hh, 2 * Hh, 1, *G.lstm[g][l][4 * d + 1],
-                               Hh, nullptr, 0, 0, &W, st));
+                const PCF dzd = W.dz + d * 4 * Hh;
+                RC(launch_gemm(m, G, 4 * Hh, K, (int)NT, dzd, 1, 8 * Hh, x, ldx, 1, Gr.lstm[g][l][4 * d], K, none, 0, 0, &W,
+                               st));
+                RC(launch_gemm(m, G, 4 * Hh, Hh, (int)NT, dzd, 1, 8 * Hh, W.hprev + d * Hh, 2 * Hh, 1,
+                               Gr.lstm[g][l][4 * d + 1], Hh, none, 0, 0, &W, st));
             }
-            RC(launch_colsum(m, W.dz, 8 * Hh, NT, 8 * Hh, W.dbias, W, st));
-            for (int d = 0; d < 2; ++d) {
-                DSP_CUDA(cudaMemcpyAsync(*G.lstm[g][l][4 * d + 2], W.dbias + d * 4 * Hh, 4 * Hh * sizeof(float),
-                                         cudaMemcpyDeviceToDevice, st));
-                DSP_CUDA(cudaMemcpyAsync(*G.lstm[g][l][4 * d + 3], W.dbias + d * 4 * Hh, 4 * Hh * sizeof(float),
-                                         cudaMemcpyDeviceToDevice, st));
-            }
-            float* dx = l ? W.dy[cur ^ 1] : dx0;
+            RC(launch_colsum(m, G, W.dz, 8 * Hh, NT, 8 * Hh, W.dbias, W, st));
+            for (int i = 0; i < G; ++i)
+                for (int d = 0; d < 2; ++d) {
+                    DSP_CUDA(cudaMemcpyAsync(Gr.lstm[g][l][4 * d + 2].p[i], W.dbias.p[i] + d * 4 * Hh, 4 * Hh * sizeof(float),
+                                             cudaMemcpyDeviceToDevice, st));
+                    DSP_CUDA(cudaMemcpyAsync(Gr.lstm[g][l][4 * d + 3].p[i], W.dbias.p[i] + d * 4 * Hh, 4 * Hh * sizeof(float),
+                                             cudaMemcpyDeviceToDevice, st));
+                }
+            const PF dx = l ? W.dy[cur ^ 1] : dx0;
             if (!dx) break;
             for (int d = 0; d < 2; ++d)
-                RC(launch_gemm(m, (int)NT, K, 4 * Hh, W.dz + d * 4 * Hh, 8 * Hh, 1, *P.lstm[g][l][4 * d], K, 1, dx, K,
-                               nullptr, 0, d, nullptr, st));
+                RC(launch_gemm(m, G, (int)NT, K, 4 * Hh, W.dz + d * 4 * Hh, 8 * Hh, 1, P.lstm[g][l][4 * d], K, 1, dx, K,
+                               none, 0, d, nullptr, st));
             if (l) {
-                const float* mk = masks[mask_base[g] + l - 1];
-                if (mk) RC(launch_ew(m, dx, K, dx, K, mk, K, nullptr, 0, 0, NT, K, st));
+                const PCF mk = mask(mask_base[g] + l - 1);
+                if (mk) RC(launch_ew(m, G, dx, K, dx, K, mk, K, none, 0, 0, NT, K, st));
                 cur ^= 1;
             }
         }
@@ -820,24 +1045,25 @@ int train_backward(Model* m, const float* const* params, const float* const* mas
     for (int g = 0; g < 2; ++g) {
         if (!s.st[g].layers) continue;
         const int hs = s.st[g].H;
-        const float* ytop = A.layer[g].back().y;
-        float* dfc = W.dfc;
+        const PF ytop = A.layer[g].back().y;
+        const PF dfc = W.dfc;
         // ReLU backward of the branch fc (models.py:199-201 / 215-217): comb_in holds relu(z)
-        RC(launch_ew(m, dfc, hs, W.dcomb + comb_off, H, nullptr, 0, A.comb_in + comb_off, H, 0, NT, hs, st));
-        RC(launch_gemm(m, hs, 2 * hs, (int)NT, dfc, 1, hs, ytop, 2 * hs, 1, *G.fcw[g], 2 * hs, nullptr, 0, 0, &W, st));
-        RC(launch_colsum(m, dfc, hs, NT, hs, *G.fcb[g], W, st));
-        RC(launch_gemm(m, (int)NT, 2 * hs, hs, dfc, hs, 1, *P.fcw[g], 2 * hs, 1, W.dy[0], 2 * hs, nullptr, 0, 0, nullptr, st));
+        RC(launch_ew(m, G, dfc, hs, W.dcomb + comb_off, H, none, 0, A.comb_in + comb_off, H, 0, NT, hs, st));
+        RC(launch_gemm(m, G, hs, 2 * hs, (int)NT, dfc, 1, hs, ytop, 2 * hs, 1, Gr.fcw[g], 2 * hs, none, 0, 0, &W, st));
+        RC(launch_colsum(m, G, dfc, hs, NT, hs, Gr.fcb[g], W, st));
+        RC(launch_gemm(m, G, (int)NT, 2 * hs, hs, dfc, hs, 1, P.fcw[g], 2 * hs, 1, W.dy[0], 2 * hs, none, 0, 0, nullptr,
+                       st));
         if (g == 0) {
             RC(back_stack(0, A.xseq, s.kseq, W.dxseq));
             if (s.E) {
-                embed_grad_kernel<<<m->cfg.vocab_size, 256, 0, st>>>(W.dxseq, s.kseq, A.codes, NT, s.E, *G.embed);
-                m->launches++;
-                DSP_CUDA(cudaGetLastError());
+                RC(launch_models(m, G, embed_grad_kernel, embed_grad_batch_kernel, dim3(m->cfg.vocab_size, G), 256, 0, st,
+                                 PCF(W.dxseq), s.kseq, Per<const int32_t>(A.codes), NT, s.E, Gr.embed));
             } else {
-                DSP_CUDA(cudaMemsetAsync(*G.embed, 0, sizeof(float) * m->cfg.vocab_size * m->cfg.embedding_size, st));
+                for (int i = 0; i < G; ++i)
+                    DSP_CUDA(cudaMemsetAsync(Gr.embed.p[i], 0, sizeof(float) * m->cfg.vocab_size * m->cfg.embedding_size, st));
             }
         } else {
-            RC(back_stack(1, A.sig, s.S, nullptr));
+            RC(back_stack(1, A.sig, s.S, PF()));
         }
         comb_off += hs;
     }

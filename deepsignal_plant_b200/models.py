@@ -101,6 +101,7 @@ class ModelBiLSTM(nn.Module):
         self.dropout_rate = float(dropout_rate)
         self.trainable = bool(trainable)
         self.last_dropout_masks = None
+        self.dropout_generator = None     # a CUDA torch.Generator for the training dropout masks; None: torch's default
         self._calls = 0
         self._handle = None
         self._handle_device = None
@@ -235,13 +236,15 @@ class ModelBiLSTM(nn.Module):
         shapes += [(n, T, 2 * H)] * (self.num_layers1 - 1)
         return shapes + [(n, 2 * H), (n, H)]
 
-    def draw_dropout_masks(self, n, dev):
+    def draw_dropout_masks(self, n, dev, generator=None):
         """keep / (1 - p) masks drawn with torch's CUDA generator (``torch.rand >= p``), as nn.Dropout
-        scales them; all ``None`` when ``dropout_rate`` is 0."""
+        scales them; all ``None`` when ``dropout_rate`` is 0.  ``generator``: a CUDA ``torch.Generator`` to draw
+        from instead of the default one."""
         p = self.dropout_rate
         if p <= 0:
             return [None] * len(self.dropout_mask_shapes(n))
-        return [None if shp is None else (torch.rand(shp, device=dev) >= p).to(torch.float32).div_(1.0 - p)
+        return [None if shp is None else
+                (torch.rand(shp, device=dev, generator=generator) >= p).to(torch.float32).div_(1.0 - p)
                 for shp in self.dropout_mask_shapes(n)]
 
     def forward(self, kmer, base_means, base_stds, base_signal_lens, signals):
@@ -287,27 +290,47 @@ class ModelBiLSTM(nn.Module):
         if dev.type != "cuda":
             raise RuntimeError("ModelBiLSTM parameters are on %s; move the model to a CUDA device "
                                "(.cuda(device)) -- this implementation has no CPU fallback" % dev)
-        T, S = self.seq_len, self.signal_len
-        has_seq = self.module != "signal_bilstm"
-        has_sig = self.module != "seq_bilstm"
-        inputs = (self._prep(kmer, dev, (-1, T)) if has_seq else None,
-                  self._prep(base_means, dev, (-1, T)) if has_seq else None,
-                  self._prep(base_stds, dev, (-1, T)) if has_seq else None,
-                  self._prep(base_signal_lens, dev, (-1, T)) if has_seq else None,
-                  self._prep(signals, dev, (-1, T, S)) if has_sig else None)
-        n = (inputs[0] if has_seq else inputs[4]).shape[0]
+        inputs = self._train_inputs(kmer, base_means, base_stds, base_signal_lens, signals)
+        n = (inputs[0] if inputs[0] is not None else inputs[4]).shape[0]
         with torch.cuda.device(dev):
             handle = self._create_handle(dev)
             states_arg, keep = self._init_hidden_states(n, dev) if self._uses_init_hidden() else (None, [])
-            masks = self.draw_dropout_masks(n, dev)
+            masks = self._draw_masks(n, dev)
             self.last_dropout_masks = masks
             self._calls += 1
-            params = [p for p in self.state_dict(keep_vars=True).values()]
-            for p in params:
-                if p.dtype != torch.float32 or not p.is_contiguous():
-                    raise RuntimeError("training needs contiguous float32 parameters")
+            params = self._train_params()
             logits = _TrainStep.apply(handle, inputs, states_arg, keep, masks, (self.seed << 20) + self._calls, *params)
         return logits, torch.softmax(logits, 1)
+
+    def _draw_masks(self, n, dev):
+        # the two-argument call when no generator is set: code may replace draw_dropout_masks with its own
+        if self.dropout_generator is None:
+            return self.draw_dropout_masks(n, dev)
+        return self.draw_dropout_masks(n, dev, generator=self.dropout_generator)
+
+    def _train_inputs(self, kmer, base_means, base_stds, base_signal_lens, signals):
+        dev = self._param_device()
+        T, S = self.seq_len, self.signal_len
+        has_seq = self.module != "signal_bilstm"
+        has_sig = self.module != "seq_bilstm"
+        return (self._prep(kmer, dev, (-1, T)) if has_seq else None,
+                self._prep(base_means, dev, (-1, T)) if has_seq else None,
+                self._prep(base_stds, dev, (-1, T)) if has_seq else None,
+                self._prep(base_signal_lens, dev, (-1, T)) if has_seq else None,
+                self._prep(signals, dev, (-1, T, S)) if has_sig else None)
+
+    def _train_params(self):
+        params = [p for p in self.state_dict(keep_vars=True).values()]
+        for p in params:
+            if p.dtype != torch.float32 or not p.is_contiguous():
+                raise RuntimeError("training needs contiguous float32 parameters")
+        return params
+
+    def _train_config(self):
+        """What the models of one batched training step must share (forward_train_batch)."""
+        return (self.module, self.seq_len, self.signal_len, self.num_layers1, self.num_layers2, self.num_classes,
+                self.hidden_size, self.vocab_size, self.embedding_size, bool(self.is_base), bool(self.is_signallen),
+                self.dropout_rate)
 
     # ---- host-buffer entry (the FloatTensor/.cpu() boundary of _call_mods) ---------------
     def forward_host(self, kmer, base_means, base_stds, base_signal_lens, signals):
@@ -428,3 +451,106 @@ class _TrainStep(torch.autograd.Function):
                                            ctx.arena.data_ptr(), dlogits.data_ptr(), ctx.n, ws.data_ptr(),
                                            _ptr_array(grads), stream), "dsp_train_backward")
         return (None,) * 6 + tuple(grads)
+
+
+class _TrainBatchStep(torch.autograd.Function):
+    """The logits of G <= DSP_TRAIN_MAX_MODELS models of one configuration, each on its own batch of n sites, from one
+    ``dsp_train_forward_batch`` call; backward hands every model's dlogits to one ``dsp_train_backward_batch``.  Each
+    model's logits and gradients are bit-identical to its own ``_TrainStep``.  ``params`` is the G models' state_dict
+    lists back to back."""
+
+    @staticmethod
+    def forward(ctx, handle, G, n, inputs, states, keep, masks, seeds, *params):
+        L = _native.lib()
+        dev = params[0].device
+        n_params = len(params) // G
+        C_ = params[n_params - 1].shape[0]
+        nbytes = int(L.dsp_train_arena_bytes(handle, n))
+        arenas = [torch.empty(nbytes, dtype=torch.uint8, device=dev) for _ in range(G)]
+        logits = [torch.empty((n, C_), dtype=torch.float32, device=dev) for _ in range(G)]
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _native.check(L.dsp_train_forward_batch(
+            handle, G, _ptr_array(params), n_params, _ptr_array([t for inp in inputs for t in inp]),
+            None if states is None else (C.c_void_p * len(states))(*states), (C.c_uint64 * G)(*seeds),
+            _ptr_array([m for ms in masks for m in ms]), n, _ptr_array(arenas), _ptr_array(logits), stream),
+            "dsp_train_forward_batch")
+        ctx.handle, ctx.G, ctx.n, ctx.arenas, ctx.masks = handle, G, n, arenas, masks
+        ctx.save_for_backward(*params)
+        return tuple(logits)
+
+    @staticmethod
+    def backward(ctx, *dlogits):
+        L = _native.lib()
+        params = ctx.saved_tensors
+        dev = params[0].device
+        C_ = params[len(params) // ctx.G - 1].shape[0]
+        dl = [torch.zeros((ctx.n, C_), dtype=torch.float32, device=dev) if d is None else d.to(torch.float32).contiguous()
+              for d in dlogits]
+        nbytes = int(L.dsp_train_workspace_bytes(ctx.handle, ctx.n))
+        ws = [torch.empty(nbytes, dtype=torch.uint8, device=dev) for _ in range(ctx.G)]
+        grads = [torch.empty_like(p) for p in params]
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _native.check(L.dsp_train_backward_batch(
+            ctx.handle, ctx.G, _ptr_array(params), len(params) // ctx.G, _ptr_array([m for ms in ctx.masks for m in ms]),
+            _ptr_array(ctx.arenas), _ptr_array(dl), ctx.n, _ptr_array(ws), _ptr_array(grads), stream),
+            "dsp_train_backward_batch")
+        return (None,) * 8 + tuple(grads)
+
+
+def forward_train_batch(models, batches):
+    """Training forward of several models at once: ``batches[i]`` is the input tuple ``(kmer, base_means, base_stds,
+    base_signal_lens, signals)`` of ``models[i]``.  Returns one logits tensor per model, each connected to its own
+    model's parameters, so ``sum(losses).backward()`` fills every model's ``.grad`` as its own ``loss.backward()``
+    would, bit for bit.
+
+    Models whose batches have the same site count run together, up to DSP_TRAIN_MAX_MODELS per kernel launch
+    (larger groups are cut into several calls).  Each model draws its dropout masks (from its
+    ``dropout_generator``), its Philox seed and its ``last_dropout_masks`` exactly as its own ``forward`` would.
+    The models must be trainable, in ``train()`` mode, on one CUDA device and of one configuration."""
+    models, batches = list(models), list(batches)
+    if len(models) != len(batches):
+        raise ValueError("forward_train_batch: %d models but %d batches" % (len(models), len(batches)))
+    if not models:
+        return []
+    dev = models[0]._param_device()
+    cfg = models[0]._train_config()
+    for m in models:
+        if not (isinstance(m, ModelBiLSTM) and m.trainable and m.training):
+            raise RuntimeError("forward_train_batch needs ModelBiLSTM(..., trainable=True) modules in train() mode")
+        if m._param_device() != dev or dev.type != "cuda":
+            raise RuntimeError("forward_train_batch: the models must share one CUDA device (%s and %s)"
+                               % (dev, m._param_device()))
+        if m._train_config() != cfg:
+            raise ValueError("forward_train_batch: the models must have equal configurations")
+    init_hidden = [m._uses_init_hidden() for m in models]
+    if any(init_hidden) and not all(init_hidden):
+        raise ValueError("forward_train_batch: either every model or none draws its states with init_hidden")
+    with torch.cuda.device(dev):
+        inputs = [m._train_inputs(*b) for m, b in zip(models, batches)]
+        sizes = [(x[0] if x[0] is not None else x[4]).shape[0] for x in inputs]
+        handle = models[0]._create_handle(dev)
+        out = [None] * len(models)
+        groups = {}
+        for i, n in enumerate(sizes):
+            groups.setdefault(n, []).append(i)
+        for n, idx in groups.items():
+            for c in range(0, len(idx), _native.TRAIN_MAX_MODELS):
+                part = idx[c:c + _native.TRAIN_MAX_MODELS]
+                states, keep, masks, seeds, params = ([] if init_hidden[0] else None), [], [], [], []
+                for i in part:
+                    m = models[i]
+                    if states is not None:
+                        ptrs, kept = m._init_hidden_states(n, dev)
+                        states += list(ptrs)          # raw device pointers; `keep` holds the tensors behind them
+                        keep += kept
+                    mk = m._draw_masks(n, dev)
+                    m.last_dropout_masks = mk
+                    masks.append(mk)
+                    m._calls += 1
+                    seeds.append((m.seed << 20) + m._calls)
+                    params += m._train_params()
+                logits = _TrainBatchStep.apply(handle, len(part), n, [inputs[i] for i in part], states, keep, masks,
+                                               seeds, *params)
+                for i, lg in zip(part, logits):
+                    out[i] = lg
+    return out

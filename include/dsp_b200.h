@@ -172,6 +172,33 @@ int dsp_train_backward(dsp_handle h, const float* const* params, int32_t n_param
                        const float* const* dropout_masks, const void* arena, const float* dlogits,
                        int64_t n, void* workspace, float* const* grads, void* stream);
 
+/* Model-batched training step: the forward (backward) of n_models <= DSP_TRAIN_MAX_MODELS independent models
+ * of the handle's configuration, each on its own batch of the same site count n, in the launches of one
+ * dsp_train_forward (dsp_train_backward) call -- the same number of launches, each covering every model.
+ * Each model gets exactly the work a one-model call does (same tiles, split-K counts and summation order),
+ * so its logits and gradients are bit-identical to dsp_train_forward / dsp_train_backward with the same
+ * inputs, states, seed and masks.  Per-model tables, model i's entries at [i * stride + k]:
+ *   params[n_models * n_params]     the one-model params list of model i;
+ *   inputs[n_models * 5]            kmer, base_means, base_stds, base_signal_lens, signals of model i
+ *                                   (the unused ones of the module may be NULL);
+ *   states[n_models * 6] or NULL    as for dsp_train_forward; NULL draws every model's states from seeds[i];
+ *   seeds[n_models];
+ *   dropout_masks[n_models * n_masks] the one-model mask slots; a slot must be NULL for all models or none;
+ *   arenas[n_models], workspaces[n_models]  one dsp_train_arena_bytes / dsp_train_workspace_bytes region each;
+ *   logits[n_models], dlogits[n_models]     (n, num_classes) each;
+ *   grads[n_models * n_params].
+ * A count outside [1, DSP_TRAIN_MAX_MODELS], a null table or a null required entry is refused before
+ * anything is launched. */
+#define DSP_TRAIN_MAX_MODELS 8
+int dsp_train_forward_batch(dsp_handle h, int32_t n_models, const float* const* params, int32_t n_params,
+                            const float* const* inputs, const float* const* states, const uint64_t* seeds,
+                            const float* const* dropout_masks, int64_t n, void* const* arenas,
+                            float* const* logits, void* stream);
+int dsp_train_backward_batch(dsp_handle h, int32_t n_models, const float* const* params, int32_t n_params,
+                             const float* const* dropout_masks, const void* const* arenas,
+                             const float* const* dlogits, int64_t n, void* const* workspaces,
+                             float* const* grads, void* stream);
+
 /* dsp_ranger_step: one step of Ranger (RAdam + Lookahead + gradient centralisation, the reference's
  * utils/ranger2020.py) for the n_tensors tensors of one parameter group, in place, on the current device.
  * Per tensor i, all DEVICE pointers to numel[i] contiguous float32 elements: params[i] (p), grads[i] (g),
